@@ -2,6 +2,7 @@
 """Benchmark of the boosted-mixture density path (BASELINE.json metric: boosted mixture log-density samples/sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg3_miniboone] [--mode f16|fp32]
+                    [--dump-outputs DIR]
 
 A "step" is ONE pass of the hot path over ONE eval batch (default 65 536 rows) of synthetic N(0,1) rows:
 fused per-component log q_c + rho-weighted logsumexp (one kernel) followed by the boosting weights.  Rows are
@@ -10,7 +11,8 @@ resident in HBM for `value` (the resident set, 2^20 rows, is larger than L2 and 
 the timed region.  Multi-GPU = batch-parallel weak scaling: every rank evaluates its own batch, the boosting
 weights use the global softmax (three scalar all-reduces over NCCL); `--parallel component` shards the components
 instead (every rank sees the batch, one all-gather of [B, C/G] log q per step, strong scaling).  One JSON line on
-stdout (rank 0).
+stdout (rank 0).  `--dump-outputs DIR` also writes what the last timed step returned (rank 0), so that two builds run with
+the same arguments, hence on the same seeded model and rows, can be compared output for output.
 """
 import argparse
 import json
@@ -24,6 +26,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree (it may be read-only)
 
 CONFIGS = {   # BASELINE.json "configs" / SURVEY 8(d)
     "cfg1_toy": dict(kind="realnvp", D=2, C=8, K=1, h=256, bn=False, toy=True, rho="uniform"),
@@ -34,6 +37,22 @@ CONFIGS = {   # BASELINE.json "configs" / SURVEY 8(d)
 }
 METRIC = "boosted_mixture_logdensity_samples_per_sec"
 UNIT = "samples/s"
+DUMP_BYTES = 60 << 20      # --dump-outputs: at most 64 MB in all, .npy headers included
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes each per-row output as out_dir/<name>.npy (float32).  When the rows would exceed DUMP_BYTES, every output keeps
+    the same fixed, seeded sample of rows (in row order), so files of two runs with the same arguments still line up."""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in outputs.items()}
+    rows = len(next(iter(arrays.values())))
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    if rows * row_bytes > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(rows, DUMP_BYTES // row_bytes, replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def flops_per_sample(cfg, depth=1):
@@ -409,7 +428,7 @@ def run_ours(a):
     start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     start.record()
     for i in range(a.steps):
-        step(batches[(a.warmup + i) % nb], evs[i])
+        last = step(batches[(a.warmup + i) % nb], evs[i])
     end.record()
     sync()
     t_wall1 = time.time()
@@ -469,6 +488,8 @@ def run_ours(a):
 
     if peer:
         gd.shutdown_peer_exchange(model)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"mixture_log_density": last[0], "boosting_weights": last[1]})
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -540,7 +561,12 @@ def main():
     p.add_argument("--nccl", action="store_true", help="N > 1: torch.distributed collectives between the staged kernels instead of "
                    "the library's peer-memory exchange (A/B measurements)")
     p.add_argument("--port", action="store_true", help="--impl reference: time the oracle's torch-CPU port even when baseline/_ref exists")
+    p.add_argument("--dump-outputs", metavar="DIR", help="write the G_ll and boosting weights of the last timed step to DIR/<name>.npy")
     a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs needs --impl ours")
     a.warmup = max(a.warmup, 3)
     if a.impl == "reference":
         run_reference(a)

@@ -1,7 +1,6 @@
 import os
 import sys
 
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -9,7 +8,8 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
-GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
+from tests.golden import store  # noqa: E402
+
 GOLDEN_CASES = ["glow_d43", "glow_d6_additive_relu", "realnvp_d6_bn", "realnvp_d5_mixed", "glow_d43_h256", "realnvp_d6_h128_bn",
                 "toy_d2", "glow_d43_h512", "glow_d43_h128_depth2"]
 # ResidualNet s / t networks: served by the exact fp32 kernel only (the f16 tensor-core modes reject them)
@@ -40,6 +40,6 @@ def golden():
 
     def load(name):
         if name not in cache:
-            cache[name] = dict(np.load(os.path.join(GOLDEN_DIR, name + ".npz"), allow_pickle=False))
+            cache[name] = store.load(name)
         return cache[name]
     return load

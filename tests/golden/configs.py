@@ -1,4 +1,5 @@
 """Fixture configurations shared by make_golden.py (needs the reference) and the tests (do not)."""
+import argparse
 
 CONFIGS = {
     # name: (args kwargs, seed, B, toy_base)
@@ -25,5 +26,29 @@ CONFIGS = {
     "glow_d6_invconv": (dict(kind="glow", D=6, C=2, K=3, h=64, flow_permutation="invconv"), 13, 150, False),
     "glow_d43_invconv_plain": (dict(kind="glow", D=43, C=2, K=2, h=64, flow_permutation="invconv", LU_decomposed=False), 14, 140, False),
 }
-# fixtures whose initial state_dict is stored as per-tensor SHA-1 digests instead of values (file size)
-STATE0_DIGEST_ONLY = {"glow_d43_h512"}
+# fixtures whose initial state_dict is stored as per-tensor SHA-1 digests instead of values (file size: every fixture stays under 1 MB)
+STATE0_DIGEST_ONLY = {"glow_d43_h512", "glow_d43_h256", "glow_d43_h128_depth2", "realnvp_d6_bn", "realnvp_d6_h128_bn",
+                      "realnvp_d5_residual2_bn"}
+# fixtures whose coupling-network weights and biases are not stored at all: they are the seeded initial values (nothing before the
+# fixture is taken changes them), rebuilt by store.load() from the seed.  Subset of STATE0_DIGEST_ONLY: the digests vouch for them.
+SEEDED_WEIGHTS = {"glow_d43_h512", "glow_d43_h256"}
+
+
+def make_args(kind, D, C, K, h, **kw):
+    """The reference's argument namespace for a fixture (density_experiment.py defaults, CPU)."""
+    import torch
+    a = argparse.Namespace(
+        flow="boosted", boosted=True, density_evaluation=True, device=torch.device("cpu"), cuda=False,
+        component_type=kind, num_components=C, num_flows=K, z_size=D, input_size=[D], h_size=h,
+        rho_init="decreasing", coupling_network="tanh", coupling_network_depth=1, batch_norm=False,
+        flow_permutation="shuffle", flow_coupling="affine", actnorm_scale=1.0, LU_decomposed=True, num_blocks=1,
+        num_dequant_blocks=0, learn_top=False, y_classes=1, y_condition=False, sample_size=16, save_results=False,
+        num_components_=C, batch_size=64, rho_iters=0)
+    for k, v in kw.items():
+        setattr(a, k, v)
+    return a
+
+
+def fixture_args(name):
+    kw = dict(CONFIGS[name][0])
+    return make_args(kw.pop("kind"), kw.pop("D"), kw.pop("C"), kw.pop("K"), kw.pop("h"), **kw)

@@ -8,7 +8,6 @@ state_dict), inputs, and the reference's outputs for every function on the hot p
 and from a .double() copy (ground truth).  The script cannot run on the GPU box (no /root/reference there); the
 fixtures travel instead.
 """
-import argparse
 import copy
 import os
 import sys
@@ -59,20 +58,8 @@ from gbnf_b200.extract import extract_model  # noqa: E402
 from oracle import gbnf_oracle as orc  # noqa: E402
 
 
-def make_args(kind, D, C, K, h, **kw):
-    a = argparse.Namespace(
-        flow="boosted", boosted=True, density_evaluation=True, device=torch.device("cpu"), cuda=False,
-        component_type=kind, num_components=C, num_flows=K, z_size=D, input_size=[D], h_size=h,
-        rho_init="decreasing", coupling_network="tanh", coupling_network_depth=1, batch_norm=False,
-        flow_permutation="shuffle", flow_coupling="affine", actnorm_scale=1.0, LU_decomposed=True, num_blocks=1,
-        num_dequant_blocks=0, learn_top=False, y_classes=1, y_condition=False, sample_size=16, save_results=False,
-        num_components_=C, batch_size=64, rho_iters=0)
-    for k, v in kw.items():
-        setattr(a, k, v)
-    return a
-
-
-from tests.golden.configs import CONFIGS, STATE0_DIGEST_ONLY  # noqa: E402
+from tests.golden.configs import CONFIGS, fixture_args  # noqa: E402
+from tests.golden.store import compact  # noqa: E402
 
 
 def eight_gaussians(n, rng):
@@ -98,9 +85,8 @@ def ref_forward_all(model, x, toy_base):
 
 def build_case(name, out_dir=None):
     """out_dir: where to write (default: next to this script); tests/test_golden_regeneration.py regenerates into a temp dir."""
-    kw, seed, B, toy_base = CONFIGS[name]
-    kw = dict(kw)
-    args = make_args(kw.pop("kind"), kw.pop("D"), kw.pop("C"), kw.pop("K"), kw.pop("h"), **kw)
+    _, seed, B, toy_base = CONFIGS[name]
+    args = fixture_args(name)
     torch.manual_seed(seed)
     model = RefBoostedFlow(args)
     state0 = {k: v.clone() for k, v in model.state_dict().items()}   # initial state, pins our constructors' RNG order
@@ -147,11 +133,7 @@ def build_case(name, out_dir=None):
     out = {"x": x_np, "x_init": x_init, "z32": z32.numpy(), "ldj32": ldj32.numpy(), "logq32": lq32.numpy(),
            "z64": z64.numpy(), "ldj64": ldj64.numpy(), "logq64": lq64.numpy()}
     for k, v in state0.items():
-        if name in STATE0_DIGEST_ONLY:
-            import hashlib
-            out["state0sha." + k] = np.frombuffer(hashlib.sha1(np.ascontiguousarray(v.numpy()).tobytes()).digest(), dtype=np.uint8)
-        else:
-            out["state0." + k] = v.numpy()
+        out["state0." + k] = v.numpy()
     out["seed"] = np.array(seed)
     # inverse direction: the reference's own decode where it is not broken upstream (1-D Glow with ADDITIVE coupling:
     # FlowStep.decode glow.py:344-366; the affine branch raises on 2-D tensors, RealNVP's decode is not an inverse -- SURVEY 7)
@@ -308,7 +290,7 @@ def build_case(name, out_dir=None):
         for c in range(C):
             out[f"grid.prob.c{c}"] = axs[(int(1 + np.floor(c / plt_width)), int(c % plt_width))].grids[0].numpy()
     path = os.path.join(out_dir or HERE, name + ".npz")
-    np.savez_compressed(path, **out)
+    np.savez_compressed(path, **compact(name, out))
     print(f"{name}: wrote {path} ({os.path.getsize(path) / 1024:.0f} KiB), |logq32-logq64|max = "
           f"{np.abs(lq32.numpy() - lq64.numpy()).max():.3e}")
 

@@ -66,6 +66,54 @@ def test_staged_reference_matches_its_source():
     assert out.returncode == 0, out.stdout + out.stderr
 
 
+def test_dump_outputs_writes_float32_rows(tmp_path):
+    import numpy as np
+    import torch
+    G, w = torch.randn(1000), torch.rand(1000)
+    bench.dump_outputs(str(tmp_path / "d"), {"mixture_log_density": G, "boosting_weights": w})
+    for name, t in (("mixture_log_density", G), ("boosting_weights", w)):
+        a = np.load(tmp_path / "d" / (name + ".npy"))
+        assert a.dtype == np.float32 and np.array_equal(a, t.numpy())
+
+
+def test_dump_outputs_samples_the_same_rows_under_the_byte_budget(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4000)
+    G = torch.arange(5000, dtype=torch.float32)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"mixture_log_density": G, "boosting_weights": -G})
+    a = np.load(tmp_path / "a" / "mixture_log_density.npy")
+    assert a.shape == (500,) and np.all(np.diff(a) > 0)                   # 4000 bytes / 8 bytes per row, in row order
+    assert np.array_equal(np.load(tmp_path / "a" / "boosting_weights.npy"), -a)
+    assert np.array_equal(np.load(tmp_path / "b" / "mixture_log_density.npy"), a)
+
+
+@pytest.mark.parametrize("args", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"]])
+def test_bench_rejects_bad_arguments(args):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args, capture_output=True, text=True, timeout=120)
+    assert out.returncode == 2 and out.stdout == ""
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_timed_path(tmp_path):
+    """Two runs with the same arguments time exactly --steps steps and dump the same G_ll and weights of the last one."""
+    import numpy as np
+    dumps = []
+    for run in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--config", "cfg1_toy", "--batch", "4096", "--rows", "16384",
+                              "--steps", "5", "--warmup", "3", "--no-cpu", "--dump-outputs", str(tmp_path / run)],
+                             capture_output=True, text=True, timeout=600)
+        assert out.returncode == 0, out.stderr[-2000:]
+        d = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][0])
+        assert d["steps"] == 5 and d["value"] > 0
+        dumps.append({n: np.load(tmp_path / run / (n + ".npy")) for n in ("mixture_log_density", "boosting_weights")})
+    for n, v in dumps[0].items():
+        assert v.dtype == np.float32 and v.shape == (4096,) and np.isfinite(v).all(), n
+        np.testing.assert_allclose(dumps[1][n], v, rtol=1e-6, atol=0)
+    assert abs(float(dumps[0]["boosting_weights"].astype(np.float64).sum()) - 1.0) < 1e-4
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1"],

@@ -11,7 +11,6 @@ from helpers import build_model, golden_model
 from oracle import gbnf_oracle as orc
 
 pytestmark = pytest.mark.gpu
-GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def _model(md, mode, tc4):
@@ -88,9 +87,9 @@ def test_partial_mixture_and_odd_counts_fall_back():
         m.release(); m0.release()
 
 
-def test_reference_golden_h512():
+def test_reference_golden_h512(golden):
     """The reference-made fixture glow_d43_h512 (C = 2, K = 2) through the two-chain kernel."""
-    g = dict(np.load(os.path.join(GOLDEN, "glow_d43_h512.npz")))
+    g = golden("glow_d43_h512")
     md = golden_model(g)
     x = torch.from_numpy(g["x"]).cuda()
     G, lq, inf = _run(md, x, "f16fast", 2)

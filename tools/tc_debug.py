@@ -5,11 +5,12 @@ sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np, torch
 from helpers import build_model, golden_model
 from oracle import gbnf_oracle as orc
+from tests.golden import store
 
 names = sys.argv[1:] or ["glow_d43", "realnvp_d6_bn", "glow_d6_additive_relu", "realnvp_d5_mixed", "toy_d2"]
 for mode in ("f16", "f16fast"):
     for name in names:
-        g = dict(np.load(os.path.join(ROOT, "tests", "golden", name + ".npz")))
+        g = store.load(name)
         md = golden_model(g)
         model = build_model(md, "cuda", gemm_mode=mode)
         x = torch.from_numpy(g["x"]).cuda()
