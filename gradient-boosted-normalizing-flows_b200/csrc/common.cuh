@@ -89,7 +89,6 @@ struct CouplingArgs {
   // [(peer_col0 + c - c0) * peer_ld + row], so that the 32 rows of a warp form one 128-byte NVLink write per peer
   float* logq_peers[kMaxRanks];
   int n_peers, peer_ld, peer_col0;
-  int exp_flags;                   // experiments (GBNF_EXP env, diagnostics only): bit 0 = producer skips the weight copies
   int terms_only;                  // 1: write the mixture terms of [c0, c1) but leave the tile's logsumexp to a LATER launch of the
                                    // remaining components (an odd number of components: two-chain kernel on the even part, then
                                    // the single-chain kernel on the last component, which reduces all n_mix terms)

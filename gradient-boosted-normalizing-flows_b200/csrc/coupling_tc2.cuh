@@ -324,12 +324,8 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
       t2_wait(&misc->empty[slot], par ^ 1u, a.error_flag, 10, lane);
       p_wait += T2_CLOCK() - tw;
       if (ptx::elect_one()) {
-        if (a.exp_flags & 1) {
-          ptx::mbar_arrive(&misc->full[slot]);          // timing experiment: no data movement (results are garbage)
-        } else {
-          ptx::mbar_arrive_expect_tx(&misc->full[slot], bytes);
-          ptx::tma_bulk_g2s(ring + (size_t)slot * kT2StageBytes, src, bytes, &misc->full[slot]);
-        }
+        ptx::mbar_arrive_expect_tx(&misc->full[slot], bytes);
+        ptx::tma_bulk_g2s(ring + (size_t)slot * kT2StageBytes, src, bytes, &misc->full[slot]);
       }
       __syncwarp();
       ++sidx;
@@ -364,12 +360,8 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
                 ph_w3 ^= 1u << b;
                 if (ptx::elect_one()) {
                   const uint32_t bytes = (uint32_t)((G.cw(x) >> 4) * np3) * 32u;
-                  if (a.exp_flags & 1) {
-                    ptx::mbar_arrive(&misc->w3full[b]);
-                  } else {
-                    ptx::mbar_arrive_expect_tx(&misc->w3full[b], bytes);
-                    ptx::tma_bulk_g2s(w3buf + (size_t)b * kT2W3Bytes, w3 + (size_t)(G.ccol(x) >> 4) * np3 * 16, bytes, &misc->w3full[b]);
-                  }
+                  ptx::mbar_arrive_expect_tx(&misc->w3full[b], bytes);
+                  ptx::tma_bulk_g2s(w3buf + (size_t)b * kT2W3Bytes, w3 + (size_t)(G.ccol(x) >> 4) * np3 * 16, bytes, &misc->w3full[b]);
                 }
                 __syncwarp();
               }

@@ -169,13 +169,8 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc4_kernel(CouplingArg
       t2_wait(&misc->empty[slot], par ^ 1u, a.error_flag, 10, lane);
       p_we += T4_CLK() - tq;
       if (ptx::elect_one()) {
-        if (a.exp_flags & 1) {
-          ptx::mbar_arrive(&misc->full[slot]);
-        } else {
-          const uint32_t nb = (a.exp_flags & 2) ? (bytes >> 1) : bytes;     // timing experiment: half the weight stream
-          ptx::mbar_arrive_expect_tx(&misc->full[slot], nb);
-          ptx::tma_bulk_g2s(ring + (size_t)slot * kT2StageBytes, src, nb, &misc->full[slot]);
-        }
+        ptx::mbar_arrive_expect_tx(&misc->full[slot], bytes);
+        ptx::tma_bulk_g2s(ring + (size_t)slot * kT2StageBytes, src, bytes, &misc->full[slot]);
       }
       __syncwarp();
       if (++slot == nst) { slot = 0; par ^= 1u; }
@@ -201,12 +196,8 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc4_kernel(CouplingArg
           ph_w3 ^= 1u << b;
           if (ptx::elect_one()) {
             const uint32_t bytes = (uint32_t)((t4_cw(x) >> 4) * np3) * 32u;
-            if (a.exp_flags & 1) {
-              ptx::mbar_arrive(&misc->w3full[b]);
-            } else {
-              ptx::mbar_arrive_expect_tx(&misc->w3full[b], bytes);
-              ptx::tma_bulk_g2s(w3buf + (size_t)b * w3_stride, w3 + (size_t)(t4_ccol(x) >> 4) * np3 * 16, bytes, &misc->w3full[b]);
-            }
+            ptx::mbar_arrive_expect_tx(&misc->w3full[b], bytes);
+            ptx::tma_bulk_g2s(w3buf + (size_t)b * w3_stride, w3 + (size_t)(t4_ccol(x) >> 4) * np3 * 16, bytes, &misc->w3full[b]);
           }
           __syncwarp();
         };

@@ -18,7 +18,6 @@
 #include "coupling_tc3.cuh"
 #include "coupling_tc4.cuh"
 #include "coupling_tc5.cuh"
-#include "coupling_tc6.cuh"
 #include "train_bwd.cuh"
 
 using namespace gbnf;
@@ -56,6 +55,14 @@ inline long long round_up_ll(long long v, long long m) { return (v + m - 1) / m 
 
 }  // namespace
 
+// The coupling kernel a handle plans for its shape: fp32 (coupling_fp32.cuh), serial (coupling_tc.cuh), pipelined
+// (coupling_tc2.cuh) or CTA pair for h = 1024 (coupling_tc3.cuh).
+enum class CouplingKernel { kFp32, kSerial, kPipelined, kPair };
+// A shape-specific kernel a launch of a pipelined plan may take instead (the values are gbnf_info::two_chain): the two-chain
+// schedule for Glow / affine / tanh at h = 512 (coupling_tc4.cuh) or the interleaved s / t networks for RealNVP / tanh at h = 256
+// (coupling_tc5.cuh).  The two shapes never overlap.
+enum class AltKernel { kNone = 0, kTwoChain = 1, kInterleaved = 2 };
+
 struct gbnf_ctx {
   gbnf_config cfg{};
   ModelDims md{};
@@ -92,17 +99,12 @@ struct gbnf_ctx {
   // coupling launch plan
   int rows_per_cta = 0, ld = 0, out_max = 0, tmem_cols = 0;
   size_t smem_bytes = 0;
-  TcPlan tc{};
-  bool tc2 = false;              // pipelined tensor-core kernel (coupling_tc2.cuh) selected
-  bool tc3 = false;              // CTA-pair tensor-core kernel for h = 1024 (coupling_tc3.cuh) selected
-  bool tc4 = false;              // two-chain kernel (coupling_tc4.cuh) available for this shape: Glow / affine / tanh, h = 512
-  TcPlan tc4plan{};
-  int last_two_chain = 0;        // the most recent coupling launch went through coupling_tc4_kernel
+  CouplingKernel kernel = CouplingKernel::kFp32;
+  TcPlan tc{};                   // plan of `kernel` (tensor-core kernels)
+  AltKernel alt = AltKernel::kNone;   // the alternative a launch of a pipelined plan may take for this shape
+  TcPlan alt_plan{};
+  AltKernel last_alt = AltKernel::kNone;   // the alternative the most recent coupling launch took
   bool tc4_force = false;        // GBNF_TC4=2
-  bool tc5 = false;              // interleaved s / t kernel (coupling_tc5.cuh) available: RealNVP / tanh, h = 256
-  TcPlan tc5plan{};
-  bool tc6 = false;              // two-chain kernel for RealNVP / tanh, h = 256 (coupling_tc6.cuh)
-  TcPlan tc6plan{};
   int tc3_pairs = 0;             // CTA pairs the device keeps resident at once (cudaOccupancyMaxActiveClusters)
   int profiling = 0;             // GBNF_PROF=1: cycle counters + event trace, 2: event trace only (gbnf_get_profile / _trace)
   int last_grid = 0;
@@ -163,7 +165,7 @@ int check_status(gbnf_ctx* h) {
     return fail(GBNF_ERR_CUDA, "kernel watchdog: a bounded wait timed out (code " + std::to_string(code) + ": " + watchdog_text(code) +
                                    "); the kernel trapped and the CUDA context is unusable");
   }
-  if (f[2] != 0 && std::getenv("GBNF_EXP") == nullptr) {     // (GBNF_EXP: timing experiments compute garbage on purpose)
+  if (f[2] != 0) {
     f[2] = 0;
     return fail(GBNF_ERR_NUMERIC, "an input or activation of an earlier launch was not finite in fp16 (|v| > 65504, inf or NaN): its "
                                   "results are invalid; standardise the data or use GBNF_GEMM_FP32");
@@ -261,38 +263,32 @@ int plan_layout(gbnf_ctx* h) {
     h->tmem_cols = 0;
     if (h->smem_bytes > 227 * 1024) return fail(GBNF_ERR_INVALID, "fp32 path: hidden width too large for shared memory");
   } else {
-    // pipelined kernel when the shape allows it (GBNF_TC_V1=1 forces the serial kernel, for A/B measurements)
-    const char* force_v1 = std::getenv("GBNF_TC_V1");
-    h->tc2 = tc2_eligible(md, h->steps_h) && !(force_v1 && force_v1[0] == '1');
-    h->tc3 = !h->tc2 && tc3_eligible(md, h->steps_h);
+    h->kernel = tc2_eligible(md, h->steps_h) ? CouplingKernel::kPipelined
+              : tc3_eligible(md, h->steps_h) ? CouplingKernel::kPair : CouplingKernel::kSerial;
     std::string why;
-    if (h->tc3) {
+    if (h->kernel == CouplingKernel::kPair) {
       if (!tc3_make_plan(md, h->steps_h, &h->tc)) return fail(GBNF_ERR_INVALID, "f16 tensor-core path (h = 1024): shared memory budget exceeded");
-    } else if (h->tc2) {
+    } else if (h->kernel == CouplingKernel::kPipelined) {
       if (!tc2_make_plan(md, h->steps_h, &h->tc)) return fail(GBNF_ERR_INVALID, "f16 tensor-core path: shared memory budget exceeded");
       for (StepDesc& sd : h->steps_h)
         for (int net = 0; net < md.nnets; ++net) {
           sd.layer[net][0].NC = kT2Chunk;
           sd.layer[net][1].NC = kT2Chunk; sd.layer[net][1].NC2 = (md.h == 512) ? kT2Piece : 0;
         }
-      // two-chain schedule on the same packed image (GBNF_TC4=0 keeps the single-chain kernel, for A/B measurements)
-      const char* no_tc4 = std::getenv("GBNF_TC4");
-      h->tc4 = tc4_eligible(md, h->steps_h) && !(no_tc4 && no_tc4[0] == '0') && tc4_make_plan(md, h->steps_h, &h->tc4plan);
-      h->tc4_force = h->tc4 && no_tc4 && no_tc4[0] == '2';
-      const char* no_tc5 = std::getenv("GBNF_TC5");    // GBNF_TC5=0 keeps the serial-network kernel (A/B measurements)
-      h->tc5 = tc5_eligible(md, h->steps_h) && !(no_tc5 && no_tc5[0] == '0') && tc5_make_plan(md, h->steps_h, &h->tc5plan);
-      // two component chains for RealNVP: OPT-IN (GBNF_TC6=1, or 2 = also prefer even work units): measured 13 % SLOWER than the
-      // interleaved s / t kernel on cfg2 (DESIGN 4.1g), kept for the A/B and as a tested building block
-      const char* use_tc6 = std::getenv("GBNF_TC6");
-      h->tc6 = use_tc6 && (use_tc6[0] == '1' || use_tc6[0] == '2') && tc6_eligible(md, h->steps_h) && tc6_make_plan(md, h->steps_h, &h->tc6plan);
-      if (h->tc6 && use_tc6[0] == '2') h->tc4_force = true;
+      // the alternatives run on the same packed image (GBNF_TC4=0 keeps the single-chain kernel, GBNF_TC5=0 the serial-network
+      // kernel: bitwise references for the tests, A/B measurements)
+      const char* tc4_env = std::getenv("GBNF_TC4");
+      const char* tc5_env = std::getenv("GBNF_TC5");
+      if (tc4_eligible(md, h->steps_h) && !(tc4_env && tc4_env[0] == '0') && tc4_make_plan(md, h->steps_h, &h->alt_plan))
+        h->alt = AltKernel::kTwoChain;
+      else if (tc5_eligible(md, h->steps_h) && !(tc5_env && tc5_env[0] == '0') && tc5_make_plan(md, h->steps_h, &h->alt_plan))
+        h->alt = AltKernel::kInterleaved;
+      h->tc4_force = h->alt == AltKernel::kTwoChain && tc4_env && tc4_env[0] == '2';
     } else if (!tc_make_plan(md, h->steps_h, &h->tc, &why)) {
       return fail(GBNF_ERR_INVALID, "f16 tensor-core path: " + why);
     }
     h->tc.tanh_mode = (c.gemm_mode == GBNF_GEMM_F16_TC_FAST) ? 0 : 1;
-    h->tc4plan.tanh_mode = h->tc.tanh_mode;
-    h->tc5plan.tanh_mode = h->tc.tanh_mode;
-    h->tc6plan.tanh_mode = h->tc.tanh_mode;
+    h->alt_plan.tanh_mode = h->tc.tanh_mode;
     { const char* pe = std::getenv("GBNF_PROF"); h->profiling = (pe && pe[0] >= '1' && pe[0] <= '2') ? pe[0] - '0' : 0; }
     h->rows_per_cta = 128;
     h->smem_bytes = h->tc.smem_bytes;
@@ -342,7 +338,7 @@ int launch_coupling(gbnf_ctx* h, const float* x, long long B, int c0, int c1, fl
   // the last component through the single-chain kernel, whose last-unit reduce covers all n_mix terms (stream order makes the first
   // launch's terms visible).  5 - 16 % faster than the single-chain kernel on all of them (training: the fixed mixture has
   // 1 .. C - 1 components).
-  if (h->tc4 && h->profiling == 0 && !terms_only && z_out == nullptr && ldj_out == nullptr && !to_peers && (c1 - c0) >= 3 && ((c1 - c0) & 1)) {
+  if (h->alt == AltKernel::kTwoChain && h->profiling == 0 && !terms_only && z_out == nullptr && ldj_out == nullptr && !to_peers && (c1 - c0) >= 3 && ((c1 - c0) & 1)) {
     int rc = launch_coupling(h, x, B, c0, c1 - 1, logq, ld_logq, nullptr, nullptr, rho, n_mix, skip_c, mix_mode, G_ll, st, false, 0, 0, true);
     if (rc != GBNF_OK) return rc;
     return launch_coupling(h, x, B, c1 - 1, c1, logq ? logq + (c1 - 1 - c0) : nullptr, ld_logq, nullptr, nullptr, rho, n_mix, skip_c, mix_mode,
@@ -359,21 +355,21 @@ int launch_coupling(gbnf_ctx* h, const float* x, long long B, int c0, int c1, fl
     a.n_peers = h->cv.world; a.peer_ld = peer_ld; a.peer_col0 = peer_col0;
     for (int q = 0; q < h->cv.world; ++q) a.logq_peers[q] = h->cv.gather[q] + (h->cv.epoch & 1u) * h->cv.gather_stride;
   }
-  { const char* ee = std::getenv("GBNF_EXP"); a.exp_flags = ee ? std::atoi(ee) : 0; }
   a.prof = h->prof;
   const int R = h->rows_per_cta;
   a.num_tiles = (int)((B + R - 1) / R);
   a.split = 1; a.comps_per_unit = c1 - c0; a.num_units = a.num_tiles;
-  const int workers = h->tc3 ? h->tc3_pairs : h->num_sms;        // CTAs, or CTA pairs, that run concurrently
-  bool two_chain = false;
-  if (h->cfg.gemm_mode != GBNF_GEMM_FP32 && (h->tc2 || h->tc3)) {
+  const bool pair = h->kernel == CouplingKernel::kPair;
+  const int workers = pair ? h->tc3_pairs : h->num_sms;        // CTAs, or CTA pairs, that run concurrently
+  AltKernel alt = (h->alt == AltKernel::kInterleaved && h->profiling == 0) ? AltKernel::kInterleaved : AltKernel::kNone;
+  if (h->kernel == CouplingKernel::kPipelined || pair) {
     // split every tile's components over S units when that shortens the critical CTA (waves x components per unit)
     const int ncomp = c1 - c0;
     long long best = -1;
     // The two-chain kernel pairs the two halves of a unit's components: every unit needs the same, even number of them.  A pass
     // of it takes ~0.8 of a single-chain pass, which the cost model weighs against the coarser units (GBNF_TC4=2: always
     // prefer it when a split allows it -- tests).
-    const bool tc4_ok = ((h->tc4 && h->profiling != 2) || (h->tc6 && h->profiling == 0)) && z_out == nullptr;
+    const bool tc4_ok = h->alt == AltKernel::kTwoChain && h->profiling != 2 && z_out == nullptr;
     bool best_two = false;
     for (int S = 1; S <= ncomp; S *= 2) {
       const int cpu = (ncomp + S - 1) / S;
@@ -383,7 +379,7 @@ int launch_coupling(gbnf_ctx* h, const float* x, long long B, int c0, int c1, fl
       if (h->tc4_force && !two) cost += 1LL << 40;
       if (best < 0 || cost < best) { best = cost; a.comps_per_unit = cpu; a.split = (ncomp + cpu - 1) / cpu; best_two = two; }
     }
-    two_chain = best_two;
+    if (best_two) alt = AltKernel::kTwoChain;
     a.num_units = a.num_tiles * a.split;
     if (G_ll != nullptr) {
       const long long need = (long long)a.num_tiles * R * std::max(1, n_mix);
@@ -406,20 +402,18 @@ int launch_coupling(gbnf_ctx* h, const float* x, long long B, int c0, int c1, fl
   }
   int grid = std::min(a.num_units, workers);
   { const char* ge = std::getenv("GBNF_GRID"); if (ge && std::atoi(ge) > 0) grid = std::min(grid, std::atoi(ge)); }   // diagnostics: fewer CTAs
-  h->last_grid = h->tc3 ? 2 * grid : grid;
-  if (h->cfg.gemm_mode == GBNF_GEMM_FP32) {
-    if (R == 64) coupling_fp32_kernel<64><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
-    else if (R == 32) coupling_fp32_kernel<32><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
-    else coupling_fp32_kernel<16><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
-  } else {
-    const bool st_interleaved = h->tc5 && h->profiling == 0 && !two_chain;
-    int rc = (two_chain && h->tc6) ? tc6_launch(a, h->tc6plan, grid, st)
-           : st_interleaved ? tc5_launch(a, h->tc5plan, grid, st)
-           : two_chain ? tc4_launch(a, h->tc4plan, grid, st, h->profiling)
-           : h->tc3 ? tc3_launch(a, h->tc, grid, st, h->profiling) : h->tc2 ? tc2_launch(a, h->tc, grid, st, h->profiling) : tc_launch(a, h->tc, grid, st);
-    h->last_two_chain = (two_chain && h->tc6) ? 3 : two_chain ? 1 : st_interleaved ? 2 : 0;
-    if (rc != 0) return fail(GBNF_ERR_INVALID, "f16 tensor-core path: launch configuration rejected");
-  }
+  h->last_grid = pair ? 2 * grid : grid;
+  h->last_alt = alt;
+  int rc = 0;
+  if (alt == AltKernel::kTwoChain) rc = tc4_launch(a, h->alt_plan, grid, st, h->profiling);
+  else if (alt == AltKernel::kInterleaved) rc = tc5_launch(a, h->alt_plan, grid, st);
+  else if (h->kernel == CouplingKernel::kPipelined) rc = tc2_launch(a, h->tc, grid, st, h->profiling);
+  else if (pair) rc = tc3_launch(a, h->tc, grid, st, h->profiling);
+  else if (h->kernel == CouplingKernel::kSerial) rc = tc_launch(a, h->tc, grid, st);
+  else if (R == 64) coupling_fp32_kernel<64><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
+  else if (R == 32) coupling_fp32_kernel<32><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
+  else coupling_fp32_kernel<16><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
+  if (rc != 0) return fail(GBNF_ERR_INVALID, "f16 tensor-core path: launch configuration rejected");
   h->launches++;
   CUDA_TRY_H(h, cudaGetLastError());
   return GBNF_OK;
@@ -513,8 +507,7 @@ int gbnf_create(gbnf_handle* out, const gbnf_config* cfg) {
     CREATE_TRY(tc3_configure());
     CREATE_TRY(tc4_configure());
     CREATE_TRY(tc5_configure());
-    CREATE_TRY(tc6_configure());
-    if (h->tc3) h->tc3_pairs = tc3_max_pairs(h->tc, h->num_sms);
+    if (h->kernel == CouplingKernel::kPair) h->tc3_pairs = tc3_max_pairs(h->tc, h->num_sms);
   }
 #undef CREATE_TRY
   *out = h;
@@ -598,7 +591,7 @@ int gbnf_pack_component(gbnf_handle h, int32_t c, const gbnf_component_params* p
         const LayerDesc& L = sd_h[k].layer[net][l];
         const long long total = (long long)L.Kp * L.Np;
         const int grid = (int)std::min<long long>((total + 255) / 256, (long long)h->num_sms * 8);
-        if (f16 && h->tc3)
+        if (h->kernel == CouplingKernel::kPair)
           pack_weight_tc3_kernel<<<grid, 256, 0, st>>>(sp.W[net][l], sp.b[net][l], L, l, (__half*)h->wblob, h->fblob, h->flags + 1);
         else if (f16)
           pack_weight_f16_kernel<<<grid, 256, 0, st>>>(sp.W[net][l], sp.b[net][l], L, (__half*)h->wblob, h->fblob, h->flags + 1);
@@ -641,7 +634,7 @@ int gbnf_component_inverse(gbnf_handle h, const float* d_z, int64_t B, int32_t c
   if (h->cfg.glow_invconv && !h->inv_ok[c])
     return fail(GBNF_ERR_STATE, "inverse direction: component " + std::to_string(c) + " was packed without invconv_winv");
   const bool f16 = h->cfg.gemm_mode != GBNF_GEMM_FP32;
-  if (f16 && !h->tc2)
+  if (f16 && h->kernel != CouplingKernel::kPipelined)
     return fail(GBNF_ERR_INVALID, "inverse direction: the f16 tensor-core modes serve it through the pipelined kernel only (hidden width a "
                                   "multiple of 128 up to 512, depth 1); use GBNF_GEMM_FP32 for this configuration");
   ENTER(h);
@@ -984,7 +977,7 @@ int gbnf_mixture_component_parallel(gbnf_handle h, const float* d_x, int64_t B, 
   const int per = n_comp / world, c0 = rank * per;
   const int ld = h->cfg.C;
   const long long tstride = h->comm_rows;                   // gather buffers are component-major: [C][comm_rows]
-  if (h->cfg.gemm_mode != GBNF_GEMM_FP32 && (h->tc2 || h->tc3)) {
+  if (h->kernel == CouplingKernel::kPipelined || h->kernel == CouplingKernel::kPair) {
     // fused: the coupling kernel's epilogue stores log q into every rank's gather buffer
     int rc = launch_coupling(h, d_x, B, c0, c0 + per, nullptr, per, nullptr, nullptr, nullptr, 0, -1, 0, nullptr, st, true, (int)tstride, c0);
     if (rc != GBNF_OK) return rc;
@@ -1109,8 +1102,8 @@ int gbnf_get_info(gbnf_handle h, gbnf_info* out) {
   out->grid = h->last_grid;
   out->packed_bytes = h->w_bytes + h->f_count * 4 + h->i_count * 4;
   out->launches = h->launches;
-  out->pipelined = h->tc3 ? 2 : h->tc2 ? 1 : 0;
-  out->two_chain = h->last_two_chain;
+  out->pipelined = h->kernel == CouplingKernel::kPair ? 2 : h->kernel == CouplingKernel::kPipelined ? 1 : 0;
+  out->two_chain = (int32_t)h->last_alt;
   return GBNF_OK;
 }
 

@@ -267,7 +267,7 @@ typedef struct {
                               kernel (coupling_tc2.cuh), 0: serial tensor-core / fp32 kernel */
   int32_t two_chain;       /* 1: the last coupling launch ran the two-chain schedule (coupling_tc4.cuh: Glow / affine / tanh, h = 512,
                               an even number of components per work unit); 2: the interleaved s / t schedule (coupling_tc5.cuh:
-                              RealNVP / tanh, h = 256); 3: two component chains for that shape (coupling_tc6.cuh) */
+                              RealNVP / tanh, h = 256) */
 } gbnf_info;
 int gbnf_get_info(gbnf_handle h, gbnf_info* out);
 

@@ -1,6 +1,9 @@
-"""GPU parity tests of the two-chain schedule (csrc/coupling_tc4.cuh): Glow / affine / tanh components of hidden width 512.
-It must be BITWISE identical to the single-chain pipelined kernel (same operands, same accumulation order) and inside the
-f16 gates against the fp64 oracle.  GBNF_TC4 is read when the handle is created: 0 = single chain, 2 = prefer two chains."""
+"""GPU parity tests of the two shape-specific alternatives to the pipelined kernel.
+The two-chain schedule (csrc/coupling_tc4.cuh): Glow / affine / tanh components of hidden width 512.  It must be BITWISE
+identical to the single-chain pipelined kernel (same operands, same accumulation order) and inside the f16 gates against the
+fp64 oracle.  GBNF_TC4 is read when the handle is created: 0 = single chain, 2 = prefer two chains.
+The interleaved s / t kernel (csrc/coupling_tc5.cuh): RealNVP / tanh, h = 256.  It differs from the serial-network kernel only
+in the fp32 summation order of the last layer.  GBNF_TC5=0 keeps the serial-network kernel."""
 import os
 
 import numpy as np
@@ -98,24 +101,22 @@ def test_reference_golden_h512(golden):
     assert np.max(np.abs(lq.cpu().numpy() - ref) / np.abs(ref)) < 1e-4
 
 
-# ---- RealNVP, h = 256: interleaved s / t kernel (csrc/coupling_tc5.cuh) and two component chains (csrc/coupling_tc6.cuh) ----------
-def _run_rnvp(md, x, mode, tc5, tc6, n_mix=None):
-    """GBNF_TC5 / GBNF_TC6 are read when the handle is created: 0 = off, 2 (TC6) = prefer even work units."""
-    old = {k: os.environ.get(k) for k in ("GBNF_TC5", "GBNF_TC6")}
+# ---- RealNVP, h = 256: interleaved s / t kernel (csrc/coupling_tc5.cuh) -------------------------------------------------------------
+def _run_rnvp(md, x, mode, tc5, n_mix=None):
+    """GBNF_TC5 is read when the handle is created: 0 = serial-network kernel."""
+    old = os.environ.get("GBNF_TC5")
     try:
-        for k, v in (("GBNF_TC5", tc5), ("GBNF_TC6", tc6)):
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = str(v)
+        if tc5 is None:
+            os.environ.pop("GBNF_TC5", None)
+        else:
+            os.environ["GBNF_TC5"] = str(tc5)
         m = build_model(md, "cuda", gemm_mode=mode)
         m.pack_all()
     finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
+        if old is None:
+            os.environ.pop("GBNF_TC5", None)
+        else:
+            os.environ["GBNF_TC5"] = old
     try:
         G, lq = m.mixture_log_density(x, md["C"] if n_mix is None else n_mix, return_logq=True)
         inf = m.info()
@@ -133,19 +134,16 @@ RNVP_SHAPES = [(6, 4, 5, 65536 + 33, False, False), (2, 8, 2, 5000, False, True)
 
 @pytest.mark.parametrize("mode", ["f16fast", "f16"])
 @pytest.mark.parametrize("D,C,K,B,bn,toy", RNVP_SHAPES)
-def test_realnvp_interleaved_and_two_chain_kernels(D, C, K, B, bn, toy, mode):
+def test_realnvp_interleaved_kernel_vs_serial_network(D, C, K, B, bn, toy, mode):
     """serial-network kernel (tc2) vs interleaved s / t (tc5): same operands, only the last layer's two k-pieces are summed in
-    registers instead of in the tensor-core accumulator -> equal to fp32 rounding; two component chains (tc6) vs tc5: BITWISE equal.
+    registers instead of in the tensor-core accumulator -> equal to fp32 rounding.
     Odd D (the halves alternate), eval-BatchNorm, the toy base, z_out (single-component launches stay on tc5 / tc2)."""
     md = orc.make_synthetic_model("realnvp", D, C, K, 256, seed=20 + D, batch_norm=bn, toy_base=toy)
     x = torch.from_numpy(np.random.default_rng(D).standard_normal((B, D)).astype(np.float32)).cuda()
-    G6, lq6, z6, l6, inf6 = _run_rnvp(md, x, mode, None, 2)
-    G5, lq5, z5, l5, inf5 = _run_rnvp(md, x, mode, None, None)     # the default
-    G2, lq2, z2, l2, inf2 = _run_rnvp(md, x, mode, 0, None)
-    assert inf6["two_chain"] == 3 and inf5["two_chain"] == 2 and inf2["two_chain"] == 0
-    if K >= 2:
-        assert torch.equal(lq6, lq5) and torch.equal(G6, G5)
-    for a_, b_ in ((lq6, lq2), (G6, G2), (z6, z2), (l6, l2)):
+    G5, lq5, z5, l5, inf5 = _run_rnvp(md, x, mode, None)     # the default
+    G2, lq2, z2, l2, inf2 = _run_rnvp(md, x, mode, 0)
+    assert inf5["two_chain"] == 2 and inf2["two_chain"] == 0
+    for a_, b_ in ((lq5, lq2), (G5, G2), (z5, z2), (l5, l2)):
         d = (a_ - b_).abs().double()
         # fp32 summation order of the last layer only: 1e-7-level differences on average; on a handful of the 400 k values that
         # last bit flips the fp16 rounding of a later step's activation (2^-11 relative), i.e. the difference between two equally
@@ -154,27 +152,22 @@ def test_realnvp_interleaved_and_two_chain_kernels(D, C, K, B, bn, toy, mode):
         assert float(rel.mean()) < 2e-6 and float(rel.max()) < 2e-3, (float(rel.mean()), float(rel.max()))
     n = min(B, 2048)
     ref = orc.all_component_logq(orc.cast_model(md, np.float64), x[:n].cpu().numpy().astype(np.float64))
-    np.testing.assert_allclose(lq6[:n].cpu().numpy(), ref, rtol=1e-4, atol=2e-2)
+    np.testing.assert_allclose(lq5[:n].cpu().numpy(), ref, rtol=1e-4, atol=2e-2)
 
 
-def test_realnvp_two_chain_partial_mixture_and_rows_independent():
+def test_realnvp_interleaved_partial_mixture_and_rows_independent():
+    """The default handle runs the interleaved s / t kernel for every component count and every work-unit split, and the last
+    unit of a tile reduces the mixture terms in component order: a row slice is BITWISE equal to the same rows of the full batch."""
     md = orc.make_synthetic_model("realnvp", 6, 4, 5, 256, seed=4)
     x = torch.from_numpy(np.random.default_rng(2).standard_normal((4096 + 5, 6)).astype(np.float32)).cuda()
-    os.environ["GBNF_TC6"] = "2"              # the two-chain kernel for RealNVP is opt-in
+    m = build_model(md, "cuda", gemm_mode="f16fast")
     try:
-        m = build_model(md, "cuda", gemm_mode="f16fast")
-        m.pack_all()
-    finally:
-        os.environ.pop("GBNF_TC6", None)
-    try:
-        G4 = m.mixture_log_density(x, 4)
-        assert m.info()["two_chain"] == 3
-        G3 = m.mixture_log_density(x, 3)                       # odd count: interleaved s / t kernel
-        assert m.info()["two_chain"] == 2
-        for a_, b_ in ((0, 1), (7, 140), (1000, 4101)):
-            assert torch.equal(m.mixture_log_density(x[a_:b_].contiguous(), 3), G3[a_:b_])
-            # (a different work-unit split may pick the other kernel: equal to the last layer's fp32 summation order)
-            np.testing.assert_allclose(m.mixture_log_density(x[a_:b_].contiguous(), 4).cpu().numpy(), G4[a_:b_].cpu().numpy(), rtol=2e-3, atol=2e-3)
+        for n_mix in (4, 3):
+            G = m.mixture_log_density(x, n_mix)
+            assert m.info()["two_chain"] == 2, (n_mix, m.info())
+            for a_, b_ in ((0, 1), (7, 140), (1000, 4101)):
+                assert torch.equal(m.mixture_log_density(x[a_:b_].contiguous(), n_mix), G[a_:b_]), (n_mix, a_, b_)
+                assert m.info()["two_chain"] == 2
         m.check_status()
     finally:
         m.release()
