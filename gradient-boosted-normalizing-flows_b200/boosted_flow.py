@@ -27,6 +27,22 @@ def _stream(device):
     return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
+# the fused backward's per-row kernel (train_bwd.cuh: train_bwd_rows_kernel) and the shared memory one block may use
+FUSED_BACKWARD_ROWS = 16
+FUSED_BACKWARD_MAX_SMEM = 227 * 1024
+
+
+def fused_backward_smem_bytes(kind, D, h, K):
+    """Dynamic shared memory of the fused backward's per-row kernel for a component of K steps, counted as
+    train_bwd_smem_bytes (train_bwd.cuh) counts it; gbnf_component_backward refuses a component above FUSED_BACKWARD_MAX_SMEM.
+    Layout: step inputs zh[K + 1][R][D] | network outputs oh[K][nets][R][64] | 3 activation rows [R][ld] | weight tiles
+    [2][32][64] | 2 x [R][D], with ld = round_up(h, 64) + 4 (the |z1| <= 32 input columns of D <= 64 never widen it)."""
+    R, nnets = FUSED_BACKWARD_ROWS, 1 if kind == "glow" else 2
+    ld = -(-h // 64) * 64 + 4
+    r4 = lambda n: (n + 3) & ~3
+    return 4 * (r4((K + 1) * R * D) + K * nnets * R * 64 + 3 * R * ld + 2 * 32 * 64 + 2 * r4(R * D))
+
+
 def _f32c(t):
     assert t.dtype == torch.float32 and t.is_cuda and t.is_contiguous(), "expected a contiguous CUDA float32 tensor"
     return t
@@ -35,7 +51,8 @@ def _f32c(t):
 class _FusedComponentFlow(torch.autograd.Function):
     """(z, log_det_j) = flows[c](x) for the component that is being TRAINED, both directions served by the library: the forward
     is the fixed-component kernel (nothing saved), the backward recomputes in-kernel and returns the gradients of every
-    parameter of the component (gbnf_component_backward).  density_experiment.py:647-661 + loss.backward() :361."""
+    parameter of the component (gbnf_component_backward), and dL/dx when x requires grad.  density_experiment.py:647-661 +
+    loss.backward() :361."""
 
     @staticmethod
     def forward(ctx, model, c, x, *params):
@@ -50,8 +67,8 @@ class _FusedComponentFlow(torch.autograd.Function):
         (x,) = ctx.saved_tensors
         dz = torch.zeros_like(x) if dz is None else dz.contiguous().float()
         dldj = torch.zeros(x.shape[0], device=x.device) if dldj is None else dldj.contiguous().float()
-        grads = ctx.model._component_backward(ctx.c, x, dz, dldj)
-        return (None, None, None) + tuple(grads[id(p)] if p.requires_grad else None for p in ctx.params)
+        grads, dx = ctx.model._component_backward(ctx.c, x, dz, dldj, with_dx=ctx.needs_input_grad[2])
+        return (None, None, dx) + tuple(grads[id(p)] if p.requires_grad else None for p in ctx.params)
 
 
 class BoostedFlow(nn.Module):
@@ -132,12 +149,12 @@ class BoostedFlow(nn.Module):
     def encode(self, x, y_onehot, components):
         c = self._sample_component(components) if isinstance(components, str) else components
         flow = self.flows[c]
-        needs_grad = torch.is_grad_enabled() and any(p.requires_grad for p in flow.parameters())
+        needs_grad = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in flow.parameters()))
         if not flow.actnorm_ready():
             z, ldj = flow.forward_autograd(x)     # first training batch: data-dependent ActNorm initialisation (layers.py:473-486)
         elif needs_grad and self._fused_backward_ok(x):
             # component under training: forward AND backward through the library (recompute-in-kernel backward)
-            z, ldj = _FusedComponentFlow.apply(self, c, x.detach().contiguous(), *list(flow.parameters()))
+            z, ldj = _FusedComponentFlow.apply(self, c, x.contiguous(), *list(flow.parameters()))
         elif needs_grad:
             z, ldj = flow.forward_autograd(x)     # configurations the fused backward does not cover: the caller's autograd
         else:
@@ -147,17 +164,26 @@ class BoostedFlow(nn.Module):
 
     @torch.no_grad()
     def _fused_backward_ok(self, x):
+        """Whether gbnf_component_backward serves this configuration.  Besides the architecture (depth-1 tanh / relu networks,
+        h <= 512, D <= 64, no invconv, no BatchNorm), the per-row kernel keeps every step's input and network outputs in shared
+        memory, so num_flows x (z_size + 64 x networks per step) must fit beside the h-wide activation rows: see
+        fused_backward_smem_bytes.  The deepest component served at D = 2 / 21 / 43 / 64 is, at h = 512, K = 27 / 20 / 15 / 12
+        for Glow and K = 14 / 11 / 9 / 8 for RealNVP; at h = 64, K = 47 / 36 / 28 / 23 and 24 / 20 / 17 / 15.  Everything
+        else trains through the caller's autograd."""
         a = self.args
         if not (self.fused_backward and x.is_cuda and x.dtype == torch.float32 and a.coupling_network_depth == 1
-                and a.h_size <= 512 and self.z_size <= 64 and a.num_flows <= 32):
+                and a.h_size <= 512 and self.z_size <= 64):
+            return False
+        if fused_backward_smem_bytes(self.component_type, self.z_size, a.h_size, a.num_flows) > FUSED_BACKWARD_MAX_SMEM:
             return False
         if self.component_type == "glow":
             return a.coupling_network in ("tanh", "relu") and getattr(a, "flow_permutation", "shuffle") != "invconv"
         # RealNVP: train-mode BatchNorm couples the rows of a batch -> those configurations stay on the caller's autograd
         return a.coupling_network in ("tanh", "relu", "mixed") and not getattr(a, "batch_norm", False)
 
-    def _component_backward(self, c, x, dz, dldj):
-        """Gradients of component c's parameters for upstream (dz, dldj): {id(param): grad} (gbnf_component_backward)."""
+    def _component_backward(self, c, x, dz, dldj, with_dx=False):
+        """Gradients of component c's parameters for upstream (dz, dldj) through gbnf_component_backward:
+        ({id(param): grad}, dL/dx if with_dx else None)."""
         lib = _lib.load()
         device = x.device
         h = self.handle(device)
@@ -189,10 +215,11 @@ class BoostedFlow(nn.Module):
         cp = _lib.ComponentParams()
         cp.flip_init, cp.n_steps = getattr(self.flows[c], "flip_init", 0), len(steps)
         cp.steps = C.cast(parr, C.POINTER(_lib.StepParams))
+        dx = torch.empty_like(x, dtype=torch.float32) if with_dx else None
         _lib.check(lib.gbnf_component_backward(h, c, C.byref(cp), _ptr(x), x.shape[0], _ptr(dz), _ptr(dldj),
-                                               C.cast(garr, C.POINTER(_lib.StepGrads)), None, _stream(device)))
+                                               C.cast(garr, C.POINTER(_lib.StepGrads)), _ptr(dx), _stream(device)))
         self._keepalive[("bwd", c)] = keep
-        return out
+        return out, dx
 
     def decode(self, z, y_onehot, temperature, components):
         """x = flows[c]^{-1}(z) for ONE component c (models/boosted_flow.py:209-218; upstream's `y_onhot` keyword typo is not

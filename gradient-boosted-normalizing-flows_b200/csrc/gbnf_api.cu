@@ -764,8 +764,7 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
   if (c < 0 || c >= h->cfg.C || p->n_steps != h->cfg.K) return fail(GBNF_ERR_INVALID, "bad component index / n_steps");
   const gbnf_config& cf = h->cfg;
   const bool glow = cf.kind == GBNF_KIND_GLOW;
-  if (cf.glow_invconv || cf.depth != 1 || cf.act == GBNF_ACT_RESIDUAL || (glow && cf.act == GBNF_ACT_MIXED) || cf.h > 512 || cf.D > 64 ||
-      cf.K > kTrMaxK)
+  if (cf.glow_invconv || cf.depth != 1 || cf.act == GBNF_ACT_RESIDUAL || (glow && cf.act == GBNF_ACT_MIXED) || cf.h > 512 || cf.D > 64)
     return fail(GBNF_ERR_INVALID, "fused backward: Glow (with a permutation) or RealNVP (without BatchNorm) components with "
                                   "coupling_network_depth 1, tanh / relu (RealNVP: or mixed) networks, h <= 512, D <= 64 (others train "
                                   "through the caller's autograd)");
@@ -798,6 +797,26 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
     need_w += g.wfloats;
     ldz1 = std::max(ldz1, g.Kp[0]);
   }
+  // every refusal comes before the first allocation, memset or copy: a refused call leaves the handle and `grads` untouched
+  for (int k = 0; k < K; ++k) {
+    const gbnf_step_params& sp = p->steps[k];
+    const gbnf_step_grads& sg = grads[k];
+    if (glow) {
+      if (!sp.an_bias || !sp.an_logs || !sp.perm || !sg.an_bias || !sg.an_logs) return fail(GBNF_ERR_INVALID, "glow step needs ActNorm / perm / gradient pointers");
+    } else if (sp.bn_log_gamma || sp.bn_beta || sp.bn_mean || sp.bn_var) {
+      return fail(GBNF_ERR_INVALID, "fused backward: RealNVP steps with BatchNorm train through the caller's autograd (train-mode batch "
+                                    "statistics couple the rows of a batch)");
+    }
+    for (int net = 0; net < nnets; ++net)
+      for (int l = 0; l < 3; ++l)
+        if (!sp.W[net][l] || !sp.b[net][l] || !sg.W[net][l] || !sg.b[net][l]) return fail(GBNF_ERR_INVALID, "missing Linear weight / bias / gradient pointer");
+  }
+  const int ld = std::max(hp, ldz1) + 4;
+  const size_t smem = train_bwd_smem_bytes(K, D, nnets, ld);
+  if (smem > kTrMaxSmem)
+    return fail(GBNF_ERR_INVALID, "fused backward: the shared-memory history of K = " + std::to_string(K) + " steps at D = " + std::to_string(D) +
+                                  ", h = " + std::to_string(cf.h) + " needs " + std::to_string(smem) + " bytes > " + std::to_string(kTrMaxSmem) +
+                                  " (train through the caller's autograd)");
   if (need_w > h->tr_w_floats) {
     if (h->tr_w) cudaFree(h->tr_w);
     h->tr_w = nullptr; h->tr_w_floats = 0;
@@ -830,12 +849,8 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
     const Geo& g = geo[k];
     TrainStep& ts = h->tr_steps_h[k];
     if (glow) {
-      if (!sp.an_bias || !sp.an_logs || !sp.perm || !sg.an_bias || !sg.an_logs) return fail(GBNF_ERR_INVALID, "glow step needs ActNorm / perm / gradient pointers");
       ts.an_bias = sp.an_bias; ts.an_logs = sp.an_logs; ts.perm = (const long long*)sp.perm;
       ts.g_bias = sg.an_bias; ts.g_logs = sg.an_logs;
-    } else if (sp.bn_log_gamma || sp.bn_beta || sp.bn_mean || sp.bn_var) {
-      return fail(GBNF_ERR_INVALID, "fused backward: RealNVP steps with BatchNorm train through the caller's autograd (train-mode batch "
-                                    "statistics couple the rows of a batch)");
     }
     ts.flipped = (!glow && (((k + c) % 2) > 0)) ? 1 : 0; ts.in_dim = g.in_dim; ts.out_dim = g.out_dim;
     float* sc = h->tr_scratch + (size_t)k * h->tr_rows * per_row;
@@ -849,7 +864,6 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
       ts.d2[net] = sc; sc += h->tr_rows * hp;
       ts.d3[net] = sc; sc += h->tr_rows * 64;
       for (int l = 0; l < 3; ++l) {
-        if (!sp.W[net][l] || !sp.b[net][l] || !sg.W[net][l] || !sg.b[net][l]) return fail(GBNF_ERR_INVALID, "missing Linear weight / bias / gradient pointer");
         TrainPackJob& pj = h->tr_pack_h[(size_t)job];
         pj.W = sp.W[net][l]; pj.b = sp.b[net][l]; pj.N = g.Nn[l]; pj.Kd = g.Kd[l]; pj.Kp = g.Kp[l]; pj.Np = g.Np[l]; pj.NKp = g.NKp[l]; pj.KNp = g.KNp[l];
         pj.Wt = w; w += (long long)g.Kp[l] * g.Np[l];
@@ -877,11 +891,8 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
   train_pack_kernel<<<dim3(32, njobs), 256, 0, st>>>(h->tr_pack_d);
   TrainArgs ta{};
   ta.x = d_x; ta.B = B; ta.dz = d_dz; ta.dldj = d_dldj; ta.steps = h->tr_steps_d; ta.K = K; ta.D = D; ta.h = cf.h; ta.hp = hp;
-  ta.act = cf.act; ta.coupling = cf.coupling; ta.kind = cf.kind; ta.nnets = nnets; ta.ld = std::max(hp, ldz1) + 4; ta.zeros = zeros; ta.dx = d_dx_opt;
-  const size_t smem = ((size_t)(((K + 1) * kTrR * D + 3) & ~3) + (size_t)K * 2 * kTrR * 64 + 3ull * kTrR * ta.ld + 2ull * kF32KT * kF32NT +
-                       2ull * ((kTrR * D + 3) & ~3)) * sizeof(float);
-  if (smem > 227 * 1024) return fail(GBNF_ERR_INVALID, "fused backward: shared-memory history too large (K x D)");
-  CUDA_TRY_H(h, cudaFuncSetAttribute(train_bwd_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  ta.act = cf.act; ta.coupling = cf.coupling; ta.kind = cf.kind; ta.nnets = nnets; ta.ld = ld; ta.zeros = zeros; ta.dx = d_dx_opt;
+  CUDA_TRY_H(h, cudaFuncSetAttribute(train_bwd_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTrMaxSmem));
   train_bwd_rows_kernel<<<(unsigned)((B + kTrR - 1) / kTrR), kF32Threads, smem, st>>>(ta);
   train_wgrad_kernel<<<tile0, 256, 0, st>>>(h->tr_jobs_d, njobs, B);
   h->launches += 3;

@@ -24,7 +24,7 @@
 namespace gbnf {
 
 constexpr int kTrR = 16;             // rows per CTA of phase A
-constexpr int kTrMaxK = 32;          // coupling steps per component supported by the shared-memory history
+constexpr size_t kTrMaxSmem = 227 * 1024;   // dynamic shared memory one block may use (sm_100)
 
 struct TrainStep {                   // one coupling step of the component under training (device pointers)
   const float* an_bias; const float* an_logs; const long long* perm;       // Glow: raw reference tensors; RealNVP: null
@@ -68,7 +68,13 @@ __device__ __forceinline__ void train_gemm(int act_kind, const float* in, float*
   else                    gemm_layer_fp32<R, 0>(in, out, ld, Wt, b, Kp, Np, Ws);
 }
 
-// Dynamic smem: zh[(K+1)][R][D] | oh[K][2][R][64] | act0[R][ld] | act1[R][ld] | act2[R][ld] | Ws[2][32][64] | dzb[R][D] | tmp[R][D]
+// Dynamic smem: zh[(K+1)][R][D] | oh[K][nnets][R][64] | act0[R][ld] | act1[R][ld] | act2[R][ld] | Ws[2][32][64] | dzb[R][D] | tmp[R][D]
+// The history zh / oh grows with K: the deepest component that fits is the bound of the fused backward (gbnf.h lists a few).
+// boosted_flow.py's fused_backward_smem_bytes() mirrors this count to route the shapes that do not fit to autograd.
+inline size_t train_bwd_smem_bytes(int K, int D, int nnets, int ld) {
+  return ((size_t)(((K + 1) * kTrR * D + 3) & ~3) + (size_t)K * nnets * kTrR * 64 + 3ull * kTrR * ld + 2ull * kF32KT * kF32NT +
+          2ull * ((kTrR * D + 3) & ~3)) * sizeof(float);
+}
 __global__ void __launch_bounds__(kF32Threads, 1) train_bwd_rows_kernel(TrainArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr int R = kTrR;
@@ -76,7 +82,7 @@ __global__ void __launch_bounds__(kF32Threads, 1) train_bwd_rows_kernel(TrainArg
   const bool glow = a.kind == GBNF_KIND_GLOW;
   float* zh = reinterpret_cast<float*>(smem_raw);
   float* oh = zh + (((K + 1) * R * D + 3) & ~3);
-  float* act0 = oh + K * 2 * R * 64;
+  float* act0 = oh + K * a.nnets * R * 64;
   float* act1 = act0 + R * ld;
   float* act2 = act1 + R * ld;
   float* Ws = act2 + R * ld;
@@ -124,11 +130,11 @@ __global__ void __launch_bounds__(kF32Threads, 1) train_bwd_rows_kernel(TrainArg
         if (gr < a.B) { s.h1[net][gr * hp + j] = act1[r * ld + j]; s.h2[net][gr * hp + j] = act2[r * ld + j]; }
       }
       train_gemm<R>(0, act2, act0, ld, s.Wt[net][2], s.b[net][2], s.Kp[2], s.Np[2], Ws);
-      for (int i = tid; i < R * 64; i += kF32Threads) oh[((k * 2 + net) * R + (i >> 6)) * 64 + (i & 63)] = act0[(i >> 6) * ld + (i & 63)];
+      for (int i = tid; i < R * 64; i += kF32Threads) oh[((k * a.nnets + net) * R + (i >> 6)) * 64 + (i & 63)] = act0[(i >> 6) * ld + (i & 63)];
       __syncthreads();
     }
-    const float* o0 = oh + (k * 2) * R * 64;
-    const float* o1 = o0 + R * 64;
+    const float* o0 = oh + k * a.nnets * R * 64;
+    const float* o1 = o0 + R * 64;                               // s-network output: read for RealNVP only
     for (int i = tid; i < R * D; i += kF32Threads) {
       const int r = i / D, j = i - r * D;
       float v = tmp[i];
@@ -159,8 +165,8 @@ __global__ void __launch_bounds__(kF32Threads, 1) train_bwd_rows_kernel(TrainArg
     const TrainStep& s = a.steps[k];
     const int h0 = s.in_dim, h1d = s.out_dim;
     const float* zin = zh + k * R * D;
-    const float* o0 = oh + (k * 2) * R * 64;
-    const float* o1 = o0 + R * 64;
+    const float* o0 = oh + k * a.nnets * R * 64;
+    const float* o1 = o0 + R * 64;                               // s-network output: read for RealNVP only
     for (int i = tid; i < R * D; i += kF32Threads) {             // recompute the coupling-order input of this step
       const int r = i / D, j = i - r * D;
       const int pj = train_src_col(s, a.kind, j, hD0);

@@ -129,3 +129,22 @@ def test_actnorm_uninitialised_raises_in_eval(golden):
     y = (torch.from_numpy(g["x"]) + st.actnorm.bias) * torch.exp(st.actnorm.logs)
     np.testing.assert_allclose(y.mean(0).detach().numpy(), 0, atol=1e-5)
     np.testing.assert_allclose((y ** 2).mean(0).detach().numpy(), 1, atol=1e-3)
+
+
+def test_fused_backward_depth_bound():
+    """The shared-memory count that decides which components train through the fused backward: the deepest component served
+    at a few shapes (the table in include/gbnf.h).  tests/test_gpu_train_backward.py pins the count to the library's own."""
+    from gbnf_b200.boosted_flow import FUSED_BACKWARD_MAX_SMEM, fused_backward_smem_bytes
+
+    def deepest(kind, D, h):
+        K = 0
+        while fused_backward_smem_bytes(kind, D, h, K + 1) <= FUSED_BACKWARD_MAX_SMEM:
+            K += 1
+        return K
+    assert [deepest("glow", D, 512) for D in (2, 21, 43, 64)] == [27, 20, 15, 12]
+    assert [deepest("realnvp", D, 512) for D in (2, 21, 43, 64)] == [14, 11, 9, 8]
+    assert [deepest("glow", D, 64) for D in (2, 21, 43, 64)] == [47, 36, 28, 23]
+    assert [deepest("realnvp", D, 64) for D in (2, 21, 43, 64)] == [24, 20, 17, 15]
+    # cfg3 / cfg4 (Glow, h = 512): one 16 x 64 output block per step, not two
+    assert fused_backward_smem_bytes("glow", 43, 512, 5) == 178432 - 5 * 16 * 64 * 4
+    assert fused_backward_smem_bytes("glow", 21, 512, 10) == 214848 - 10 * 16 * 64 * 4
