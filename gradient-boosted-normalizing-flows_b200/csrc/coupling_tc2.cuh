@@ -111,18 +111,18 @@ __device__ __forceinline__ void t2_wait(uint64_t* bar, uint32_t parity, int* err
 __device__ __forceinline__ void t2_quad_bar(int quad) { asm volatile("bar.sync %0, 128;" ::"r"(2 + quad) : "memory"); }
 __device__ __forceinline__ void t2_epi_bar() { asm volatile("bar.sync 1, 512;" ::: "memory"); }
 
-// 16 accumulator values of one row -> bias + activation -> 8 packed fp16 pairs
+// N (16 or 32) accumulator values of one row -> bias + activation -> N / 2 packed fp16 pairs
 // (ReLU activations are unbounded: a value that is not finite in fp16 raises status word 2, see CouplingArgs::error_flag)
-template <int ACT, int TANH_MODE>
-__device__ __forceinline__ void t2_act_pack16(const uint32_t (&r)[16], const float* __restrict__ bias, uint32_t* p, int* status) {
+template <int ACT, int TANH_MODE, int N>
+__device__ __forceinline__ void t2_act_pack(const uint32_t (&r)[N], const float* __restrict__ bias, uint32_t* p, int* status) {
   if (ACT == 2) {
     float mx = 0.f;
 #pragma unroll
-    for (int q = 0; q < 16; ++q) mx = fmax_nan(mx, __uint_as_float(r[q]) + bias[q]);
+    for (int q = 0; q < N; ++q) mx = fmax_nan(mx, __uint_as_float(r[q]) + bias[q]);
     if (!(mx <= 65504.f)) *reinterpret_cast<volatile int*>(status + 2) = 1;
   }
 #pragma unroll
-  for (int q = 0; q < 4; ++q) {
+  for (int q = 0; q < N / 4; ++q) {
     const float4 b = *reinterpret_cast<const float4*>(bias + 4 * q);      // staged in shared memory (broadcast read)
     float v0 = __uint_as_float(r[4 * q + 0]) + b.x, v1 = __uint_as_float(r[4 * q + 1]) + b.y;
     float v2 = __uint_as_float(r[4 * q + 2]) + b.z, v3 = __uint_as_float(r[4 * q + 3]) + b.w;
@@ -131,23 +131,122 @@ __device__ __forceinline__ void t2_act_pack16(const uint32_t (&r)[16], const flo
     p[2 * q + 1] = pack_half2(v2, v3);
   }
 }
-// 32 accumulator values of one row -> bias + activation -> 16 packed fp16 pairs
-template <int ACT, int TANH_MODE>
-__device__ __forceinline__ void t2_act_pack32(const uint32_t (&r)[32], const float* __restrict__ bias, uint32_t* p, int* status) {
-  if (ACT == 2) {
-    float mx = 0.f;
+
+// ---- per-row epilogue code shared by the persistent tensor-core kernels (coupling_tc2/3/4/5.cuh): 512 epilogue threads,
+//      four per row (column group g), et = epilogue thread index ----
+
+// x tile of 128 rows -> xs (row-major, D floats a row, zero beyond row B), 8 independent loads in flight per thread
+__device__ __forceinline__ void t2_load_x_tile(float* xs, const CouplingArgs& a, int D, long long row0, int et) {
+  const int total = kTcRows * D;
+  const long long gbase = row0 * D;
+  const long long glimit = a.B * (long long)D;
+  for (int i0 = et; i0 < total; i0 += 8 * kT2EpiThreads) {
+    float v[8];
 #pragma unroll
-    for (int q = 0; q < 32; ++q) mx = fmax_nan(mx, __uint_as_float(r[q]) + bias[q]);
-    if (!(mx <= 65504.f)) *reinterpret_cast<volatile int*>(status + 2) = 1;
+    for (int u = 0; u < 8; ++u) {
+      const int i = i0 + u * kT2EpiThreads;
+      v[u] = (i < total && gbase + i < glimit) ? __ldg(a.x + gbase + i) : 0.f;
+    }
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+      const int i = i0 + u * kT2EpiThreads;
+      if (i < total) xs[i] = v[u];
+    }
   }
+}
+
+// ActNorm / eval-BatchNorm affine fused into the gather of z1 -> A0 (fp16, canonical layout, zero padded): this thread's
+// 8-element chunks g, g + 4, ... of nch.  Forward: the row keeps the normalised value.  INV: the MLP input is z1 as it
+// stands and the row keeps the un-normalised value (inverse tables).
+template <int INV = 0>
+__device__ __forceinline__ void t2_gather_z1(float* zrow, const float4* tab1, int in_dim, int nch, int g, int row,
+                                             unsigned char* A0, int* status) {
+  for (int ch = g; ch < nch; ch += 4) {
+    // loads first, stores last: the compiler cannot prove that the gathered columns are distinct, so an interleaved
+    // load / store sequence would be serialised on shared-memory latency
+    float4 t[8];
+    float v[8];
 #pragma unroll
-  for (int q = 0; q < 8; ++q) {
-    const float4 b = *reinterpret_cast<const float4*>(bias + 4 * q);
-    float v0 = __uint_as_float(r[4 * q + 0]) + b.x, v1 = __uint_as_float(r[4 * q + 1]) + b.y;
-    float v2 = __uint_as_float(r[4 * q + 2]) + b.z, v3 = __uint_as_float(r[4 * q + 3]) + b.w;
-    tc_act4<ACT, TANH_MODE>(v0, v1, v2, v3);
-    p[2 * q + 0] = pack_half2(v0, v1);
-    p[2 * q + 1] = pack_half2(v2, v3);
+    for (int e = 0; e < 8; ++e) t[e] = tab1[ch * 8 + e];
+#pragma unroll
+    for (int e = 0; e < 8; ++e) v[e] = zrow[__float_as_int(t[e].w)];
+    if (INV) {
+#pragma unroll
+      for (int e = 0; e < 8; ++e) if (ch * 8 + e < in_dim) zrow[__float_as_int(t[e].w)] = (v[e] + t[e].x) * t[e].y + t[e].z;
+    } else {
+#pragma unroll
+      for (int e = 0; e < 8; ++e) v[e] = (v[e] + t[e].x) * t[e].y + t[e].z;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) if (ch * 8 + e < in_dim) zrow[__float_as_int(t[e].w)] = v[e];   // never write the scratch column
+    }
+#pragma unroll
+    for (int e = 0; e < 8; ++e) v[e] = (ch * 8 + e < in_dim) ? v[e] : 0.f;
+    {   // a value that fp16 cannot hold (|v| > 65504, inf, NaN) would silently become inf / NaN in the GEMM operand
+      const float mx = fmax_nan(fmax_nan(fmax_nan(fabsf(v[0]), fabsf(v[1])), fmax_nan(fabsf(v[2]), fabsf(v[3]))),
+                                fmax_nan(fmax_nan(fabsf(v[4]), fabsf(v[5])), fmax_nan(fabsf(v[6]), fabsf(v[7]))));
+      if (!(mx <= 65504.f)) *reinterpret_cast<volatile int*>(status + 2) = 1;
+    }
+    st_shared_v4(A0 + a_chunk_off(row, ch * 8), pack_half2(v[0], v[1]), pack_half2(v[2], v[3]), pack_half2(v[4], v[5]),
+                 pack_half2(v[6], v[7]));
+  }
+}
+
+// End of component c for this row: base-density quadratic over the thread's columns [h0col, h1col), the four groups'
+// partial sums combined through part (quadratic) / part + 3 kTcRows (log-det) -- A0 is dead by then -- and, by the
+// writer's group-0 thread, log q and the total log-det stored to logq / the peer gather buffers / ldj_out and coef[c] + log q
+// to the mixture-term scratch.  base_off, ldj_const and base_const are the caller's: it loads them where their latency hides.
+__device__ __forceinline__ void t2_component_logq(const CouplingArgs& a, const float* zrow, float lsum, float* part, int row, int g,
+                                                  int quad, int h0col, int h1col, int Dv, long long base_off, float ldj_const,
+                                                  float base_const, const float* coef, int c, int tile, bool writer) {
+  const long long gr = (long long)tile * kTcRows + row;
+  float* const part2 = part + 3 * kTcRows;
+  float q = 0.f;
+  if (a.md.base == GBNF_BASE_STD_NORMAL) {       // mean 0, 1 / (2 var) = 0.5: the same arithmetic as the table path, no loads
+    for (int p = h0col; p < h1col; ++p) { const float d = zrow[p]; q = fmaf(d * d, 0.5f, q); }
+  } else {
+    const float* bm = a.fblob + base_off;
+    const float* bi = bm + Dv;
+    for (int p = h0col; p < h1col; ++p) { const float d = zrow[p] - __ldg(bm + p); q = fmaf(d * d, __ldg(bi + p), q); }
+  }
+  if (g > 0) { part[(g - 1) * kTcRows + row] = q; part2[(g - 1) * kTcRows + row] = lsum; }
+  t2_quad_bar(quad);
+  if (writer && g == 0) {
+    q += part[row] + part[kTcRows + row] + part[2 * kTcRows + row];
+    const float ldj_tot = (lsum + part2[row] + part2[kTcRows + row] + part2[2 * kTcRows + row]) + ldj_const;
+    const float lq = (base_const - q) + ldj_tot;
+    if (gr < a.B) {
+      if (a.logq) a.logq[gr * a.ld_logq + (c - a.c0)] = lq;
+      // component-parallel multi-GPU: the same value straight into every rank's gather buffer (peer memory over NVLink)
+      for (int i = 0; i < a.n_peers; ++i) a.logq_peers[i][(long long)(a.peer_col0 + (c - a.c0)) * a.peer_ld + gr] = lq;
+      if (a.ldj_out) a.ldj_out[gr] = ldj_tot;
+    }
+    if (a.G_ll != nullptr && c < a.n_mix) __stcg(a.lse_terms + gr * a.n_mix + c, coef[c] + lq);
+  }
+}
+
+// G_ll of the tile's rows: logsumexp over their mixture terms in component order (two passes: exact max, then the sum), by
+// the last of the tile's `split` units to arrive.  All 512 epilogue threads of the CTA call it together (the ticket takes
+// two epilogue barriers).  gr = tile * kTcRows + row.
+__device__ __forceinline__ void t2_tile_logsumexp(const CouplingArgs& a, int tile, long long gr, int g, int et, uint32_t* last_flag) {
+  bool last = true;
+  if (a.split > 1) {
+    if (g == 0) __threadfence();
+    t2_epi_bar();
+    if (et == 0) *last_flag = (atomicAdd(a.tile_ctr + tile, 1u) == (unsigned)(a.split - 1)) ? 1u : 0u;
+    t2_epi_bar();
+    last = *last_flag != 0u;
+    if (last && et == 0) a.tile_ctr[tile] = 0u;
+    if (last && g == 0) __threadfence();
+  }
+  if (last && g == 0 && gr < a.B) {
+    const float* tv = a.lse_terms + gr * a.n_mix;
+    float M = -INFINITY;
+    bool has_nan = false;
+    for (int i = 0; i < a.n_mix; ++i) { const float t = __ldcg(tv + i); M = fmaxf(M, t); has_nan |= (t != t); }
+    float S = 0.f;
+    for (int i = 0; i < a.n_mix; ++i) { const float t = __ldcg(tv + i); if (t != -INFINITY) S += expf(t - M); }
+    // torch.logsumexp semantics: a NaN term -> NaN (fmaxf drops it), +inf -> +inf, all terms -inf -> -inf
+    a.G_ll[gr] = has_nan ? __int_as_float(0x7fc00000) : (M == INFINITY || M == -INFINITY) ? M : M + logf(S);
   }
 }
 
@@ -555,7 +654,6 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
     uint32_t units = 0, stepc = 0;
     uint32_t ph_l2f = 0;
     float* const part = reinterpret_cast<float*>(A0);   // per-row partial sums of a component's log-density (A0 is dead by then)
-    float* const part2 = part + 3 * kTcRows;
     const uint32_t bstride = t2_bias_stride(md.h);
     // the first step's gather-order tables, scalars and biases; afterwards every pass stages what the next one needs
     // (cp.async issued while this pass waits for the tensor core, completed and published at the end of the pass)
@@ -585,34 +683,17 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
         const long long base_off = (md.base == GBNF_BASE_STD_NORMAL) ? 0LL : __ldg(&cdp->base_off);
         const float ldj_const = cconst.x, base_const = cconst.y;
         t2_epi_bar();                                // previous component's readers are done with zs / part
-        {
-          const int total = kTcRows * D;
-          if (c == cb) {
-            const long long gbase = row0 * D;
-            const long long glimit = a.B * (long long)D;
-            for (int i0 = et; i0 < total; i0 += 8 * kT2EpiThreads) {
-              float v[8];
-#pragma unroll
-              for (int u = 0; u < 8; ++u) {
-                const int i = i0 + u * kT2EpiThreads;
-                v[u] = (i < total && gbase + i < glimit) ? __ldg(a.x + gbase + i) : 0.f;
-              }
-#pragma unroll
-              for (int u = 0; u < 8; ++u) {
-                const int i = i0 + u * kT2EpiThreads;
-                if (i < total) xs[i] = v[u];
-              }
-            }
-            t2_epi_bar();
-          }
-          if (INV) {   // z arrives in the flow's OUTPUT column order: logical column p lives at physical column sigma[p]
-            const int* sig = a.iblob + __ldg(&cdp->sigma_off);
-            for (int p = h0col; p < h1col; ++p) zrow[__ldg(sig + p)] = xs[row * D + p];
-          } else {
-            for (int p = h0col; p < h1col; ++p) zrow[p] = xs[row * D + p];   // this thread's quarter of its own row (no div / mod)
-          }
-          if (g == 0) for (int p = D; p < Dv; ++p) zrow[p] = 0.f;         // scratch column(s): target of padded table entries
+        if (c == cb) {
+          t2_load_x_tile(xs, a, D, row0, et);
+          t2_epi_bar();
         }
+        if (INV) {   // z arrives in the flow's OUTPUT column order: logical column p lives at physical column sigma[p]
+          const int* sig = a.iblob + __ldg(&cdp->sigma_off);
+          for (int p = h0col; p < h1col; ++p) zrow[__ldg(sig + p)] = xs[row * D + p];
+        } else {
+          for (int p = h0col; p < h1col; ++p) zrow[p] = xs[row * D + p];   // this thread's quarter of its own row (no div / mod)
+        }
+        if (g == 0) for (int p = D; p < Dv; ++p) zrow[p] = 0.f;           // scratch column(s): target of padded table entries
         ptx::cp_async_wait_all();                    // (first component of the launch: the prologue's staging copies)
         t2_epi_bar();
         e_x += T2_CLOCK() - e_tmp;
@@ -634,38 +715,8 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
                                     : (u + (int)gridDim.x < a.num_units)
                                         ? a.steps + (a.c0 + ((u + (int)gridDim.x) % a.split) * a.comps_per_unit) * md.K + kfirst
                                         : nullptr;
-          // ---- ActNorm / eval-BatchNorm affine fused into the gather of z1 -> A0 (fp16, canonical layout, zero padded) ----
-          {
-            const int nch = meta[2] >> 3;                                    // 8-element chunks
-            for (int ch = g; ch < nch; ch += 4) {
-              // loads first, stores last: the compiler cannot prove that the gathered columns are distinct, so an
-              // interleaved load / store sequence would be serialised on shared-memory latency
-              float4 t[8];
-              float v[8];
-#pragma unroll
-              for (int e = 0; e < 8; ++e) t[e] = tab1[ch * 8 + e];
-#pragma unroll
-              for (int e = 0; e < 8; ++e) v[e] = zrow[__float_as_int(t[e].w)];
-              if (INV) {   // the MLP input is z1 as it stands; the row keeps the un-normalised value (inverse tables)
-#pragma unroll
-                for (int e = 0; e < 8; ++e) if (ch * 8 + e < in_dim) zrow[__float_as_int(t[e].w)] = (v[e] + t[e].x) * t[e].y + t[e].z;
-              } else {
-#pragma unroll
-                for (int e = 0; e < 8; ++e) v[e] = (v[e] + t[e].x) * t[e].y + t[e].z;
-#pragma unroll
-                for (int e = 0; e < 8; ++e) if (ch * 8 + e < in_dim) zrow[__float_as_int(t[e].w)] = v[e];   // never write the scratch column
-              }
-#pragma unroll
-              for (int e = 0; e < 8; ++e) v[e] = (ch * 8 + e < in_dim) ? v[e] : 0.f;
-              {   // a value that fp16 cannot hold (|v| > 65504, inf, NaN) would silently become inf / NaN in the GEMM operand
-                const float mx = fmax_nan(fmax_nan(fmax_nan(fabsf(v[0]), fabsf(v[1])), fmax_nan(fabsf(v[2]), fabsf(v[3]))),
-                                          fmax_nan(fmax_nan(fabsf(v[4]), fabsf(v[5])), fmax_nan(fabsf(v[6]), fabsf(v[7]))));
-                if (!(mx <= 65504.f)) *reinterpret_cast<volatile int*>(a.error_flag + 2) = 1;
-              }
-              st_shared_v4(A0 + a_chunk_off(row, ch * 8), pack_half2(v[0], v[1]), pack_half2(v[2], v[3]), pack_half2(v[4], v[5]),
-                           pack_half2(v[6], v[7]));
-            }
-          }
+          // ---- ActNorm / eval-BatchNorm affine fused into the gather of z1 -> A0 ----
+          t2_gather_z1<INV>(zrow, tab1, in_dim, meta[2] >> 3, g, row, A0, a.error_flag);
           e_pro += T2_CLOCK() - e_tmp;
           if (tr) T2_TRACE(73 + 40 * (g & 1));
           for (int net = 0; net < nnets; ++net, ++units) {
@@ -700,8 +751,8 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
                 ptx::tmem_ld32(lane_base + G.l1_col[q & 1] + (uint32_t)g * 32u, r);
                 ptx::tmem_ld_wait();
                 if (PROF && warp_e == 0 && q == 1) T2_TRACE(120);
-                if (act_kind == 1) t2_act_pack32<1, TANH_MODE>(r, b1 + q * kT2Chunk, p, a.error_flag);
-                else               t2_act_pack32<2, TANH_MODE>(r, b1 + q * kT2Chunk, p, a.error_flag);
+                if (act_kind == 1) t2_act_pack<1, TANH_MODE>(r, b1 + q * kT2Chunk, p, a.error_flag);
+                else               t2_act_pack<2, TANH_MODE>(r, b1 + q * kT2Chunk, p, a.error_flag);
                 if (PROF && warp_e == 0 && q == 1) T2_TRACE(121);
               }
               if (G.l1_even_inplace && !(q & 1)) t2_quad_bar(quad);   // packed quarter may overlap the row's unread accumulator
@@ -748,8 +799,8 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
                   uint32_t r[32];
                   ptx::tmem_ld32(sc + (uint32_t)g * 32u, r);
                   ptx::tmem_ld_wait();
-                  if (act_kind == 1) t2_act_pack32<1, TANH_MODE>(r, bj + g * 32, p, a.error_flag);
-                  else               t2_act_pack32<2, TANH_MODE>(r, bj + g * 32, p, a.error_flag);
+                  if (act_kind == 1) t2_act_pack<1, TANH_MODE>(r, bj + g * 32, p, a.error_flag);
+                  else               t2_act_pack<2, TANH_MODE>(r, bj + g * 32, p, a.error_flag);
                 }
                 t2_quad_bar(quad);             // all four threads of the row have read their columns
                 ptx::tmem_st16(sc + (uint32_t)g * 16u, p);
@@ -759,8 +810,8 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
                   uint32_t r[16];
                   ptx::tmem_ld16(sc + (uint32_t)g * 16u, r);
                   ptx::tmem_ld_wait();
-                  if (act_kind == 1) t2_act_pack16<1, TANH_MODE>(r, bj + g * 16, p, a.error_flag);
-                  else               t2_act_pack16<2, TANH_MODE>(r, bj + g * 16, p, a.error_flag);
+                  if (act_kind == 1) t2_act_pack<1, TANH_MODE>(r, bj + g * 16, p, a.error_flag);
+                  else               t2_act_pack<2, TANH_MODE>(r, bj + g * 16, p, a.error_flag);
                 }
                 ptx::tmem_st8(sc + (uint32_t)g * 16u, p);
               }
@@ -859,28 +910,8 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
           }
         }
         // ---- component log-density for this row ----
-        float q = 0.f;
-        if (md.base == GBNF_BASE_STD_NORMAL) {       // mean 0, 1 / (2 var) = 0.5: the same arithmetic as the table path, no loads
-          for (int p = h0col; p < h1col; ++p) { const float d = zrow[p]; q = fmaf(d * d, 0.5f, q); }
-        } else {
-          const float* bm = a.fblob + base_off;
-          const float* bi = bm + Dv;
-          for (int p = h0col; p < h1col; ++p) { const float d = zrow[p] - __ldg(bm + p); q = fmaf(d * d, __ldg(bi + p), q); }
-        }
-        if (g > 0) { part[(g - 1) * kTcRows + row] = q; part2[(g - 1) * kTcRows + row] = lsum; }
-        t2_quad_bar(quad);
-        if (g == 0) {
-          q += part[row] + part[kTcRows + row] + part[2 * kTcRows + row];
-          const float ldj_tot = (lsum + part2[row] + part2[kTcRows + row] + part2[2 * kTcRows + row]) + (INV ? -ldj_const : ldj_const);
-          const float lq = (base_const - q) + ldj_tot;
-          if (gr < a.B) {
-            if (a.logq) a.logq[gr * a.ld_logq + (c - a.c0)] = lq;
-            // component-parallel multi-GPU: the same value straight into every rank's gather buffer (peer memory over NVLink)
-            for (int q = 0; q < a.n_peers; ++q) a.logq_peers[q][(long long)(a.peer_col0 + (c - a.c0)) * a.peer_ld + gr] = lq;
-            if (a.ldj_out) a.ldj_out[gr] = ldj_tot;
-          }
-          if (a.G_ll != nullptr && c < a.n_mix) __stcg(a.lse_terms + ((long long)tile * kTcRows + row) * a.n_mix + c, misc->coef[c] + lq);
-        }
+        t2_component_logq(a, zrow, lsum, part, row, g, quad, h0col, h1col, Dv, base_off, INV ? -ldj_const : ldj_const, base_const,
+                          misc->coef, c, tile, true);
         if (a.z_out != nullptr && gr < a.B) {
           if (INV) {   // physical == logical column order at the flow's input
             for (int j = h0col; j < h1col; ++j) a.z_out[gr * D + j] = zrow[j];
@@ -890,30 +921,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
           }
         }
       }
-      if (a.G_ll != nullptr) {
-        // logsumexp over the tile's terms in component order (two passes: exact max, then the sum), by the last of the
-        // tile's `split` units to arrive
-        bool last = true;
-        if (a.split > 1) {
-          if (g == 0) __threadfence();
-          t2_epi_bar();
-          if (et == 0) misc->last_flag = (atomicAdd(a.tile_ctr + tile, 1u) == (unsigned)(a.split - 1)) ? 1u : 0u;
-          t2_epi_bar();
-          last = misc->last_flag != 0u;
-          if (last && et == 0) a.tile_ctr[tile] = 0u;
-          if (last && g == 0) __threadfence();
-        }
-        if (last && g == 0 && gr < a.B) {
-          const float* tv = a.lse_terms + ((long long)tile * kTcRows + row) * a.n_mix;
-          float M = -INFINITY;
-          bool has_nan = false;
-          for (int i = 0; i < a.n_mix; ++i) { const float t = __ldcg(tv + i); M = fmaxf(M, t); has_nan |= (t != t); }
-          float S = 0.f;
-          for (int i = 0; i < a.n_mix; ++i) { const float t = __ldcg(tv + i); if (t != -INFINITY) S += expf(t - M); }
-          // torch.logsumexp semantics: a NaN term -> NaN (fmaxf drops it), +inf -> +inf, all terms -inf -> -inf
-          a.G_ll[gr] = has_nan ? __int_as_float(0x7fc00000) : (M == INFINITY || M == -INFINITY) ? M : M + logf(S);
-        }
-      }
+      if (a.G_ll != nullptr) t2_tile_logsumexp(a, tile, gr, g, et, &misc->last_flag);
     }
     if (PROF == 1 && a.prof != nullptr && blockIdx.x == 0 && et == 0) {
       a.prof[8] = T2_CLOCK() - e_t0; a.prof[9] = e_w1 + e_w2 + e_w3; a.prof[10] = e_l1 + e_l2; a.prof[11] = e_l3; a.prof[12] = e_pro + e_x;

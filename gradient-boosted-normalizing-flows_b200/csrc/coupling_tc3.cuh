@@ -407,7 +407,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
     const long long e_t0 = T3_CLK();
     long long e_l1f = 0, e_own = 0, e_xfull = 0, e_ship = 0, e_xfree = 0, e_l3f = 0, e_x3 = 0, e_g = 0, e_c1 = 0, e_c2 = 0, e_c3 = 0, e_c4 = 0, tq;
     float* const part = reinterpret_cast<float*>(A0);
-    float* const part2 = part + 3 * kTcRows;
     const uint32_t peer = (uint32_t)(p ^ 1);
     const uint32_t xb_peer = ptx::mapa(ptx::smem_u32(xb), peer);                 // the PEER's exchange buffer
     const uint32_t xfull_peer = ptx::mapa(ptx::smem_u32(&misc->xfull), peer);
@@ -490,30 +489,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
           const int act_kind = (md.act == GBNF_ACT_RELU) ? 2 : 1;
           // ---- ActNorm affine fused into the gather of z1 -> A0 (both CTAs build the same image) ----
           tq = T3_CLK();
-          {
-            const int nch = meta[2] >> 3;
-            for (int ch = g; ch < nch; ch += 4) {
-              float4 t[8];
-              float v[8];
-#pragma unroll
-              for (int e = 0; e < 8; ++e) t[e] = tab1[ch * 8 + e];
-#pragma unroll
-              for (int e = 0; e < 8; ++e) v[e] = zrow[__float_as_int(t[e].w)];
-#pragma unroll
-              for (int e = 0; e < 8; ++e) v[e] = (v[e] + t[e].x) * t[e].y + t[e].z;
-#pragma unroll
-              for (int e = 0; e < 8; ++e) if (ch * 8 + e < in_dim) zrow[__float_as_int(t[e].w)] = v[e];
-#pragma unroll
-              for (int e = 0; e < 8; ++e) v[e] = (ch * 8 + e < in_dim) ? v[e] : 0.f;
-              {
-                const float mx = fmax_nan(fmax_nan(fmax_nan(fabsf(v[0]), fabsf(v[1])), fmax_nan(fabsf(v[2]), fabsf(v[3]))),
-                                          fmax_nan(fmax_nan(fabsf(v[4]), fabsf(v[5])), fmax_nan(fabsf(v[6]), fabsf(v[7]))));
-                if (!(mx <= 65504.f)) *reinterpret_cast<volatile int*>(a.error_flag + 2) = 1;
-              }
-              st_shared_v4(A0 + a_chunk_off(row, ch * 8), pack_half2(v[0], v[1]), pack_half2(v[2], v[3]), pack_half2(v[4], v[5]),
-                           pack_half2(v[6], v[7]));
-            }
-          }
+          t2_gather_z1(zrow, tab1, in_dim, meta[2] >> 3, g, row, A0, a.error_flag);
           ptx::fence_proxy_async_smem();
           ptx::tc_fence_before();
           t2_warp_arrive(&misc->a0r, lane);
@@ -532,8 +508,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
               uint32_t r[32];
               ptx::tmem_ld32(lane_base + ((q & 1) ? kT3SlotB0 : kT3SlotA) + (uint32_t)g * 32u, r);
               ptx::tmem_ld_wait();
-              if (act_kind == 1) t2_act_pack32<1, TANH_MODE>(r, bias_c + q * 128 + g * 32, pk, a.error_flag);
-              else               t2_act_pack32<2, TANH_MODE>(r, bias_c + q * 128 + g * 32, pk, a.error_flag);
+              if (act_kind == 1) t2_act_pack<1, TANH_MODE>(r, bias_c + q * 128 + g * 32, pk, a.error_flag);
+              else               t2_act_pack<2, TANH_MODE>(r, bias_c + q * 128 + g * 32, pk, a.error_flag);
             }
             ptx::tmem_st16(lane_base + (uint32_t)q * 64u + (uint32_t)g * 16u, pk);
             ptx::tmem_st_wait();
@@ -718,53 +694,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
           e_c4 += T3_CLK() - tq;
         }
         // ---- component log-density for this row (both CTAs hold the same z; rank 0 writes) ----
-        float q = 0.f;
-        if (md.base == GBNF_BASE_STD_NORMAL) {
-          for (int c2 = h0col; c2 < h1col; ++c2) { const float d = zrow[c2]; q = fmaf(d * d, 0.5f, q); }
-        } else {
-          const float* bm = a.fblob + base_off;
-          const float* bi = bm + Dv;
-          for (int c2 = h0col; c2 < h1col; ++c2) { const float d = zrow[c2] - __ldg(bm + c2); q = fmaf(d * d, __ldg(bi + c2), q); }
-        }
-        if (g > 0) { part[(g - 1) * kTcRows + row] = q; part2[(g - 1) * kTcRows + row] = lsum; }
-        t2_quad_bar(quad);
-        if (g == 0 && p == 0) {
-          q += part[row] + part[kTcRows + row] + part[2 * kTcRows + row];
-          const float ldj_tot = (lsum + part2[row] + part2[kTcRows + row] + part2[2 * kTcRows + row]) + ldj_const;
-          const float lq = (base_const - q) + ldj_tot;
-          if (gr < a.B) {
-            if (a.logq) a.logq[gr * a.ld_logq + (c - a.c0)] = lq;
-            for (int q = 0; q < a.n_peers; ++q) a.logq_peers[q][(long long)(a.peer_col0 + (c - a.c0)) * a.peer_ld + gr] = lq;   // see coupling_tc2.cuh
-            if (a.ldj_out) a.ldj_out[gr] = ldj_tot;
-          }
-          if (a.G_ll != nullptr && c < a.n_mix) __stcg(a.lse_terms + ((long long)tile * kTcRows + row) * a.n_mix + c, misc->coef[c] + lq);
-        }
+        t2_component_logq(a, zrow, lsum, part, row, g, quad, h0col, h1col, Dv, base_off, ldj_const, base_const, misc->coef, c, tile,
+                          p == 0);
         if (p == 0 && a.z_out != nullptr && gr < a.B) {
           const int* sig = a.iblob + __ldg(&cdp->sigma_off);
           for (int j = h0col; j < h1col; ++j) a.z_out[gr * D + j] = zrow[__ldg(sig + j)];
         }
       }
-      if (a.G_ll != nullptr && p == 0) {
-        bool last = true;
-        if (a.split > 1) {
-          if (g == 0) __threadfence();
-          t2_epi_bar();
-          if (et == 0) misc->last_flag = (atomicAdd(a.tile_ctr + tile, 1u) == (unsigned)(a.split - 1)) ? 1u : 0u;
-          t2_epi_bar();
-          last = misc->last_flag != 0u;
-          if (last && et == 0) a.tile_ctr[tile] = 0u;
-          if (last && g == 0) __threadfence();
-        }
-        if (last && g == 0 && gr < a.B) {
-          const float* tv = a.lse_terms + ((long long)tile * kTcRows + row) * a.n_mix;
-          float M = -INFINITY;
-          bool has_nan = false;
-          for (int i = 0; i < a.n_mix; ++i) { const float t = __ldcg(tv + i); M = fmaxf(M, t); has_nan |= (t != t); }
-          float S = 0.f;
-          for (int i = 0; i < a.n_mix; ++i) { const float t = __ldcg(tv + i); if (t != -INFINITY) S += expf(t - M); }
-          a.G_ll[gr] = has_nan ? __int_as_float(0x7fc00000) : (M == INFINITY || M == -INFINITY) ? M : M + logf(S);
-        }
-      }
+      if (a.G_ll != nullptr && p == 0) t2_tile_logsumexp(a, tile, gr, g, et, &misc->last_flag);
     }
     if (et == 0) ptx::bulk_wait0();                  // my last bulk copy into the peer has completed
     if (PROF && a.prof != nullptr && blockIdx.x == 0 && et == 0) {

@@ -440,31 +440,6 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc4_kernel(CouplingArg
     const long long e_t0 = T4_CLK();
     long long e_l1f = 0, e_l2f = 0, e_l3f = 0, e_fin = 0, e_bar = 0, e_e1 = 0, e_e2 = 0, e_tr = 0, e_ga = 0, tq;
 
-    // ---- z1 gather with the ActNorm affine fused -> A0 (fp16 canonical image) ----
-    auto gather = [&](float* zrow, const float4* tab1, unsigned char* A0) {
-      const int nch = k0p >> 3;
-      for (int chn = g; chn < nch; chn += 4) {
-        float4 t[8];
-        float v[8];
-#pragma unroll
-        for (int e = 0; e < 8; ++e) t[e] = tab1[chn * 8 + e];
-#pragma unroll
-        for (int e = 0; e < 8; ++e) v[e] = zrow[__float_as_int(t[e].w)];
-#pragma unroll
-        for (int e = 0; e < 8; ++e) v[e] = (v[e] + t[e].x) * t[e].y + t[e].z;
-#pragma unroll
-        for (int e = 0; e < 8; ++e) if (chn * 8 + e < in_dim) zrow[__float_as_int(t[e].w)] = v[e];
-#pragma unroll
-        for (int e = 0; e < 8; ++e) v[e] = (chn * 8 + e < in_dim) ? v[e] : 0.f;
-        {
-          const float mx = fmax_nan(fmax_nan(fmax_nan(fabsf(v[0]), fabsf(v[1])), fmax_nan(fabsf(v[2]), fabsf(v[3]))),
-                                    fmax_nan(fmax_nan(fabsf(v[4]), fabsf(v[5])), fmax_nan(fabsf(v[6]), fabsf(v[7]))));
-          if (!(mx <= 65504.f)) *reinterpret_cast<volatile int*>(a.error_flag + 2) = 1;
-        }
-        st_shared_v4(A0 + a_chunk_off(row, chn * 8), pack_half2(v[0], v[1]), pack_half2(v[2], v[3]), pack_half2(v[4], v[5]),
-                     pack_half2(v[6], v[7]));
-      }
-    };
     // ---- x rows of a component's start -> z tile (this thread's quarter of its own row) ----
     auto load_x = [&](const T4Pos& p, float* zrow) {
       const long long gr = (long long)(p.u / a.split) * kTcRows + row;
@@ -521,7 +496,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc4_kernel(CouplingArg
           ptx::tc_fence_before();             // runs under this chunk's activation instead of after it
           t2_warp_arrive(&misc->c2r, lane);
         }
-        t2_act_pack32<1, TANH_MODE>(r, bias_c + g * 32 + q * kT2Chunk, pk, a.error_flag);
+        t2_act_pack<1, TANH_MODE>(r, bias_c + g * 32 + q * kT2Chunk, pk, a.error_flag);
       }
       if (q >= 2) t2_quad_bar(quad);         // chunk 2 and half of chunk 3 accumulate inside the A1 region they are packed into
       ptx::tmem_st16(lane_base + (uint32_t)q * 64u + (uint32_t)g * 16u, pk);
@@ -547,7 +522,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc4_kernel(CouplingArg
           uint32_t r[32];
           ptx::tmem_ld32(sc + (uint32_t)g * 32u, r);
           ptx::tmem_ld_wait();
-          t2_act_pack32<1, TANH_MODE>(r, bj + g * 32, pk, a.error_flag);
+          t2_act_pack<1, TANH_MODE>(r, bj + g * 32, pk, a.error_flag);
         }
         t2_quad_bar(quad);
         ptx::tmem_st16(sc + (uint32_t)g * 16u, pk);
@@ -557,7 +532,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc4_kernel(CouplingArg
           uint32_t r[16];
           ptx::tmem_ld16(sc + (uint32_t)g * 16u, r);
           ptx::tmem_ld_wait();
-          t2_act_pack16<1, TANH_MODE>(r, bj + g * 16, pk, a.error_flag);
+          t2_act_pack<1, TANH_MODE>(r, bj + g * 16, pk, a.error_flag);
         }
         ptx::tmem_st8(sc + (uint32_t)g * 16u, pk);
       }
@@ -608,49 +583,9 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc4_kernel(CouplingArg
       const long long gr = (long long)tile * kTcRows + row;
       const int c = p.c;
       const float2 cconst = __ldg(reinterpret_cast<const float2*>(a.fblob + a.cc_off) + c);
-      float q = 0.f;
-      if (md.base == GBNF_BASE_STD_NORMAL) {
-        for (int pc = h0col; pc < h1col; ++pc) { const float d = zrow[pc]; q = fmaf(d * d, 0.5f, q); }
-      } else {
-        const float* bm = a.fblob + __ldg(&a.comps[c].base_off);
-        const float* bi = bm + Dv;
-        for (int pc = h0col; pc < h1col; ++pc) { const float d = zrow[pc] - __ldg(bm + pc); q = fmaf(d * d, __ldg(bi + pc), q); }
-      }
-      float* part2 = part + 3 * kTcRows;
-      if (g > 0) { part[(g - 1) * kTcRows + row] = q; part2[(g - 1) * kTcRows + row] = lsum; }
-      t2_quad_bar(quad);
-      if (g == 0) {
-        q += part[row] + part[kTcRows + row] + part[2 * kTcRows + row];
-        const float ldj_tot = (lsum + part2[row] + part2[kTcRows + row] + part2[2 * kTcRows + row]) + cconst.x;
-        const float lq = (cconst.y - q) + ldj_tot;
-        if (gr < a.B) {
-          if (a.logq) a.logq[gr * a.ld_logq + (c - a.c0)] = lq;
-          for (int qq = 0; qq < a.n_peers; ++qq) a.logq_peers[qq][(long long)(a.peer_col0 + (c - a.c0)) * a.peer_ld + gr] = lq;
-          if (a.ldj_out) a.ldj_out[gr] = ldj_tot;
-        }
-        if (a.G_ll != nullptr && c < a.n_mix) __stcg(a.lse_terms + ((long long)tile * kTcRows + row) * a.n_mix + c, misc->coef[c] + lq);
-      }
-      if (chain == 1 && c + 1 == p.cend && a.G_ll != nullptr && !a.terms_only) {
-        bool last = true;
-        if (a.split > 1) {
-          if (g == 0) __threadfence();
-          t2_epi_bar();
-          if (et == 0) misc->last_flag = (atomicAdd(a.tile_ctr + tile, 1u) == (unsigned)(a.split - 1)) ? 1u : 0u;
-          t2_epi_bar();
-          last = misc->last_flag != 0u;
-          if (last && et == 0) a.tile_ctr[tile] = 0u;
-          if (last && g == 0) __threadfence();
-        }
-        if (last && g == 0 && gr < a.B) {
-          const float* tv = a.lse_terms + ((long long)tile * kTcRows + row) * a.n_mix;
-          float M = -INFINITY;
-          bool has_nan = false;
-          for (int i = 0; i < a.n_mix; ++i) { const float t = __ldcg(tv + i); M = fmaxf(M, t); has_nan |= (t != t); }
-          float S = 0.f;
-          for (int i = 0; i < a.n_mix; ++i) { const float t = __ldcg(tv + i); if (t != -INFINITY) S += expf(t - M); }
-          a.G_ll[gr] = has_nan ? __int_as_float(0x7fc00000) : (M == INFINITY || M == -INFINITY) ? M : M + logf(S);
-        }
-      }
+      const long long base_off = (md.base == GBNF_BASE_STD_NORMAL) ? 0LL : __ldg(&a.comps[c].base_off);
+      t2_component_logq(a, zrow, lsum, part, row, g, quad, h0col, h1col, Dv, base_off, cconst.x, cconst.y, misc->coef, c, tile, true);
+      if (chain == 1 && c + 1 == p.cend && a.G_ll != nullptr && !a.terms_only) t2_tile_logsumexp(a, tile, gr, g, et, &misc->last_flag);
     };
     // ---- everything a chain does between two of its passes: transform of the finishing pass, (end of component), gather of
     //      the next pass, staging ----
@@ -683,7 +618,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc4_kernel(CouplingArg
           t2_quad_bar(quad);
         }
         const long long tg = T4_CLK();
-        gather(zrow, tab_s + (2 * chain + (ng & 1u)) * kEpPad, A0_b);
+        t2_gather_z1(zrow, tab_s + (2 * chain + (ng & 1u)) * kEpPad, in_dim, k0p >> 3, g, row, A0_b, a.error_flag);
         ptx::fence_proxy_async_smem();
         ptx::tc_fence_before();
         t2_warp_arrive(&misc->a0r[chain], lane);

@@ -272,8 +272,6 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc5_kernel(CouplingArg
     const int h0col = min(D, g * dq), h1col = min(D, (g + 1) * dq);
     const int c0 = g * 16;
     uint32_t npass = 0, ph_l1f = 0, ph_l2f = 0, ph_l3f = 0;
-    float* const part = part_s;
-    float* const part2 = part + 3 * kTcRows;
 
     // staging for a pass: biases of both networks (contiguous in fblob: b1 b2 b3 of t, then of s) and the step's two tables
     auto stage = [&](const StepDesc* sd, uint32_t buf) {
@@ -299,22 +297,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc5_kernel(CouplingArg
         // ---- x tile: fetched from HBM once per unit (coalesced, 8 loads in flight per thread) and kept in shared memory; every
         //      component restarts from it (with K = 1 a component is one step: a global reload per component cost 2 %) ----
         if (c == cb) {
-          const int total = kTcRows * D;
-          const long long gbase = (long long)tile * kTcRows * D;
-          const long long glimit = a.B * (long long)D;
-          for (int i0 = et; i0 < total; i0 += 8 * kT2EpiThreads) {
-            float v[8];
-#pragma unroll
-            for (int uu = 0; uu < 8; ++uu) {
-              const int i = i0 + uu * kT2EpiThreads;
-              v[uu] = (i < total && gbase + i < glimit) ? __ldg(a.x + gbase + i) : 0.f;
-            }
-#pragma unroll
-            for (int uu = 0; uu < 8; ++uu) {
-              const int i = i0 + uu * kT2EpiThreads;
-              if (i < total) xs[i] = v[uu];
-            }
-          }
+          t2_load_x_tile(xs, a, D, (long long)tile * kTcRows, et);
           t2_epi_bar();
         }
         for (int pc = h0col; pc < h1col; ++pc) zrow[pc] = xs[row * D + pc];
@@ -335,6 +318,9 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc5_kernel(CouplingArg
                                     : (u + (int)gridDim.x < a.num_units) ? a.steps + (a.c0 + ((u + (int)gridDim.x) % a.split) * a.comps_per_unit) * K
                                     : nullptr;
           // ---- eval-BatchNorm affine fused into the gather of z1 -> A0 (one A0 feeds both networks) ----
+          // The same code as t2_gather_z1, kept inline on purpose: called through the helper, the compiler keeps the table
+          // pointer live across the pass and reschedules this MUFU-bound kernel, which measured 1.5 % slower on cfg1 / cfg2
+          // (NVIDIA B200, 1000 W power limit).
           {
             const int nch = k0p >> 3;
             for (int chn = g; chn < nch; chn += 4) {
@@ -376,7 +362,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc5_kernel(CouplingArg
                 uint32_t r[32];
                 ptx::tmem_ld32(lane_base + kT5Slot + 128u * n + (uint32_t)g * 32u, r);
                 ptx::tmem_ld_wait();
-                t2_act_pack32<1, TANH_MODE>(r, bias_c + n * (512 + np3) + q * 128 + g * 32, pk, a.error_flag);
+                t2_act_pack<1, TANH_MODE>(r, bias_c + n * (512 + np3) + q * 128 + g * 32, pk, a.error_flag);
               }
               ptx::tmem_st16(lane_base + kT5A1 + 128u * n + 64u * q + (uint32_t)g * 16u, pk);
               ptx::tmem_st_wait();
@@ -402,7 +388,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc5_kernel(CouplingArg
                 uint32_t r[32];
                 ptx::tmem_ld32(sc + (uint32_t)g * 32u, r);
                 ptx::tmem_ld_wait();
-                t2_act_pack32<1, TANH_MODE>(r, bias_c + n * (512 + np3) + 256 + j * 128 + g * 32, pk, a.error_flag);
+                t2_act_pack<1, TANH_MODE>(r, bias_c + n * (512 + np3) + 256 + j * 128 + g * 32, pk, a.error_flag);
               }
               t2_quad_bar(quad);
               ptx::tmem_st16(sc + (uint32_t)g * 16u, pk);
@@ -455,54 +441,15 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc5_kernel(CouplingArg
           t2_epi_bar();
         }
         // ---- component log-density for this row ----
-        float q = 0.f;
-        if (md.base == GBNF_BASE_STD_NORMAL) {
-          for (int p = h0col; p < h1col; ++p) { const float d = zrow[p]; q = fmaf(d * d, 0.5f, q); }
-        } else {
-          const float* bm = a.fblob + base_off;
-          const float* bi = bm + Dv;
-          for (int p = h0col; p < h1col; ++p) { const float d = zrow[p] - __ldg(bm + p); q = fmaf(d * d, __ldg(bi + p), q); }
-        }
-        if (g > 0) { part[(g - 1) * kTcRows + row] = q; part2[(g - 1) * kTcRows + row] = lsum; }
-        t2_quad_bar(quad);
-        if (g == 0) {
-          q += part[row] + part[kTcRows + row] + part[2 * kTcRows + row];
-          const float ldj_tot = (lsum + part2[row] + part2[kTcRows + row] + part2[2 * kTcRows + row]) + cconst.x;
-          const float lq = (cconst.y - q) + ldj_tot;
-          if (gr < a.B) {
-            if (a.logq) a.logq[gr * a.ld_logq + (c - a.c0)] = lq;
-            for (int qq = 0; qq < a.n_peers; ++qq) a.logq_peers[qq][(long long)(a.peer_col0 + (c - a.c0)) * a.peer_ld + gr] = lq;
-            if (a.ldj_out) a.ldj_out[gr] = ldj_tot;
-          }
-          if (a.G_ll != nullptr && c < a.n_mix) __stcg(a.lse_terms + ((long long)tile * kTcRows + row) * a.n_mix + c, misc->coef[c] + lq);
-        }
+        t2_component_logq(a, zrow, lsum, part_s, row, g, quad, h0col, h1col, Dv, base_off, cconst.x, cconst.y, misc->coef, c, tile,
+                          true);
         if (a.z_out != nullptr && gr < a.B) {
           const int* sig = a.iblob + __ldg(&cdp->sigma_off);
           for (int j = h0col; j < h1col; ++j) a.z_out[gr * D + j] = zrow[__ldg(sig + j)];
         }
         t2_epi_bar();                                  // partial sums / z rows are dead before the next component overwrites them
       }
-      if (a.G_ll != nullptr) {
-        bool last = true;
-        if (a.split > 1) {
-          if (g == 0) __threadfence();
-          t2_epi_bar();
-          if (et == 0) misc->last_flag = (atomicAdd(a.tile_ctr + tile, 1u) == (unsigned)(a.split - 1)) ? 1u : 0u;
-          t2_epi_bar();
-          last = misc->last_flag != 0u;
-          if (last && et == 0) a.tile_ctr[tile] = 0u;
-          if (last && g == 0) __threadfence();
-        }
-        if (last && g == 0 && gr < a.B) {
-          const float* tv = a.lse_terms + ((long long)tile * kTcRows + row) * a.n_mix;
-          float M = -INFINITY;
-          bool has_nan = false;
-          for (int i = 0; i < a.n_mix; ++i) { const float t = __ldcg(tv + i); M = fmaxf(M, t); has_nan |= (t != t); }
-          float S = 0.f;
-          for (int i = 0; i < a.n_mix; ++i) { const float t = __ldcg(tv + i); if (t != -INFINITY) S += expf(t - M); }
-          a.G_ll[gr] = has_nan ? __int_as_float(0x7fc00000) : (M == INFINITY || M == -INFINITY) ? M : M + logf(S);
-        }
-      }
+      if (a.G_ll != nullptr) t2_tile_logsumexp(a, tile, gr, g, et, &misc->last_flag);
     }
     ptx::tc_fence_before();
   }

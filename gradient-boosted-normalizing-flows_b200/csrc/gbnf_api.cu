@@ -315,6 +315,15 @@ int ensure_scan_workspace(gbnf_ctx* h, long long B) {
   return GBNF_OK;
 }
 
+// Launch arguments that come from the handle (packed model, status words); the caller fills in rows, components and outputs.
+CouplingArgs coupling_args(const gbnf_ctx* h) {
+  CouplingArgs a{};
+  a.steps = h->steps_d; a.comps = h->comps_d; a.fblob = h->fblob; a.iblob = h->iblob; a.wblob = h->wblob; a.md = h->md;
+  a.cc_off = h->cc_off;
+  a.error_flag = h->flags;
+  return a;
+}
+
 int launch_coupling(gbnf_ctx* h, const float* x, long long B, int c0, int c1, float* logq, int ld_logq, float* z_out,
                     float* ldj_out, const float* rho, int n_mix, int skip_c, int mix_mode, float* G_ll, cudaStream_t st,
                     bool to_peers = false, int peer_ld = 0, int peer_col0 = 0, bool terms_only = false) {
@@ -344,13 +353,10 @@ int launch_coupling(gbnf_ctx* h, const float* x, long long B, int c0, int c1, fl
     return launch_coupling(h, x, B, c1 - 1, c1, logq ? logq + (c1 - 1 - c0) : nullptr, ld_logq, nullptr, nullptr, rho, n_mix, skip_c, mix_mode,
                            G_ll, st, false, 0, 0, false);
   }
-  CouplingArgs a{};
+  CouplingArgs a = coupling_args(h);
   a.terms_only = terms_only ? 1 : 0;
   a.x = x; a.B = B; a.c0 = c0; a.c1 = c1; a.logq = logq; a.ld_logq = ld_logq; a.z_out = z_out; a.ldj_out = ldj_out;
   a.rho = rho; a.n_mix = n_mix; a.skip_c = skip_c; a.mix_mode = mix_mode; a.G_ll = G_ll;
-  a.steps = h->steps_d; a.comps = h->comps_d; a.fblob = h->fblob; a.iblob = h->iblob; a.wblob = h->wblob; a.md = h->md;
-  a.cc_off = h->cc_off;
-  a.error_flag = h->flags;
   if (to_peers) {
     a.n_peers = h->cv.world; a.peer_ld = peer_ld; a.peer_col0 = peer_col0;
     for (int q = 0; q < h->cv.world; ++q) a.logq_peers[q] = h->cv.gather[q] + (h->cv.epoch & 1u) * h->cv.gather_stride;
@@ -642,11 +648,9 @@ int gbnf_component_inverse(gbnf_handle h, const float* d_z, int64_t B, int32_t c
   constexpr long long kMaxRowsPerLaunch = 1LL << 22;
   for (long long r0 = 0; r0 < B; r0 += kMaxRowsPerLaunch) {
     const long long nb = std::min(kMaxRowsPerLaunch, (long long)B - r0);
-    CouplingArgs a{};
+    CouplingArgs a = coupling_args(h);
     a.x = d_z + r0 * h->md.D; a.B = nb; a.c0 = c; a.c1 = c + 1; a.z_out = d_x + r0 * h->md.D; a.ldj_out = d_ldj_opt ? d_ldj_opt + r0 : nullptr;
     a.n_mix = 0; a.skip_c = -1;
-    a.steps = h->steps_d; a.comps = h->comps_d; a.fblob = h->fblob; a.iblob = h->iblob; a.wblob = h->wblob; a.md = h->md;
-    a.cc_off = h->cc_off; a.error_flag = h->flags; a.prof = nullptr;
     const int R = h->rows_per_cta;
     a.num_tiles = (int)((nb + R - 1) / R);
     a.split = 1; a.comps_per_unit = 1; a.num_units = a.num_tiles;
