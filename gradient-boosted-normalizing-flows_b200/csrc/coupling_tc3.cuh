@@ -153,8 +153,12 @@ __device__ __forceinline__ void t3_act_pack32_add(const uint32_t (&r)[32], const
 // [2] wait a0r + a1r, [3] wait slot B, [4] wait packed piece, [5] passes; [8] epilogue (thread 0) total, [9] wait l1f, [10] wait l2own,
 // [11] wait xfull, [12] wait l2ship, [13] wait xfree, [14] wait l3f, [15] wait x3full, [19] gather, [20] layer-1 epilogues,
 // [21] own epilogues, [22] ship epilogues, [23] transform + end-of-pass barrier; [16] producer total, [17] wait empty.
+// INV: 1 = inverse direction (sampling), the contract of coupling_tc2_kernel's INV: a.x = z in the flow's output column order,
+// ONE component (c0), steps walked from the last to the first by all three roles (the ring and barrier phases stay in step);
+// the gather and the coupling epilogue use the INVERSE gather-order tables; writes a.z_out = x and a.ldj_out = log-det of the
+// inverse map.  The exchange, the TMEM plan, the barriers and the weight image are those of the forward.
 #define T3_CLK() (PROF ? clock64() : 0LL)
-template <int TANH_MODE, int PROF = 0>
+template <int TANH_MODE, int PROF = 0, int INV = 0>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupling_tc3_kernel(CouplingArgs a, TcPlan plan) {
   extern __shared__ __align__(1024) unsigned char smem[];
   asm volatile(".reg .pred t3_p_full;" ::);
@@ -213,7 +217,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
     for (int u = pair; u < a.num_units; u += npairs) {
       const int cb = a.c0 + (u % a.split) * a.comps_per_unit, ce = min(a.c1, cb + a.comps_per_unit);
       for (int c = cb; c < ce; ++c)
-        for (int k = 0; k < md.K; ++k) {
+        for (int kk = 0; kk < md.K; ++kk) {
+          const int k = INV ? md.K - 1 - kk : kk;
           const StepDesc* sd = a.steps + (c * md.K + k);
           const int kp0 = __ldg(&sd->layer[0][0].Kp);
           const int np3 = __ldg(&sd->layer[0][2].Np);
@@ -225,7 +230,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
           // into L2 well ahead of the ring (256 KB within the step, the head of the next step at the start of this one).
           constexpr uint32_t kAhead = 262144;
           if (ptx::elect_one()) {
-            const StepDesc* sn = (k + 1 < md.K) ? sd + 1 : (c + 1 < ce) ? a.steps + (c + 1) * md.K : nullptr;
+            const StepDesc* sn = (kk + 1 < md.K) ? (INV ? sd - 1 : sd + 1)
+                               : (c + 1 < ce) ? a.steps + (c + 1) * md.K + (INV ? md.K - 1 : 0) : nullptr;
             if (sn != nullptr) {
               const int kpn = __ldg(&sn->layer[0][0].Kp), npn = __ldg(&sn->layer[0][2].Np);
               ptx::prefetch_l2(wb + __ldg(&sn->layer[0][0].w_off) + (size_t)p * kT3HH * kpn, (uint32_t)(kT3HH * kpn * 2));
@@ -293,7 +299,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
     for (int u = pair; u < a.num_units; u += npairs) {
       const int cb = a.c0 + (u % a.split) * a.comps_per_unit, ce = min(a.c1, cb + a.comps_per_unit);
       for (int c = cb; c < ce; ++c)
-        for (int k = 0; k < md.K; ++k, ++units) {
+        for (int kk = 0; kk < md.K; ++kk, ++units) {
+          const int k = INV ? md.K - 1 - kk : kk;
           const StepDesc* sd = a.steps + (c * md.K + k);
           const int k0s = __ldg(&sd->layer[0][0].Kp) >> 4;
           const int np3 = __ldg(&sd->layer[0][2].Np);
@@ -430,7 +437,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
       if (et < 128) ptx::cp_async16(bdst + 4 * et, b1 + 4 * et);
       else if (et < 256) { const int i = et - 128; const int m = i >> 5, w = i & 31; ptx::cp_async16(bdst + 512 + 128 * m + 4 * w, b2 + 128 * (2 * m + p) + 4 * w); }
       else if (et < 272) ptx::cp_async16(bdst + 1024 + 4 * (et - 256), b3 + 4 * (et - 256));
-      else if (et >= 384) { const int i = et - 384; ptx::cp_async16(tab_s + buf * (2 * kEpPad) + i, reinterpret_cast<const float4*>(a.fblob + __ldg(&sd->ep_off)) + i); }
+      else if (et >= 384) {
+        const int i = et - 384;
+        ptx::cp_async16(tab_s + buf * (2 * kEpPad) + i, reinterpret_cast<const float4*>(a.fblob + __ldg(&sd->ep_off)) + (INV ? 2 * kEpPad : 0) + i);
+      }
       if (et == 300) {
         int* m = misc->meta[buf];
         m[0] = __ldg(&sd->in_dim); m[1] = __ldg(&sd->out_dim); m[2] = __ldg(&sd->layer[0][0].Kp); m[3] = __ldg(&sd->layer[0][2].Np);
@@ -438,7 +448,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
     };
     if (pair < a.num_units) {
       const int cb0 = a.c0 + (pair % a.split) * a.comps_per_unit;
-      stage_pass(a.steps + cb0 * md.K, 0);
+      stage_pass(a.steps + cb0 * md.K + (INV ? md.K - 1 : 0), 0);
     }
     for (int u = pair; u < a.num_units; u += npairs) {
       const int tile = u / a.split, cs = u - tile * a.split;
@@ -452,6 +462,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
         const float ldj_const = cconst.x, base_const = cconst.y;
         t2_epi_bar();                                // previous component's readers are done with zs / part
         {                                            // x tile (L2-resident after the first component) -> this thread's share of zs
+          // INV: z arrives in the flow's OUTPUT column order, logical column j lives at physical column sigma[j]
+          const int* sig = INV ? a.iblob + __ldg(&cdp->sigma_off) : nullptr;
           const long long gbase = row0 * D;
           const long long glimit = a.B * (long long)D;
           const int total = kTcRows * D;
@@ -465,7 +477,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
 #pragma unroll
             for (int q = 0; q < 8; ++q) {
               const int i = i0 + q * kT3EpiThreads;
-              if (i < total) { const int r = i / D; zs[r * Dv + (i - r * D)] = v[q]; }
+              if (i < total) { const int r = i / D, j = i - r * D; zs[r * Dv + (INV ? __ldg(sig + j) : j)] = v[q]; }
             }
           }
           if (g == 0) for (int q = D; q < Dv; ++q) zrow[q] = 0.f;
@@ -473,7 +485,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
         ptx::cp_async_wait_all();
         t2_epi_bar();
         float lsum = 0.f;
-        for (int k = 0; k < md.K; ++k, ++units) {
+        for (int kk = 0; kk < md.K; ++kk, ++units) {
+          const int k = INV ? md.K - 1 - kk : kk;
           const StepDesc* sd = a.steps + (c * md.K + k);
           const int buf = units & 1u;
           const int* meta = misc->meta[buf];
@@ -482,14 +495,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
           const float4* tab2 = tab1 + kEpPad;
           const float* bias_c = bias_s + buf * kT3BiasFloats;
           const uint32_t upar = units & 1u;
-          const StepDesc* sd_next = (k + 1 < md.K) ? sd + 1
-                                    : (c + 1 < ce) ? a.steps + (c + 1) * md.K
-                                    : (u + npairs < a.num_units) ? a.steps + (a.c0 + ((u + npairs) % a.split) * a.comps_per_unit) * md.K
+          const int kfirst = INV ? md.K - 1 : 0;
+          const StepDesc* sd_next = (kk + 1 < md.K) ? (INV ? sd - 1 : sd + 1)
+                                    : (c + 1 < ce) ? a.steps + (c + 1) * md.K + kfirst
+                                    : (u + npairs < a.num_units) ? a.steps + (a.c0 + ((u + npairs) % a.split) * a.comps_per_unit) * md.K + kfirst
                                                                  : nullptr;
           const int act_kind = (md.act == GBNF_ACT_RELU) ? 2 : 1;
           // ---- ActNorm affine fused into the gather of z1 -> A0 (both CTAs build the same image) ----
           tq = T3_CLK();
-          t2_gather_z1(zrow, tab1, in_dim, meta[2] >> 3, g, row, A0, a.error_flag);
+          t2_gather_z1<INV>(zrow, tab1, in_dim, meta[2] >> 3, g, row, A0, a.error_flag);
           ptx::fence_proxy_async_smem();
           ptx::tc_fence_before();
           t2_warp_arrive(&misc->a0r, lane);
@@ -661,9 +675,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
                 const float shift = acc[2 * jj] + b.x;
                 const float raw = acc[2 * jj + 1] + b.y;
                 const float s = __fdividef(1.0f, 1.0f + __expf(-(raw + 2.0f)));      // sigmoid(raw + 2), glow.py:333
-                const float zn = (z[jj] + t[jj].x) * t[jj].y + t[jj].z;
-                z[jj] = (zn + shift) * s;                                             // glow.py:334-335
-                lsum += (j < out_dim) ? __logf(s) : 0.f;                              // glow.py:338
+                if (INV) {
+                  const float y = __fdividef(z[jj], s) - shift;                       // glow.py:354-356
+                  z[jj] = (y + t[jj].x) * t[jj].y + t[jj].z;                          // ActNorm reverse, layers.py:505-518
+                  lsum -= (j < out_dim) ? __logf(s) : 0.f;                            // glow.py:357
+                } else {
+                  const float zn = (z[jj] + t[jj].x) * t[jj].y + t[jj].z;
+                  z[jj] = (zn + shift) * s;                                           // glow.py:334-335
+                  lsum += (j < out_dim) ? __logf(s) : 0.f;                            // glow.py:338
+                }
               }
 #pragma unroll
               for (int jj = 0; jj < 8; ++jj) if (g * 8 + jj < out_dim) zrow[__float_as_int(t[jj].w)] = z[jj];
@@ -679,8 +699,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
 #pragma unroll
                 for (int jj = 0; jj < 8; ++jj) {
                   const int j = c0 + half * 8 + jj;
-                  const float zn = (z[jj] + t[jj].x) * t[jj].y + t[jj].z;
-                  z[jj] = zn + (acc[half * 8 + jj] + bias[j]);                        // additive coupling, glow.py:328-329
+                  if (INV) {
+                    z[jj] = ((z[jj] - (acc[half * 8 + jj] + bias[j])) + t[jj].x) * t[jj].y + t[jj].z;   // glow.py:350, then ActNorm reverse
+                  } else {
+                    const float zn = (z[jj] + t[jj].x) * t[jj].y + t[jj].z;
+                    z[jj] = zn + (acc[half * 8 + jj] + bias[j]);                      // additive coupling, glow.py:328-329
+                  }
                 }
 #pragma unroll
                 for (int jj = 0; jj < 8; ++jj) if (c0 + half * 8 + jj < out_dim) zrow[__float_as_int(t[jj].w)] = z[jj];
@@ -694,11 +718,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
           e_c4 += T3_CLK() - tq;
         }
         // ---- component log-density for this row (both CTAs hold the same z; rank 0 writes) ----
-        t2_component_logq(a, zrow, lsum, part, row, g, quad, h0col, h1col, Dv, base_off, ldj_const, base_const, misc->coef, c, tile,
-                          p == 0);
+        t2_component_logq(a, zrow, lsum, part, row, g, quad, h0col, h1col, Dv, base_off, INV ? -ldj_const : ldj_const, base_const,
+                          misc->coef, c, tile, p == 0);
         if (p == 0 && a.z_out != nullptr && gr < a.B) {
-          const int* sig = a.iblob + __ldg(&cdp->sigma_off);
-          for (int j = h0col; j < h1col; ++j) a.z_out[gr * D + j] = zrow[__ldg(sig + j)];
+          if (INV) {   // physical == logical column order at the flow's input
+            for (int j = h0col; j < h1col; ++j) a.z_out[gr * D + j] = zrow[j];
+          } else {
+            const int* sig = a.iblob + __ldg(&cdp->sigma_off);
+            for (int j = h0col; j < h1col; ++j) a.z_out[gr * D + j] = zrow[__ldg(sig + j)];
+          }
         }
       }
       if (a.G_ll != nullptr && p == 0) t2_tile_logsumexp(a, tile, gr, g, et, &misc->last_flag);
@@ -724,6 +752,8 @@ inline cudaError_t tc3_configure() {
   cudaError_t e = cudaFuncSetAttribute(coupling_tc3_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(coupling_tc3_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(coupling_tc3_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(coupling_tc3_kernel<0, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(coupling_tc3_kernel<1, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   return e;
 }
 
@@ -748,6 +778,12 @@ inline int tc3_launch(const CouplingArgs& a, const TcPlan& p, int pairs, cudaStr
   if (prof) { coupling_tc3_kernel<0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p); return 0; }
   if (p.tanh_mode == 0) coupling_tc3_kernel<0><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
   else                  coupling_tc3_kernel<1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
+  return 0;
+}
+
+inline int tc3_launch_inverse(const CouplingArgs& a, const TcPlan& p, int pairs, cudaStream_t st) {
+  if (p.tanh_mode == 0) coupling_tc3_kernel<0, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
+  else                  coupling_tc3_kernel<1, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
   return 0;
 }
 

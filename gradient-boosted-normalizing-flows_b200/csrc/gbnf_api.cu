@@ -640,9 +640,10 @@ int gbnf_component_inverse(gbnf_handle h, const float* d_z, int64_t B, int32_t c
   if (h->cfg.glow_invconv && !h->inv_ok[c])
     return fail(GBNF_ERR_STATE, "inverse direction: component " + std::to_string(c) + " was packed without invconv_winv");
   const bool f16 = h->cfg.gemm_mode != GBNF_GEMM_FP32;
-  if (f16 && h->kernel != CouplingKernel::kPipelined)
-    return fail(GBNF_ERR_INVALID, "inverse direction: the f16 tensor-core modes serve it through the pipelined kernel only (hidden width a "
-                                  "multiple of 128 up to 512, depth 1); use GBNF_GEMM_FP32 for this configuration");
+  if (f16 && h->kernel == CouplingKernel::kSerial)
+    return fail(GBNF_ERR_INVALID, "inverse direction: the serial tensor-core kernel (hidden width not a multiple of 128, or depth > 1) "
+                                  "does not serve it; use GBNF_GEMM_FP32 for this configuration");
+  const bool pair = h->kernel == CouplingKernel::kPair;
   ENTER(h);
   cudaStream_t st = (cudaStream_t)stream;
   constexpr long long kMaxRowsPerLaunch = 1LL << 22;
@@ -654,12 +655,14 @@ int gbnf_component_inverse(gbnf_handle h, const float* d_z, int64_t B, int32_t c
     const int R = h->rows_per_cta;
     a.num_tiles = (int)((nb + R - 1) / R);
     a.split = 1; a.comps_per_unit = 1; a.num_units = a.num_tiles;
-    const int grid = std::min(a.num_tiles, h->num_sms);
-    h->last_grid = grid;
+    const int grid = std::min(a.num_tiles, pair ? h->tc3_pairs : h->num_sms);     // CTAs, or CTA pairs
+    h->last_grid = pair ? 2 * grid : grid;
     if (!f16) {
       if (R == 64) coupling_fp32_inverse_kernel<64><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
       else if (R == 32) coupling_fp32_inverse_kernel<32><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
       else coupling_fp32_inverse_kernel<16><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
+    } else if (pair) {
+      tc3_launch_inverse(a, h->tc, grid, st);
     } else {
       tc2_launch_inverse(a, h->tc, grid, st);
     }

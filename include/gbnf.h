@@ -150,7 +150,9 @@ int gbnf_component_logq(gbnf_handle h, const float* d_x, int64_t B, int32_t c0, 
  * models/realnvp.py:97-113 (upstream's RealNVP decode pairs the wrong halves and its 1-D affine Glow decode raises; this is
  * the mathematical inverse, pinned by decode(encode(x)) == x and by the reference's additive-Glow decode).
  * d_z [B, D] in the flow's output column order, d_x [B, D]; d_ldj_opt [B] (may be NULL) receives the log-det of the
- * inverse map (= -log_det_j of the forward map at x). */
+ * inverse map (= -log_det_j of the forward map at x).  Served in GBNF_GEMM_FP32 and, in the f16 tensor-core modes, by the
+ * pipelined kernel (hidden width a multiple of 128 up to 512, depth 1) and the CTA-pair kernel (Glow, h = 1024); handles
+ * that run the serial tensor-core kernel return GBNF_ERR_INVALID. */
 int gbnf_component_inverse(gbnf_handle h, const float* d_z, int64_t B, int32_t c, float* d_x, float* d_ldj_opt, void* stream);
 
 /* Mixture log-density from materialised per-component log q (d_logq is [B, ld], first n_comp columns used):
