@@ -54,7 +54,10 @@ constexpr uint32_t kTcMiscBytes = 5120;   // >= sizeof(TcMisc), sizeof(Tc2Misc)
 static_assert(sizeof(TcMisc) <= kTcMiscBytes, "misc region too small");
 
 inline bool tc_make_plan(const ModelDims& md, const std::vector<StepDesc>& steps, TcPlan* p, std::string* why) {
-  if (md.h % 64 != 0 || md.h > 512) { *why = "hidden width must be a multiple of 64 and <= 512 (use GBNF_GEMM_FP32 otherwise)"; return false; }
+  if (md.h % 64 != 0 || md.h > 512) {
+    *why = "hidden width must be <= 512, or <= 1024 with coupling_network_depth 1 and D <= 64 (use GBNF_GEMM_FP32 otherwise)";
+    return false;
+  }
   if (md.D > kTcMaxD) { *why = "D must be <= 64"; return false; }
   int k0p = 16, out_max = 1;
   for (const StepDesc& s : steps) {

@@ -157,8 +157,9 @@ __device__ __forceinline__ void t2_load_x_tile(float* xs, const CouplingArgs& a,
 
 // ActNorm / eval-BatchNorm affine fused into the gather of z1 -> A0 (fp16, canonical layout, zero padded): this thread's
 // 8-element chunks g, g + 4, ... of nch.  Forward: the row keeps the normalised value.  INV: the MLP input is z1 as it
-// stands and the row keeps the un-normalised value (inverse tables).
-template <int INV = 0>
+// stands and the row keeps the un-normalised value (inverse tables).  FEED: the MLP input is z1 as it stands and the row is
+// left untouched (a second network on the same z1, coupling_tc3.cuh).
+template <int INV = 0, int FEED = 0>
 __device__ __forceinline__ void t2_gather_z1(float* zrow, const float4* tab1, int in_dim, int nch, int g, int row,
                                              unsigned char* A0, int* status) {
   for (int ch = g; ch < nch; ch += 4) {
@@ -170,7 +171,9 @@ __device__ __forceinline__ void t2_gather_z1(float* zrow, const float4* tab1, in
     for (int e = 0; e < 8; ++e) t[e] = tab1[ch * 8 + e];
 #pragma unroll
     for (int e = 0; e < 8; ++e) v[e] = zrow[__float_as_int(t[e].w)];
-    if (INV) {
+    if (FEED) {
+      // the row keeps its values
+    } else if (INV) {
 #pragma unroll
       for (int e = 0; e < 8; ++e) if (ch * 8 + e < in_dim) zrow[__float_as_int(t[e].w)] = (v[e] + t[e].x) * t[e].y + t[e].z;
     } else {

@@ -26,6 +26,12 @@
 //   2 m + 1 - p, then the own chunk 2 m + p [32 k-slabs][128 x 16] | last-layer pieces [8 k-slabs][Np3 x 16] per own chunk.
 //
 // Warp roles as in coupling_tc2.cuh: warp 0 = TMA producer, warp 1 = MMA issuer, warps 2..17 = epilogue (four threads per row).
+//
+// RealNVP (RNVP = 1): a step is TWO coupling passes on the same z1, one per network, each with the schedule, exchange and weight
+// stream of a Glow step (the image is laid out per (step, net, layer)).  The pass order needs no buffer for the shift (shared
+// memory is nearly exhausted): forward s then t (z2 = BN(z2) * exp(s), then z2 += t), inverse t then s (z2 -= t, then
+// z2 = BN^-1(z2 * exp(-s))).  A0 aliases the staging buffer, so the second pass gathers z1 again; only the pass of the s network
+// applies the BatchNorm tables (t3_net).  The per-pass code is one copy with the network as a runtime index.
 #pragma once
 #include "coupling_tc2.cuh"
 
@@ -66,10 +72,11 @@ constexpr uint32_t kT3MiscBytes = 1536;
 static_assert(sizeof(Tc3Misc) <= kT3MiscBytes, "misc region too small");
 
 inline bool tc3_eligible(const ModelDims& md, const std::vector<StepDesc>& steps) {
-  if (md.kind != GBNF_KIND_GLOW || md.nnets != 1 || md.nlayers != 3 || md.h != kT3H || md.D > kTcMaxD) return false;
-  if (md.act == GBNF_ACT_MIXED) return false;
+  if (md.nlayers != 3 || md.h != kT3H || md.D > kTcMaxD) return false;
+  if (md.kind == GBNF_KIND_GLOW ? (md.nnets != 1 || md.act == GBNF_ACT_MIXED) : md.nnets != 2) return false;
   for (const StepDesc& s : steps)
-    if (s.layer[0][0].Kp > 32 || s.layer[0][2].Np > 64) return false;
+    for (int n = 0; n < md.nnets; ++n)
+      if (s.layer[n][0].Kp > 32 || s.layer[n][2].Np > 64) return false;
   return true;
 }
 
@@ -121,6 +128,10 @@ __device__ __forceinline__ void t3_schedule(int p, F&& f) {
   f(T3_OP_L3, 3, 0);
 }
 
+// Network of pass i (0, 1) of a step: Glow has one pass (net 0); RealNVP runs net 1 (s) first forward, net 0 (t) first inverse.
+template <int RNVP, int INV>
+__device__ __forceinline__ int t3_net(int i) { return RNVP ? (INV ? i : 1 - i) : 0; }
+
 template <int ACT, int TANH_MODE>
 __device__ __forceinline__ void t3_act_pack32_add(const uint32_t (&r)[32], const float4* __restrict__ xb, const float* __restrict__ bias,
                                                   uint32_t* p, int* status) {
@@ -157,9 +168,11 @@ __device__ __forceinline__ void t3_act_pack32_add(const uint32_t (&r)[32], const
 // ONE component (c0), steps walked from the last to the first by all three roles (the ring and barrier phases stay in step);
 // the gather and the coupling epilogue use the INVERSE gather-order tables; writes a.z_out = x and a.ldj_out = log-det of the
 // inverse map.  The exchange, the TMEM plan, the barriers and the weight image are those of the forward.
+// RNVP: 1 = RealNVP components (two passes per step, see the header), 0 = Glow.
 #define T3_CLK() (PROF ? clock64() : 0LL)
-template <int TANH_MODE, int PROF = 0, int INV = 0>
+template <int TANH_MODE, int PROF = 0, int INV = 0, int RNVP = 0>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupling_tc3_kernel(CouplingArgs a, TcPlan plan) {
+  constexpr int kPasses = RNVP ? 2 : 1;              // coupling passes per step
   extern __shared__ __align__(1024) unsigned char smem[];
   asm volatile(".reg .pred t3_p_full;" ::);
   const ModelDims& md = a.md;
@@ -217,26 +230,29 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
     for (int u = pair; u < a.num_units; u += npairs) {
       const int cb = a.c0 + (u % a.split) * a.comps_per_unit, ce = min(a.c1, cb + a.comps_per_unit);
       for (int c = cb; c < ce; ++c)
-        for (int kk = 0; kk < md.K; ++kk) {
+        for (int pi = 0; pi < md.K * kPasses; ++pi) {
+          const int kk = RNVP ? pi >> 1 : pi, net = t3_net<RNVP, INV>(pi & 1);
           const int k = INV ? md.K - 1 - kk : kk;
           const StepDesc* sd = a.steps + (c * md.K + k);
-          const int kp0 = __ldg(&sd->layer[0][0].Kp);
-          const int np3 = __ldg(&sd->layer[0][2].Np);
-          const __half* w1 = wb + __ldg(&sd->layer[0][0].w_off) + (size_t)p * kT3HH * kp0;
-          const __half* w2 = wb + __ldg(&sd->layer[0][1].w_off) + (size_t)p * kT3H * kT3HH;
-          const __half* w3 = wb + __ldg(&sd->layer[0][2].w_off) + (size_t)p * np3 * kT3HH;
+          const int kp0 = __ldg(&sd->layer[net][0].Kp);
+          const int np3 = __ldg(&sd->layer[net][2].Np);
+          const __half* w1 = wb + __ldg(&sd->layer[net][0].w_off) + (size_t)p * kT3HH * kp0;
+          const __half* w2 = wb + __ldg(&sd->layer[net][1].w_off) + (size_t)p * kT3H * kT3HH;
+          const __half* w3 = wb + __ldg(&sd->layer[net][2].w_off) + (size_t)p * np3 * kT3HH;
           // The packed weights of this configuration (184 MB at cfg5) do not fit in L2 and every CTA pair reaches a step at about
           // the same time, so without help each ring stage's first touch is an HBM miss that ALL pairs wait for: pull the stream
-          // into L2 well ahead of the ring (256 KB within the step, the head of the next step at the start of this one).
+          // into L2 well ahead of the ring (256 KB within the pass, the head of the next pass at the start of this one).
           constexpr uint32_t kAhead = 262144;
           if (ptx::elect_one()) {
-            const StepDesc* sn = (kk + 1 < md.K) ? (INV ? sd - 1 : sd + 1)
+            const bool same = RNVP && (pi & 1) == 0;     // the step's second pass is next
+            const int nn = t3_net<RNVP, INV>(same ? 1 : 0);
+            const StepDesc* sn = same ? sd : (kk + 1 < md.K) ? (INV ? sd - 1 : sd + 1)
                                : (c + 1 < ce) ? a.steps + (c + 1) * md.K + (INV ? md.K - 1 : 0) : nullptr;
             if (sn != nullptr) {
-              const int kpn = __ldg(&sn->layer[0][0].Kp), npn = __ldg(&sn->layer[0][2].Np);
-              ptx::prefetch_l2(wb + __ldg(&sn->layer[0][0].w_off) + (size_t)p * kT3HH * kpn, (uint32_t)(kT3HH * kpn * 2));
-              ptx::prefetch_l2(wb + __ldg(&sn->layer[0][1].w_off) + (size_t)p * kT3H * kT3HH, kAhead);
-              ptx::prefetch_l2(wb + __ldg(&sn->layer[0][2].w_off) + (size_t)p * npn * kT3HH, (uint32_t)(npn * kT3HH * 2));
+              const int kpn = __ldg(&sn->layer[nn][0].Kp), npn = __ldg(&sn->layer[nn][2].Np);
+              ptx::prefetch_l2(wb + __ldg(&sn->layer[nn][0].w_off) + (size_t)p * kT3HH * kpn, (uint32_t)(kT3HH * kpn * 2));
+              ptx::prefetch_l2(wb + __ldg(&sn->layer[nn][1].w_off) + (size_t)p * kT3H * kT3HH, kAhead);
+              ptx::prefetch_l2(wb + __ldg(&sn->layer[nn][2].w_off) + (size_t)p * npn * kT3HH, (uint32_t)(npn * kT3HH * 2));
             }
           }
           __syncwarp();
@@ -299,11 +315,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
     for (int u = pair; u < a.num_units; u += npairs) {
       const int cb = a.c0 + (u % a.split) * a.comps_per_unit, ce = min(a.c1, cb + a.comps_per_unit);
       for (int c = cb; c < ce; ++c)
-        for (int kk = 0; kk < md.K; ++kk, ++units) {
+        for (int pi = 0; pi < md.K * kPasses; ++pi, ++units) {
+          const int kk = RNVP ? pi >> 1 : pi, net = t3_net<RNVP, INV>(pi & 1);
           const int k = INV ? md.K - 1 - kk : kk;
           const StepDesc* sd = a.steps + (c * md.K + k);
-          const int k0s = __ldg(&sd->layer[0][0].Kp) >> 4;
-          const int np3 = __ldg(&sd->layer[0][2].Np);
+          const int k0s = __ldg(&sd->layer[net][0].Kp) >> 4;
+          const int np3 = __ldg(&sd->layer[net][2].Np);
           const uint32_t idesc_o = ptx::make_idesc_f16(128, np3);
           const uint32_t b3_step = (uint32_t)np3 * 2u;
           const uint32_t upar = units & 1u;
@@ -428,12 +445,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive_remote_relaxed(bar_cluster_addr);
     };
-    // staging of one pass's constants: biases (b1 own half | b2 own chunks | b3), gather-order tables, scalars
-    auto stage_pass = [&](const StepDesc* sd, int buf) {
+    // staging of one pass's constants: biases of network `net` (b1 own half | b2 own chunks | b3), gather-order tables, scalars
+    auto stage_pass = [&](const StepDesc* sd, int net, int buf) {
       float* bdst = bias_s + buf * kT3BiasFloats;
-      const float* b1 = a.fblob + __ldg(&sd->layer[0][0].b_off) + p * kT3HH;
-      const float* b2 = a.fblob + __ldg(&sd->layer[0][1].b_off);
-      const float* b3 = a.fblob + __ldg(&sd->layer[0][2].b_off);
+      const float* b1 = a.fblob + __ldg(&sd->layer[net][0].b_off) + p * kT3HH;
+      const float* b2 = a.fblob + __ldg(&sd->layer[net][1].b_off);
+      const float* b3 = a.fblob + __ldg(&sd->layer[net][2].b_off);
       if (et < 128) ptx::cp_async16(bdst + 4 * et, b1 + 4 * et);
       else if (et < 256) { const int i = et - 128; const int m = i >> 5, w = i & 31; ptx::cp_async16(bdst + 512 + 128 * m + 4 * w, b2 + 128 * (2 * m + p) + 4 * w); }
       else if (et < 272) ptx::cp_async16(bdst + 1024 + 4 * (et - 256), b3 + 4 * (et - 256));
@@ -443,12 +460,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
       }
       if (et == 300) {
         int* m = misc->meta[buf];
-        m[0] = __ldg(&sd->in_dim); m[1] = __ldg(&sd->out_dim); m[2] = __ldg(&sd->layer[0][0].Kp); m[3] = __ldg(&sd->layer[0][2].Np);
+        m[0] = __ldg(&sd->in_dim); m[1] = __ldg(&sd->out_dim); m[2] = __ldg(&sd->layer[net][0].Kp); m[3] = __ldg(&sd->layer[net][2].Np);
       }
     };
     if (pair < a.num_units) {
       const int cb0 = a.c0 + (pair % a.split) * a.comps_per_unit;
-      stage_pass(a.steps + cb0 * md.K + (INV ? md.K - 1 : 0), 0);
+      stage_pass(a.steps + cb0 * md.K + (INV ? md.K - 1 : 0), t3_net<RNVP, INV>(0), 0);
     }
     for (int u = pair; u < a.num_units; u += npairs) {
       const int tile = u / a.split, cs = u - tile * a.split;
@@ -485,7 +502,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
         ptx::cp_async_wait_all();
         t2_epi_bar();
         float lsum = 0.f;
-        for (int kk = 0; kk < md.K; ++kk, ++units) {
+        for (int pi = 0; pi < md.K * kPasses; ++pi, ++units) {
+          const int kk = RNVP ? pi >> 1 : pi, net = t3_net<RNVP, INV>(pi & 1);
           const int k = INV ? md.K - 1 - kk : kk;
           const StepDesc* sd = a.steps + (c * md.K + k);
           const int buf = units & 1u;
@@ -496,14 +514,18 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
           const float* bias_c = bias_s + buf * kT3BiasFloats;
           const uint32_t upar = units & 1u;
           const int kfirst = INV ? md.K - 1 : 0;
-          const StepDesc* sd_next = (kk + 1 < md.K) ? (INV ? sd - 1 : sd + 1)
+          const bool same = RNVP && (pi & 1) == 0;     // the step's second pass is next
+          const StepDesc* sd_next = same ? sd : (kk + 1 < md.K) ? (INV ? sd - 1 : sd + 1)
                                     : (c + 1 < ce) ? a.steps + (c + 1) * md.K + kfirst
                                     : (u + npairs < a.num_units) ? a.steps + (a.c0 + ((u + npairs) % a.split) * a.comps_per_unit) * md.K + kfirst
                                                                  : nullptr;
-          const int act_kind = (md.act == GBNF_ACT_RELU) ? 2 : 1;
-          // ---- ActNorm affine fused into the gather of z1 -> A0 (both CTAs build the same image) ----
+          // mixed RealNVP networks: t = ReLU, s = tanh (as in coupling_tc2.cuh)
+          const int act_kind = (md.act == GBNF_ACT_RELU || (RNVP && md.act == GBNF_ACT_MIXED && net == 0)) ? 2 : 1;
+          // ---- ActNorm / eval-BatchNorm affine fused into the gather of z1 -> A0 (both CTAs build the same image); the RealNVP
+          //      t pass feeds z1 as the s pass of the step leaves it (forward) or finds it (inverse) ----
           tq = T3_CLK();
-          t2_gather_z1<INV>(zrow, tab1, in_dim, meta[2] >> 3, g, row, A0, a.error_flag);
+          if (RNVP && net == 0) t2_gather_z1<0, 1>(zrow, tab1, in_dim, meta[2] >> 3, g, row, A0, a.error_flag);
+          else                  t2_gather_z1<INV>(zrow, tab1, in_dim, meta[2] >> 3, g, row, A0, a.error_flag);
           ptx::fence_proxy_async_smem();
           ptx::tc_fence_before();
           t2_warp_arrive(&misc->a0r, lane);
@@ -532,7 +554,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
             e_c1 += T3_CLK() - tq;
           }
           // the next pass's constants (other buffer: its last readers finished a pass ago)
-          if (sd_next != nullptr) stage_pass(sd_next, buf ^ 1);
+          if (sd_next != nullptr) stage_pass(sd_next, t3_net<RNVP, INV>(same ? 1 : 0), buf ^ 1);
           // ---- layer 2: per chunk pair m -- [read out the previous own chunk's last-layer product] -> the two shipped halves
           //      (their MMAs ran under the previous own epilogue) -> my own chunk ----
           const int c0 = g * 16;
@@ -660,7 +682,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
               acc[4 * i + 3] = acc3[4 * i + 3] + o.w;
             }
             const float* bias = bias_c + 1024;
-            if (md.coupling == GBNF_COUPLING_AFFINE) {
+            if (!RNVP && md.coupling == GBNF_COUPLING_AFFINE) {
               const float2* bias2 = reinterpret_cast<const float2*>(bias);
               float4 t[8];
               float z[8];
@@ -699,7 +721,20 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
 #pragma unroll
                 for (int jj = 0; jj < 8; ++jj) {
                   const int j = c0 + half * 8 + jj;
-                  if (INV) {
+                  if (RNVP) {                                                       // transformations.py:575-577
+                    const float v = acc[half * 8 + jj] + bias[j];
+                    if (net == 0) {                                                 // t_net: shift
+                      z[jj] = INV ? z[jj] - v : z[jj] + v;
+                    } else if (INV) {                                               // s_net: scale, then eval-BatchNorm inverse
+                      const float y = z[jj] * __expf(-v);
+                      z[jj] = (y + t[jj].x) * t[jj].y + t[jj].z;
+                      lsum -= (j < out_dim) ? v : 0.f;
+                    } else {                                                        // eval-BatchNorm, then s_net: scale
+                      const float zn = (z[jj] + t[jj].x) * t[jj].y + t[jj].z;
+                      z[jj] = zn * __expf(v);
+                      lsum += (j < out_dim) ? v : 0.f;
+                    }
+                  } else if (INV) {
                     z[jj] = ((z[jj] - (acc[half * 8 + jj] + bias[j])) + t[jj].x) * t[jj].y + t[jj].z;   // glow.py:350, then ActNorm reverse
                   } else {
                     const float zn = (z[jj] + t[jj].x) * t[jj].y + t[jj].z;
@@ -754,6 +789,10 @@ inline cudaError_t tc3_configure() {
   if (e == cudaSuccess) e = cudaFuncSetAttribute(coupling_tc3_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(coupling_tc3_kernel<0, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(coupling_tc3_kernel<1, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(coupling_tc3_kernel<0, 0, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(coupling_tc3_kernel<1, 0, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(coupling_tc3_kernel<0, 0, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(coupling_tc3_kernel<1, 0, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   return e;
 }
 
@@ -773,8 +812,14 @@ inline int tc3_max_pairs(const TcPlan& p, int num_sms) {
   return std::min(n, num_sms / 2);
 }
 
-// grid = 2 x (CTA pairs): the cluster dimension is a compile-time attribute of the kernel
+// grid = 2 x (CTA pairs): the cluster dimension is a compile-time attribute of the kernel.  The cycle-counter build exists for
+// Glow only: a profiling RealNVP handle runs the production kernel.
 inline int tc3_launch(const CouplingArgs& a, const TcPlan& p, int pairs, cudaStream_t st, int prof = 0) {
+  if (a.md.nnets == 2) {
+    if (p.tanh_mode == 0) coupling_tc3_kernel<0, 0, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
+    else                  coupling_tc3_kernel<1, 0, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
+    return 0;
+  }
   if (prof) { coupling_tc3_kernel<0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p); return 0; }
   if (p.tanh_mode == 0) coupling_tc3_kernel<0><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
   else                  coupling_tc3_kernel<1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
@@ -782,6 +827,11 @@ inline int tc3_launch(const CouplingArgs& a, const TcPlan& p, int pairs, cudaStr
 }
 
 inline int tc3_launch_inverse(const CouplingArgs& a, const TcPlan& p, int pairs, cudaStream_t st) {
+  if (a.md.nnets == 2) {
+    if (p.tanh_mode == 0) coupling_tc3_kernel<0, 0, 1, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
+    else                  coupling_tc3_kernel<1, 0, 1, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
+    return 0;
+  }
   if (p.tanh_mode == 0) coupling_tc3_kernel<0, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
   else                  coupling_tc3_kernel<1, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
   return 0;

@@ -56,7 +56,7 @@ inline long long round_up_ll(long long v, long long m) { return (v + m - 1) / m 
 }  // namespace
 
 // The coupling kernel a handle plans for its shape: fp32 (coupling_fp32.cuh), serial (coupling_tc.cuh), pipelined
-// (coupling_tc2.cuh) or CTA pair for h = 1024 (coupling_tc3.cuh).
+// (coupling_tc2.cuh) or CTA pair for h = 1024 (coupling_tc3.cuh), at the padded width of plan_layout.
 enum class CouplingKernel { kFp32, kSerial, kPipelined, kPair };
 // A shape-specific kernel a launch of a pipelined plan may take instead (the values are gbnf_info::two_chain): the two-chain
 // schedule for Glow / affine / tanh at h = 512 (coupling_tc4.cuh) or the interleaved s / t networks for RealNVP / tanh at h = 256
@@ -198,6 +198,14 @@ int plan_layout(gbnf_ctx* h) {
   const bool f16 = (c.gemm_mode != GBNF_GEMM_FP32);
   const int kq = f16 ? 16 : kF32KT, nq = f16 ? 16 : kF32NT;
   const int h0 = c.D / 2, h1 = c.D - h0;
+  // f16: the tensor-core kernels run the hidden width padded to a width they serve.  A padded hidden unit has zero weights
+  // and a zero bias, so it computes act(0) = 0 exactly and meets zero weights in the next layer: the results are those of
+  // the true width, bit for bit.  md.h = h_pad is the geometry every tensor-core plan and kernel reads; the hidden layers'
+  // K_in / N_out keep the true width (the raw row stride and the zero-fill bound of the pack).
+  int h_pad = c.h;
+  if (f16 && c.h % 64 != 0 && c.h <= 512) h_pad = (c.depth == 1) ? round_up(c.h, kT2Chunk) : round_up(c.h, 64);
+  else if (f16 && c.depth == 1 && c.h > 512 && c.h <= kT3H) h_pad = kT3H;
+  md.h = h_pad;
   long long f = 0, i = 0, w = 0;   // running offsets (floats / ints / weight elements)
   h->steps_h.assign((size_t)c.C * c.K, StepDesc{});
   h->comps_h.assign((size_t)c.C, CompDesc{});
@@ -231,9 +239,8 @@ int plan_layout(gbnf_ctx* h) {
           LayerDesc& L = sd.layer[net][l];
           L.K_in = (l == 0) ? sd.in_dim : c.h;
           L.N_out = (l == md.nlayers - 1) ? n_last : c.h;
-          L.Kp = round_up(L.K_in, kq);
-          L.Np = round_up(L.N_out, nq);
-          if (!f16 && l > 0) L.Kp = round_up(c.h, kF32KT);
+          L.Kp = (l == 0) ? round_up(L.K_in, kq) : f16 ? h_pad : round_up(c.h, kF32KT);
+          L.Np = (l == md.nlayers - 1) ? round_up(L.N_out, nq) : f16 ? h_pad : round_up(c.h, nq);
           L.NC = L.Np; L.NC2 = 0;
           L.w_off = w; w += (long long)L.Kp * L.Np;
           L.b_off = f; f += round_up_ll(L.Np, 4);
@@ -641,7 +648,7 @@ int gbnf_component_inverse(gbnf_handle h, const float* d_z, int64_t B, int32_t c
     return fail(GBNF_ERR_STATE, "inverse direction: component " + std::to_string(c) + " was packed without invconv_winv");
   const bool f16 = h->cfg.gemm_mode != GBNF_GEMM_FP32;
   if (f16 && h->kernel == CouplingKernel::kSerial)
-    return fail(GBNF_ERR_INVALID, "inverse direction: the serial tensor-core kernel (hidden width not a multiple of 128, or depth > 1) "
+    return fail(GBNF_ERR_INVALID, "inverse direction: the serial tensor-core kernel (hidden width 64, 192, 320 or 448, or depth > 1) "
                                   "does not serve it; use GBNF_GEMM_FP32 for this configuration");
   const bool pair = h->kernel == CouplingKernel::kPair;
   ENTER(h);

@@ -62,6 +62,10 @@ enum {
                            (abs err ~1e-7): <= 1e-4 rel on log q                                                   */
   GBNF_GEMM_F16_TC_FAST = 2 /* same GEMMs, tanh.approx.f32 (one MUFU op, rel err 2^-11): <= 2e-4 rel on log q      */
 };
+/* Hidden widths in the f16 modes: coupling_network_depth 1 serves any h <= 1024 (D <= 64), depth > 1 any h <= 512.  The
+ * kernels run the width padded with zero units (depth 1: h <= 512 to a multiple of 128 unless it is one of 64, h > 512 to
+ * 1024; depth > 1: to a multiple of 64), which gives the results of the true width bit for bit.  Wider networks, and
+ * depth > 1 above 512, need GBNF_GEMM_FP32. */
 enum { GBNF_WEIGHTS_DENSITY = 0, GBNF_WEIGHTS_TOY = 1 }; /* density_experiment.py:627-641 | toy_experiment.py:440-459 */
 enum {
   GBNF_MIX_SIMPLEX = 0,   /* logsumexp_c(log(rho_c / sum rho) + log q_c): density_experiment.py:612-622              */
@@ -151,8 +155,9 @@ int gbnf_component_logq(gbnf_handle h, const float* d_x, int64_t B, int32_t c0, 
  * the mathematical inverse, pinned by decode(encode(x)) == x and by the reference's additive-Glow decode).
  * d_z [B, D] in the flow's output column order, d_x [B, D]; d_ldj_opt [B] (may be NULL) receives the log-det of the
  * inverse map (= -log_det_j of the forward map at x).  Served in GBNF_GEMM_FP32 and, in the f16 tensor-core modes, by the
- * pipelined kernel (hidden width a multiple of 128 up to 512, depth 1) and the CTA-pair kernel (Glow, h = 1024); handles
- * that run the serial tensor-core kernel return GBNF_ERR_INVALID. */
+ * pipelined kernel (depth 1, hidden width up to 512 except 64, 192, 320 and 448) and the CTA-pair kernel (depth 1,
+ * 512 < h <= 1024, Glow and RealNVP); handles that run the serial tensor-core kernel (depth > 1, or h = 64 / 192 / 320 /
+ * 448) return GBNF_ERR_INVALID. */
 int gbnf_component_inverse(gbnf_handle h, const float* d_z, int64_t B, int32_t c, float* d_x, float* d_ldj_opt, void* stream);
 
 /* Mixture log-density from materialised per-component log q (d_logq is [B, ld], first n_comp columns used):
@@ -269,7 +274,7 @@ typedef struct {
   int32_t grid;            /* CTAs launched by the last coupling launch */
   int64_t packed_bytes;    /* size of the packed parameter blob */
   int64_t launches;        /* kernels launched through this handle so far */
-  int32_t pipelined;       /* 2: CTA-pair tensor-core kernel for h = 1024 (coupling_tc3.cuh), 1: chunk-pipelined tensor-core
+  int32_t pipelined;       /* 2: CTA-pair tensor-core kernel for 512 < h <= 1024 (coupling_tc3.cuh), 1: chunk-pipelined tensor-core
                               kernel (coupling_tc2.cuh), 0: serial tensor-core / fp32 kernel */
   int32_t two_chain;       /* 1: the last coupling launch ran the two-chain schedule (coupling_tc4.cuh: Glow / affine / tanh, h = 512,
                               an even number of components per work unit); 2: the interleaved s / t schedule (coupling_tc5.cuh:
