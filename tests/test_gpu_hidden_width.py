@@ -83,6 +83,9 @@ PAD_CASES = {
     "glow_h215_single_chain": ("glow", 43, 2, 2, 215, {}, 1, 0),
     "glow_h430_two_chain": ("glow", 43, 2, 2, 430, {}, 1, 1),
     "glow_depth2_h100_serial": ("glow", 10, 2, 2, 100, dict(depth=2), 0, 0),
+    "glow_depth0_h100_serial": ("glow", 21, 2, 2, 100, dict(depth=0), 0, 0),
+    "glow_depth2_h300_serial": ("glow", 43, 2, 2, 300, dict(depth=2), 0, 0),
+    "realnvp_bn_d64_depth3_h450_serial": ("realnvp", 64, 2, 2, 450, dict(depth=3, batch_norm=True), 0, 0),
     "glow_h600_pair": ("glow", 21, 2, 2, 600, {}, 2, 0),
     "glow_h630_pair": ("glow", 63, 2, 2, 630, {}, 2, 0),
     "realnvp_h600_pair": ("realnvp", 21, 2, 2, 600, dict(batch_norm=True), 2, 0),

@@ -64,6 +64,9 @@ INV_VARIANTS = {
     "realnvp_mixed_d5_h256": dict(kind="realnvp", D=5, C=3, K=4, h=256, act="mixed"),
     "realnvp_toy_d2_h128": dict(kind="realnvp", D=2, C=3, K=2, h=128, rho_init="uniform", toy_base=True),
     "glow_depth2_h64_fp32only": dict(kind="glow", D=10, C=2, K=2, h=64, depth=2),
+    "glow_depth0_h128_fp32only": dict(kind="glow", D=10, C=2, K=2, h=128, depth=0),
+    "realnvp_bn_depth3_h256_fp32only": dict(kind="realnvp", D=9, C=2, K=3, h=256, depth=3, batch_norm=True),
+    "glow_additive_depth4_h192_fp32only": dict(kind="glow", D=7, C=2, K=2, h=192, depth=4, coupling="additive"),
     "glow_h1024_fp32only": dict(kind="glow", D=12, C=1, K=2, h=1024),
 }
 
