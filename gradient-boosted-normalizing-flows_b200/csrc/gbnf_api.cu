@@ -331,6 +331,36 @@ CouplingArgs coupling_args(const gbnf_ctx* h) {
   return a;
 }
 
+// Work units of a coupling launch over `ncomp` components of `num_tiles` row tiles.  The pipelined kernels split every tile's
+// components over `split` units when that shortens the critical CTA (waves x components per unit); the other kernels run one
+// unit per tile.  The two-chain kernel pairs the two halves of a unit's components: every unit needs the same, even number of
+// them.  A pass of it takes ~0.8 of a single-chain pass, which the cost model weighs against the coarser units (GBNF_TC4=2:
+// always prefer it when a split allows it -- tests).
+struct UnitPlan { int split, comps_per_unit; bool two_chain; };
+UnitPlan plan_units(const gbnf_ctx* h, int num_tiles, int ncomp, bool z_out) {
+  UnitPlan p{1, ncomp, false};
+  const bool pair = h->kernel == CouplingKernel::kPair;
+  if (h->kernel != CouplingKernel::kPipelined && !pair) return p;
+  const int workers = pair ? h->tc3_pairs : h->num_sms;        // CTAs, or CTA pairs, that run concurrently
+  const bool tc4_ok = h->alt == AltKernel::kTwoChain && h->profiling != 2 && !z_out;
+  long long best = -1;
+  for (int S = 1; S <= ncomp; S *= 2) {
+    const int cpu = (ncomp + S - 1) / S;
+    const int units = num_tiles * ((ncomp + cpu - 1) / cpu);
+    const bool two = tc4_ok && cpu % 2 == 0 && ncomp % cpu == 0;
+    long long cost = (long long)((units + workers - 1) / workers) * cpu * (two ? 4 : 5);
+    if (h->tc4_force && !two) cost += 1LL << 40;
+    if (best < 0 || cost < best) { best = cost; p.comps_per_unit = cpu; p.split = (ncomp + cpu - 1) / cpu; p.two_chain = two; }
+  }
+  return p;
+}
+
+// GBNF_GRID=n caps the grid of a coupling launch at n CTAs, or n CTA pairs (diagnostics and tests: every CTA walks more units)
+int capped_grid(int grid) {
+  const char* ge = std::getenv("GBNF_GRID");
+  return (ge && std::atoi(ge) > 0) ? std::min(grid, std::atoi(ge)) : grid;
+}
+
 int launch_coupling(gbnf_ctx* h, const float* x, long long B, int c0, int c1, float* logq, int ld_logq, float* z_out,
                     float* ldj_out, const float* rho, int n_mix, int skip_c, int mix_mode, float* G_ll, cudaStream_t st,
                     bool to_peers = false, int peer_ld = 0, int peer_col0 = 0, bool terms_only = false) {
@@ -350,11 +380,15 @@ int launch_coupling(gbnf_ctx* h, const float* x, long long B, int c0, int c1, fl
     }
     return GBNF_OK;
   }
-  // An ODD number (>= 3) of components on a shape the two-chain kernel serves: the even part goes through it (mixture terms only),
-  // the last component through the single-chain kernel, whose last-unit reduce covers all n_mix terms (stream order makes the first
-  // launch's terms visible).  5 - 16 % faster than the single-chain kernel on all of them (training: the fixed mixture has
-  // 1 .. C - 1 components).
-  if (h->alt == AltKernel::kTwoChain && h->profiling == 0 && !terms_only && z_out == nullptr && ldj_out == nullptr && !to_peers && (c1 - c0) >= 3 && ((c1 - c0) & 1)) {
+  const int R = h->rows_per_cta;
+  const int num_tiles = (int)((B + R - 1) / R);
+  // An ODD number (>= 3) of components on a shape the two-chain kernel serves, when the cost model puts the even part on it: the
+  // even part goes through the two-chain kernel (mixture terms only), the last component through the single-chain kernel, whose
+  // last-unit reduce covers all n_mix terms (stream order makes the first launch's terms visible).  Faster than the single-chain
+  // kernel on all of them at training batches (the fixed mixture has 1 .. C - 1 components).  When the even part would run on
+  // the single chain anyway, one single-chain launch over all n computes the same bits: the reduce runs in component order.
+  if (h->alt == AltKernel::kTwoChain && h->profiling == 0 && !terms_only && z_out == nullptr && ldj_out == nullptr && !to_peers &&
+      (c1 - c0) >= 3 && ((c1 - c0) & 1) && plan_units(h, num_tiles, c1 - c0 - 1, false).two_chain) {
     int rc = launch_coupling(h, x, B, c0, c1 - 1, logq, ld_logq, nullptr, nullptr, rho, n_mix, skip_c, mix_mode, G_ll, st, false, 0, 0, true);
     if (rc != GBNF_OK) return rc;
     return launch_coupling(h, x, B, c1 - 1, c1, logq ? logq + (c1 - 1 - c0) : nullptr, ld_logq, nullptr, nullptr, rho, n_mix, skip_c, mix_mode,
@@ -369,31 +403,17 @@ int launch_coupling(gbnf_ctx* h, const float* x, long long B, int c0, int c1, fl
     for (int q = 0; q < h->cv.world; ++q) a.logq_peers[q] = h->cv.gather[q] + (h->cv.epoch & 1u) * h->cv.gather_stride;
   }
   a.prof = h->prof;
-  const int R = h->rows_per_cta;
-  a.num_tiles = (int)((B + R - 1) / R);
-  a.split = 1; a.comps_per_unit = c1 - c0; a.num_units = a.num_tiles;
+  a.num_tiles = num_tiles;
   const bool pair = h->kernel == CouplingKernel::kPair;
   const int workers = pair ? h->tc3_pairs : h->num_sms;        // CTAs, or CTA pairs, that run concurrently
   AltKernel alt = (h->alt == AltKernel::kInterleaved && h->profiling == 0) ? AltKernel::kInterleaved : AltKernel::kNone;
+  const UnitPlan up = plan_units(h, a.num_tiles, c1 - c0, z_out != nullptr);
+  a.split = up.split; a.comps_per_unit = up.comps_per_unit; a.num_units = a.num_tiles * a.split;
+  if (up.two_chain) alt = AltKernel::kTwoChain;
+  // only the two-chain kernel leaves the tile's logsumexp to a later launch; any other kernel would reduce terms not yet written
+  if (terms_only && alt != AltKernel::kTwoChain)
+    return fail(GBNF_ERR_INVALID, "internal: a mixture-terms-only coupling launch must run on the two-chain kernel");
   if (h->kernel == CouplingKernel::kPipelined || pair) {
-    // split every tile's components over S units when that shortens the critical CTA (waves x components per unit)
-    const int ncomp = c1 - c0;
-    long long best = -1;
-    // The two-chain kernel pairs the two halves of a unit's components: every unit needs the same, even number of them.  A pass
-    // of it takes ~0.8 of a single-chain pass, which the cost model weighs against the coarser units (GBNF_TC4=2: always
-    // prefer it when a split allows it -- tests).
-    const bool tc4_ok = h->alt == AltKernel::kTwoChain && h->profiling != 2 && z_out == nullptr;
-    bool best_two = false;
-    for (int S = 1; S <= ncomp; S *= 2) {
-      const int cpu = (ncomp + S - 1) / S;
-      const int units = a.num_tiles * ((ncomp + cpu - 1) / cpu);
-      const bool two = tc4_ok && cpu % 2 == 0 && ncomp % cpu == 0;
-      long long cost = (long long)((units + workers - 1) / workers) * cpu * (two ? 4 : 5);
-      if (h->tc4_force && !two) cost += 1LL << 40;
-      if (best < 0 || cost < best) { best = cost; a.comps_per_unit = cpu; a.split = (ncomp + cpu - 1) / cpu; best_two = two; }
-    }
-    if (best_two) alt = AltKernel::kTwoChain;
-    a.num_units = a.num_tiles * a.split;
     if (G_ll != nullptr) {
       const long long need = (long long)a.num_tiles * R * std::max(1, n_mix);
       if (need > h->lse_cap) {
@@ -413,8 +433,7 @@ int launch_coupling(gbnf_ctx* h, const float* x, long long B, int c0, int c1, fl
       a.lse_terms = h->lse_part; a.tile_ctr = h->tile_ctr;
     }
   }
-  int grid = std::min(a.num_units, workers);
-  { const char* ge = std::getenv("GBNF_GRID"); if (ge && std::atoi(ge) > 0) grid = std::min(grid, std::atoi(ge)); }   // diagnostics: fewer CTAs
+  const int grid = capped_grid(std::min(a.num_units, workers));
   h->last_grid = pair ? 2 * grid : grid;
   h->last_alt = alt;
   int rc = 0;
@@ -662,7 +681,7 @@ int gbnf_component_inverse(gbnf_handle h, const float* d_z, int64_t B, int32_t c
     const int R = h->rows_per_cta;
     a.num_tiles = (int)((nb + R - 1) / R);
     a.split = 1; a.comps_per_unit = 1; a.num_units = a.num_tiles;
-    const int grid = std::min(a.num_tiles, pair ? h->tc3_pairs : h->num_sms);     // CTAs, or CTA pairs
+    const int grid = capped_grid(std::min(a.num_tiles, pair ? h->tc3_pairs : h->num_sms));     // CTAs, or CTA pairs
     h->last_grid = pair ? 2 * grid : grid;
     if (!f16) {
       if (R == 64) coupling_fp32_inverse_kernel<64><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
