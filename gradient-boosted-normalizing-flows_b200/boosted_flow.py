@@ -164,15 +164,14 @@ class BoostedFlow(nn.Module):
 
     @torch.no_grad()
     def _fused_backward_ok(self, x):
-        """Whether gbnf_component_backward serves this configuration.  Besides the architecture (depth-1 tanh / relu networks,
-        h <= 512, D <= 64, no invconv, no BatchNorm), the per-row kernel keeps every step's input and network outputs in shared
-        memory, so num_flows x (z_size + 64 x networks per step) must fit beside the h-wide activation rows: see
-        fused_backward_smem_bytes.  The deepest component served at D = 2 / 21 / 43 / 64 is, at h = 512, K = 27 / 20 / 15 / 12
-        for Glow and K = 14 / 11 / 9 / 8 for RealNVP; at h = 64, K = 47 / 36 / 28 / 23 and 24 / 20 / 17 / 15.  Everything
-        else trains through the caller's autograd."""
+        """Whether gbnf_component_backward serves this configuration.  Besides the architecture (tanh / relu networks of any
+        coupling_network_depth gbnf_create accepts, h <= 512, D <= 64, no invconv, no BatchNorm), the per-row kernel keeps every
+        step's input and network outputs in shared memory, so num_flows x (z_size + 64 x networks per step) must fit beside the
+        h-wide activation rows: see fused_backward_smem_bytes, which does not depend on the depth.  The deepest component served
+        at D = 2 / 21 / 43 / 64 is, at h = 512, K = 27 / 20 / 15 / 12 for Glow and K = 14 / 11 / 9 / 8 for RealNVP; at h = 64,
+        K = 47 / 36 / 28 / 23 and 24 / 20 / 17 / 15.  Everything else trains through the caller's autograd."""
         a = self.args
-        if not (self.fused_backward and x.is_cuda and x.dtype == torch.float32 and a.coupling_network_depth == 1
-                and a.h_size <= 512 and self.z_size <= 64):
+        if not (self.fused_backward and x.is_cuda and x.dtype == torch.float32 and a.h_size <= 512 and self.z_size <= 64):
             return False
         if fused_backward_smem_bytes(self.component_type, self.z_size, a.h_size, a.num_flows) > FUSED_BACKWARD_MAX_SMEM:
             return False
@@ -183,7 +182,8 @@ class BoostedFlow(nn.Module):
 
     def _component_backward(self, c, x, dz, dldj, with_dx=False):
         """Gradients of component c's parameters for upstream (dz, dldj) through gbnf_component_backward:
-        ({id(param): grad}, dL/dx if with_dx else None)."""
+        ({id(param): grad}, dL/dx if with_dx else None).  Every Linear layer of every coupling network is passed, depth + 2 per
+        network at any coupling_network_depth."""
         lib = _lib.load()
         device = x.device
         h = self.handle(device)

@@ -797,19 +797,22 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
   if (c < 0 || c >= h->cfg.C || p->n_steps != h->cfg.K) return fail(GBNF_ERR_INVALID, "bad component index / n_steps");
   const gbnf_config& cf = h->cfg;
   const bool glow = cf.kind == GBNF_KIND_GLOW;
-  if (cf.glow_invconv || cf.depth != 1 || cf.act == GBNF_ACT_RESIDUAL || (glow && cf.act == GBNF_ACT_MIXED) || cf.h > 512 || cf.D > 64)
+  if (cf.glow_invconv || cf.act == GBNF_ACT_RESIDUAL || (glow && cf.act == GBNF_ACT_MIXED) || cf.h > 512 || cf.D > 64)
     return fail(GBNF_ERR_INVALID, "fused backward: Glow (with a permutation) or RealNVP (without BatchNorm) components with "
-                                  "coupling_network_depth 1, tanh / relu (RealNVP: or mixed) networks, h <= 512, D <= 64 (others train "
-                                  "through the caller's autograd)");
+                                  "coupling_network_depth 0 to 4, tanh / relu (RealNVP: or mixed) networks, h <= 512, D <= 64 (others "
+                                  "train through the caller's autograd)");
   if (!glow && p->flip_init != c) return fail(GBNF_ERR_INVALID, "RealNVP component c must have flip_init == c (models/boosted_flow.py:46)");
   if (B <= 0) return fail(GBNF_ERR_INVALID, "empty batch");
   ENTER(h);
   cudaStream_t st = (cudaStream_t)stream;
   const int K = cf.K, D = cf.D, hD0 = D / 2, hD1 = D - hD0;
   const int nnets = glow ? 1 : 2;
+  const int L = cf.depth + 2;                  // Linear layers per coupling network (gbnf_create bounds L <= GBNF_MAX_LAYERS)
   const int hp = round_up(cf.h, 64);
-  // per-step geometry: RealNVP steps alternate |z1| / |z2| when D is odd (flipped iff (k + c) is odd, models/realnvp.py:37-43)
-  struct Geo { int in_dim, out_dim, Kd[3], Nn[3], Kp[3], Np[3], NKp[3], KNp[3]; long long wfloats; };
+  // per-step geometry: RealNVP steps alternate |z1| / |z2| when D is odd (flipped iff (k + c) is odd, models/realnvp.py:37-43);
+  // layer l maps Kd[l] -> Nn[l]: in_dim -> h, then depth times h -> h, then h -> the coupling's output width
+  struct Geo { int in_dim, out_dim, Kd[GBNF_MAX_LAYERS], Nn[GBNF_MAX_LAYERS], Kp[GBNF_MAX_LAYERS], Np[GBNF_MAX_LAYERS],
+               NKp[GBNF_MAX_LAYERS], KNp[GBNF_MAX_LAYERS]; long long wfloats; };
   std::vector<Geo> geo(K);
   long long need_w = 1024;
   int ldz1 = 0;
@@ -818,12 +821,11 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
     const bool flipped = !glow && (((k + c) % 2) > 0);
     g.in_dim = flipped ? hD1 : hD0; g.out_dim = flipped ? hD0 : hD1;
     const int n3 = glow ? ((cf.coupling == GBNF_COUPLING_AFFINE) ? 2 * g.out_dim : g.out_dim) : g.out_dim;
-    const int Kd[3] = {g.in_dim, cf.h, cf.h}, Nn[3] = {cf.h, cf.h, n3};
     g.wfloats = 0;
-    for (int l = 0; l < 3; ++l) {
-      g.Kd[l] = Kd[l]; g.Nn[l] = Nn[l];
-      g.Kp[l] = round_up(Kd[l], kF32KT); g.Np[l] = round_up(Nn[l], kF32NT);
-      g.NKp[l] = round_up(Nn[l], kF32KT); g.KNp[l] = round_up(Kd[l], kF32NT);
+    for (int l = 0; l < L; ++l) {
+      g.Kd[l] = (l == 0) ? g.in_dim : cf.h; g.Nn[l] = (l == L - 1) ? n3 : cf.h;
+      g.Kp[l] = round_up(g.Kd[l], kF32KT); g.Np[l] = round_up(g.Nn[l], kF32NT);
+      g.NKp[l] = round_up(g.Nn[l], kF32KT); g.KNp[l] = round_up(g.Kd[l], kF32NT);
       g.wfloats += (long long)g.Kp[l] * g.Np[l] + (long long)g.NKp[l] * g.KNp[l] + g.Np[l];
     }
     g.wfloats *= nnets;
@@ -841,7 +843,7 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
                                     "statistics couple the rows of a batch)");
     }
     for (int net = 0; net < nnets; ++net)
-      for (int l = 0; l < 3; ++l)
+      for (int l = 0; l < L; ++l)
         if (!sp.W[net][l] || !sp.b[net][l] || !sg.W[net][l] || !sg.b[net][l]) return fail(GBNF_ERR_INVALID, "missing Linear weight / bias / gradient pointer");
   }
   const int ld = std::max(hp, ldz1) + 4;
@@ -856,7 +858,8 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
     CUDA_TRY_H(h, cudaMalloc(&h->tr_w, need_w * sizeof(float)));
     h->tr_w_floats = need_w;
   }
-  const long long per_row = (long long)ldz1 + nnets * (4LL * hp + 64);
+  // per row and step: z1, then per network depth + 1 hidden activations, as many hidden d pre-activations and the last layer's
+  const long long per_row = (long long)ldz1 + nnets * (2LL * (L - 1) * hp + 64);
   if (B > h->tr_rows || per_row > h->tr_per_row) {
     if (h->tr_scratch) cudaFree(h->tr_scratch);
     h->tr_scratch = nullptr; h->tr_rows = 0;
@@ -864,7 +867,7 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
     CUDA_TRY_H(h, cudaMalloc(&h->tr_scratch, (size_t)rows * per_row * K * sizeof(float)));
     h->tr_rows = rows; h->tr_per_row = per_row;
   }
-  const int njobs = K * nnets * 3;
+  const int njobs = K * nnets * L;
   if (!h->tr_steps_d || njobs > h->tr_njobs) {
     if (h->tr_steps_d) { cudaFree(h->tr_steps_d); cudaFree(h->tr_pack_d); cudaFree(h->tr_jobs_d); }
     CUDA_TRY_H(h, cudaMalloc(&h->tr_steps_d, (size_t)K * sizeof(TrainStep)));
@@ -888,15 +891,13 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
     ts.flipped = (!glow && (((k + c) % 2) > 0)) ? 1 : 0; ts.in_dim = g.in_dim; ts.out_dim = g.out_dim;
     float* sc = h->tr_scratch + (size_t)k * h->tr_rows * per_row;
     ts.z1 = sc; sc += h->tr_rows * ldz1;
-    for (int l = 0; l < 3; ++l) { ts.Kp[l] = g.Kp[l]; ts.Np[l] = g.Np[l]; ts.NKp[l] = g.NKp[l]; ts.KNp[l] = g.KNp[l]; }
+    for (int l = 0; l < L; ++l) { ts.Kp[l] = g.Kp[l]; ts.Np[l] = g.Np[l]; ts.NKp[l] = g.NKp[l]; ts.KNp[l] = g.KNp[l]; }
     // note: z1 rows are stored with stride Kp[0] of THIS step (<= ldz1)
     for (int net = 0; net < nnets; ++net) {
-      ts.h1[net] = sc; sc += h->tr_rows * hp;
-      ts.h2[net] = sc; sc += h->tr_rows * hp;
-      ts.d1[net] = sc; sc += h->tr_rows * hp;
-      ts.d2[net] = sc; sc += h->tr_rows * hp;
-      ts.d3[net] = sc; sc += h->tr_rows * 64;
-      for (int l = 0; l < 3; ++l) {
+      for (int l = 0; l < L - 1; ++l) { ts.hid[net][l] = sc; sc += h->tr_rows * hp; }
+      for (int l = 0; l < L - 1; ++l) { ts.dpre[net][l] = sc; sc += h->tr_rows * hp; }
+      ts.dpre[net][L - 1] = sc; sc += h->tr_rows * 64;
+      for (int l = 0; l < L; ++l) {
         TrainPackJob& pj = h->tr_pack_h[(size_t)job];
         pj.W = sp.W[net][l]; pj.b = sp.b[net][l]; pj.N = g.Nn[l]; pj.Kd = g.Kd[l]; pj.Kp = g.Kp[l]; pj.Np = g.Np[l]; pj.NKp = g.NKp[l]; pj.KNp = g.KNp[l];
         pj.Wt = w; w += (long long)g.Kp[l] * g.Np[l];
@@ -904,8 +905,8 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
         pj.bp = w; w += g.Np[l];
         ts.Wt[net][l] = pj.Wt; ts.Wn[net][l] = pj.Wn; ts.b[net][l] = pj.bp;
         WgradJob& wj = h->tr_jobs_h[(size_t)job];
-        wj.dact = (l == 0) ? ts.d1[net] : (l == 1) ? ts.d2[net] : ts.d3[net];  wj.ld_d = (l == 2) ? g.Np[2] : hp;
-        wj.in = (l == 0) ? ts.z1 : (l == 1) ? ts.h1[net] : ts.h2[net];          wj.ld_i = (l == 0) ? g.Kp[0] : hp;
+        wj.dact = ts.dpre[net][l];                        wj.ld_d = (l == L - 1) ? g.Np[L - 1] : hp;
+        wj.in = (l == 0) ? ts.z1 : ts.hid[net][l - 1];    wj.ld_i = (l == 0) ? g.Kp[0] : hp;
         wj.dW = sg.W[net][l]; wj.db = sg.b[net][l]; wj.N = g.Nn[l]; wj.Kd = g.Kd[l];
         wj.tiles_n = (g.Nn[l] + 63) / 64; wj.tiles_k = (g.Kd[l] + 63) / 64; wj.tile0 = tile0;
         tile0 += wj.tiles_n * wj.tiles_k;
@@ -924,7 +925,7 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
   train_pack_kernel<<<dim3(32, njobs), 256, 0, st>>>(h->tr_pack_d);
   TrainArgs ta{};
   ta.x = d_x; ta.B = B; ta.dz = d_dz; ta.dldj = d_dldj; ta.steps = h->tr_steps_d; ta.K = K; ta.D = D; ta.h = cf.h; ta.hp = hp;
-  ta.act = cf.act; ta.coupling = cf.coupling; ta.kind = cf.kind; ta.nnets = nnets; ta.ld = ld; ta.zeros = zeros; ta.dx = d_dx_opt;
+  ta.act = cf.act; ta.coupling = cf.coupling; ta.kind = cf.kind; ta.nnets = nnets; ta.nlayers = L; ta.ld = ld; ta.zeros = zeros; ta.dx = d_dx_opt;
   CUDA_TRY_H(h, cudaFuncSetAttribute(train_bwd_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTrMaxSmem));
   train_bwd_rows_kernel<<<(unsigned)((B + kTrR - 1) / kTrR), kF32Threads, smem, st>>>(ta);
   train_wgrad_kernel<<<tile0, 256, 0, st>>>(h->tr_jobs_d, njobs, B);

@@ -5,19 +5,22 @@
 //
 //   phase A  train_bwd_rows_kernel   one CTA per 16 rows, all K steps: forward sweep in shared memory (keeps every step's
 //            input and coupling-network output), then the backward sweep from the last step to the first: coupling
-//            transform, the three data-gradient GEMMs (d act = d out . W, nn.Linear layout) with the tanh / ReLU derivative,
-//            permutation and ActNorm.  Leaves h1, h2 and the three "d pre-activation" matrices of every step in an L2-resident
-//            scratch, accumulates the ActNorm gradients.
+//            transform, the L = depth + 2 data-gradient GEMMs (d act = d out . W, nn.Linear layout) with the tanh / ReLU
+//            derivative, permutation and ActNorm.  Leaves the depth + 1 hidden activations and the L "d pre-activation"
+//            matrices of every step in an L2-resident scratch, accumulates the ActNorm gradients.
 //   phase B  train_wgrad_kernel      dW[n][k] = sum_rows dact[r][n] * in[r][k] and db[n] = sum_rows dact[r][n] for every
 //            (step, layer): 64 x 64 output tiles over ALL rows, written straight into the caller's gradient tensors
 //            (deterministic: no atomics on the weight gradients).
 // fp32 CUDA-core arithmetic throughout (reference-class numerics: the gate is 1e-4 on the gradients).
-// Models, in the reference's own (logical) column order, coupling networks of depth 1:
+// Models, in the reference's own (logical) column order, coupling networks of every depth the library accepts (0 .. 4:
+// Linear(in, h), depth x Linear(h, h), Linear(h, out), an activation after every layer but the last):
 //   Glow step    = ActNorm1d -> Permute1d -> affine / additive coupling with ONE MLP (models/glow.py:317-342,
 //                  models/layers.py:208-243,488-518,661-668);
 //   RealNVP step = [z1 | z2] split (swapped when the step is flipped) -> z2' = t(z1) + z2 exp(s(z1)) with TWO MLPs, output
 //                  [z1, z2'] (models/transformations.py:560-579, models/realnvp.py:35-76); steps WITHOUT BatchNorm only
 //                  (train-mode BatchNorm couples the rows of a batch: those configurations train through autograd).
+// Shared memory holds three activation rows whatever the depth (the hidden layers ping-pong between two of them; what phase B
+// needs goes to the scratch), so the deepest component served at a given (kind, D, h) does not depend on the depth.
 #pragma once
 #include "coupling_fp32.cuh"
 
@@ -29,14 +32,16 @@ constexpr size_t kTrMaxSmem = 227 * 1024;   // dynamic shared memory one block m
 struct TrainStep {                   // one coupling step of the component under training (device pointers)
   const float* an_bias; const float* an_logs; const long long* perm;       // Glow: raw reference tensors; RealNVP: null
   int flipped, in_dim, out_dim, pad_;                                      // RealNVP: (k + flip_init) odd; |z1|, |z2| of this step
-  const float* Wt[2][3];             // forward layout  Wt[Kp][Np]   (k-major, n contiguous, zero padded); net 0 = glow block / t, 1 = s
-  const float* Wn[2][3];             // backward layout Wn[NKp][KNp] (nn.Linear rows = n, k contiguous, zero padded)
-  const float* b[2][3];              // biases padded to Np
-  int Kp[3], Np[3];                  // forward padding (Kp % 32 == 0, Np % 64 == 0)
-  int NKp[3], KNp[3];                // backward padding: rows (n) to a multiple of 32, columns (k) to a multiple of 64
+  // per Linear layer l < L = depth + 2 of network net (0 = glow block / t, 1 = s)
+  const float* Wt[2][GBNF_MAX_LAYERS];   // forward layout  Wt[Kp][Np]   (k-major, n contiguous, zero padded)
+  const float* Wn[2][GBNF_MAX_LAYERS];   // backward layout Wn[NKp][KNp] (nn.Linear rows = n, k contiguous, zero padded)
+  const float* b[2][GBNF_MAX_LAYERS];    // biases padded to Np
+  int Kp[GBNF_MAX_LAYERS], Np[GBNF_MAX_LAYERS];     // forward padding (Kp % 32 == 0, Np % 64 == 0)
+  int NKp[GBNF_MAX_LAYERS], KNp[GBNF_MAX_LAYERS];   // backward padding: rows (n) to a multiple of 32, columns (k) to a multiple of 64
   float* g_bias; float* g_logs;      // ActNorm gradients [D] (accumulated with atomics; zeroed by the host)
-  // scratch (per step, [B][ld]): activations and d pre-activations for phase B
-  float* z1; float* h1[2]; float* h2[2]; float* d1[2]; float* d2[2]; float* d3[2];
+  // scratch (per step, [B][ld]) for phase B: the network input z1 [B][Kp[0]], the output of hidden layer l < L - 1
+  // hid[net][l] [B][hp], and the d pre-activation of layer l dpre[net][l] ([B][hp]; the last layer [B][Np[L - 1]])
+  float* z1; float* hid[2][GBNF_MAX_LAYERS - 1]; float* dpre[2][GBNF_MAX_LAYERS];
 };
 
 struct TrainArgs {
@@ -44,6 +49,7 @@ struct TrainArgs {
   const float* dz; const float* dldj;          // upstream gradients dL/dz [B, D], dL/dldj [B]
   const TrainStep* steps; int K;
   int D, h, hp, act, coupling, kind, nnets;
+  int nlayers;                                 // Linear layers per coupling network: depth + 2
   int ld;                                      // row stride of the shared activation buffers
   const float* zeros;                          // >= 1024 zero floats (bias of the data-gradient GEMMs)
   float* dx;                                   // optional dL/dx [B, D]
@@ -78,7 +84,7 @@ inline size_t train_bwd_smem_bytes(int K, int D, int nnets, int ld) {
 __global__ void __launch_bounds__(kF32Threads, 1) train_bwd_rows_kernel(TrainArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr int R = kTrR;
-  const int D = a.D, K = a.K, ld = a.ld, hD0 = a.D / 2;
+  const int D = a.D, K = a.K, L = a.nlayers, ld = a.ld, hD0 = a.D / 2;
   const bool glow = a.kind == GBNF_KIND_GLOW;
   float* zh = reinterpret_cast<float*>(smem_raw);
   float* oh = zh + (((K + 1) * R * D + 3) & ~3);
@@ -122,14 +128,20 @@ __global__ void __launch_bounds__(kF32Threads, 1) train_bwd_rows_kernel(TrainArg
       }
       __syncthreads();
       const int ak = act_of(net);
-      train_gemm<R>(ak, act0, act1, ld, s.Wt[net][0], s.b[net][0], s.Kp[0], s.Np[0], Ws);
-      train_gemm<R>(ak, act1, act2, ld, s.Wt[net][1], s.b[net][1], s.Kp[1], s.Np[1], Ws);
-      for (int i = tid; i < R * hp; i += kF32Threads) {          // h1, h2 for the backward sweep and for phase B
-        const int r = i / hp, j = i - r * hp;
-        const long long gr = row0 + r;
-        if (gr < a.B) { s.h1[net][gr * hp + j] = act1[r * ld + j]; s.h2[net][gr * hp + j] = act2[r * ld + j]; }
+      // act0 -> layer 0 -> act1; the hidden layers ping-pong between act1 and act2; the last layer writes act0
+      float* in = act0;
+      float* out = act1;
+      for (int l = 0; l < L - 1; ++l) {
+        train_gemm<R>(ak, in, out, ld, s.Wt[net][l], s.b[net][l], s.Kp[l], s.Np[l], Ws);
+        for (int i = tid; i < R * hp; i += kF32Threads) {        // hidden activation for the backward sweep and for phase B
+          const int r = i / hp, j = i - r * hp;
+          const long long gr = row0 + r;
+          if (gr < a.B) s.hid[net][l][gr * hp + j] = out[r * ld + j];
+        }
+        in = out;
+        out = (out == act1) ? act2 : act1;
       }
-      train_gemm<R>(0, act2, act0, ld, s.Wt[net][2], s.b[net][2], s.Kp[2], s.Np[2], Ws);
+      train_gemm<R>(0, in, act0, ld, s.Wt[net][L - 1], s.b[net][L - 1], s.Kp[L - 1], s.Np[L - 1], Ws);
       for (int i = tid; i < R * 64; i += kF32Threads) oh[((k * a.nnets + net) * R + (i >> 6)) * 64 + (i & 63)] = act0[(i >> 6) * ld + (i & 63)];
       __syncthreads();
     }
@@ -174,8 +186,9 @@ __global__ void __launch_bounds__(kF32Threads, 1) train_bwd_rows_kernel(TrainArg
     }
     __syncthreads();
     for (int net = a.nnets - 1; net >= 0; --net) {
-      // coupling transform backward -> d out of this network in act0 [R][Np3]; after the LAST network (net 0) dzb[:, h0:] = d z2
-      for (int i = tid; i < R * s.Np[2]; i += kF32Threads) act0[(i / s.Np[2]) * ld + (i % s.Np[2])] = 0.f;
+      // coupling transform backward -> d out of this network in act0 [R][Np[L - 1]]; after the LAST network (net 0) dzb[:, h0:] = d z2
+      const int NpL = s.Np[L - 1];
+      for (int i = tid; i < R * NpL; i += kF32Threads) act0[(i / NpL) * ld + (i % NpL)] = 0.f;
       __syncthreads();
       for (int i = tid; i < R * h1d; i += kF32Threads) {
         const int r = i / h1d, jj = i - r * h1d;
@@ -199,34 +212,31 @@ __global__ void __launch_bounds__(kF32Threads, 1) train_bwd_rows_kernel(TrainArg
         }
       }
       __syncthreads();
-      for (int i = tid; i < R * s.Np[2]; i += kF32Threads) {
-        const int r = i / s.Np[2], j = i - r * s.Np[2];
+      for (int i = tid; i < R * NpL; i += kF32Threads) {
+        const int r = i / NpL, j = i - r * NpL;
         const long long gr = row0 + r;
-        if (gr < a.B) s.d3[net][gr * s.Np[2] + j] = act0[r * ld + j];
+        if (gr < a.B) s.dpre[net][L - 1][gr * NpL + j] = act0[r * ld + j];
       }
       const int ak = act_of(net);
-      // d h2 = d3 . W3   (nn.Linear layout: rows n, columns k)
-      gemm_layer_fp32<R, 0>(act0, act1, ld, s.Wn[net][2], a.zeros, s.NKp[2], s.KNp[2], Ws);
-      for (int i = tid; i < R * hp; i += kF32Threads) {
-        const int r = i / hp, j = i - r * hp;
-        const long long gr = row0 + r;
-        const float hv = (gr < a.B) ? s.h2[net][gr * hp + j] : 0.f;
-        const float d = act1[r * ld + j] * (ak == 2 ? act_grad_from_output<2>(hv) : act_grad_from_output<1>(hv));
-        act1[r * ld + j] = d;
-        if (gr < a.B) s.d2[net][gr * hp + j] = d;
+      // mirror of the forward sweep: d h_l = d_l . W_l (nn.Linear layout: rows n, columns k) into act1, act2, act1, ...,
+      // times the activation derivative read from the stored h_l; d z1 = d_0 . W_0 ends in act0
+      float* din = act0;
+      float* dout = act1;
+      for (int l = L - 1; l > 0; --l) {
+        gemm_layer_fp32<R, 0>(din, dout, ld, s.Wn[net][l], a.zeros, s.NKp[l], s.KNp[l], Ws);
+        for (int i = tid; i < R * hp; i += kF32Threads) {
+          const int r = i / hp, j = i - r * hp;
+          const long long gr = row0 + r;
+          const float hv = (gr < a.B) ? s.hid[net][l - 1][gr * hp + j] : 0.f;
+          const float d = dout[r * ld + j] * (ak == 2 ? act_grad_from_output<2>(hv) : act_grad_from_output<1>(hv));
+          dout[r * ld + j] = d;
+          if (gr < a.B) s.dpre[net][l - 1][gr * hp + j] = d;
+        }
+        __syncthreads();
+        din = dout;
+        dout = (dout == act1) ? act2 : act1;
       }
-      __syncthreads();
-      gemm_layer_fp32<R, 0>(act1, act2, ld, s.Wn[net][1], a.zeros, s.NKp[1], s.KNp[1], Ws);
-      for (int i = tid; i < R * hp; i += kF32Threads) {
-        const int r = i / hp, j = i - r * hp;
-        const long long gr = row0 + r;
-        const float hv = (gr < a.B) ? s.h1[net][gr * hp + j] : 0.f;
-        const float d = act2[r * ld + j] * (ak == 2 ? act_grad_from_output<2>(hv) : act_grad_from_output<1>(hv));
-        act2[r * ld + j] = d;
-        if (gr < a.B) s.d1[net][gr * hp + j] = d;
-      }
-      __syncthreads();
-      gemm_layer_fp32<R, 0>(act2, act0, ld, s.Wn[net][0], a.zeros, s.NKp[0], s.KNp[0], Ws);      // d z1 [R][KNp0] (first h0 columns valid)
+      gemm_layer_fp32<R, 0>(din, act0, ld, s.Wn[net][0], a.zeros, s.NKp[0], s.KNp[0], Ws);      // d z1 [R][KNp0] (first h0 columns valid)
       for (int i = tid; i < R * h0; i += kF32Threads) {
         const int r = i / h0, j = i - r * h0;
         dzb[r * D + j] += act0[r * ld + j];                                  // z1 passes through AND feeds the network(s)

@@ -203,11 +203,15 @@ int gbnf_weight_renorm(gbnf_handle h, float* d_w, int64_t B, const double* d_wsu
  * `p` holds the component's CURRENT raw parameters (as for gbnf_pack_component), `grads` the same tensors' gradient
  * buffers, which are OVERWRITTEN.  Glow components with a permutation (tanh / relu) and RealNVP components WITHOUT BatchNorm
  * (tanh / relu / mixed; models/transformations.py:560-579 -- train-mode BatchNorm couples the rows of a batch), with
- * coupling_network_depth 1, h <= 512, D <= 64.  The per-row kernel keeps every step's input and coupling-network outputs
- * in shared memory, so K x (D + 64 x networks per step) must fit in it beside the h-wide activation rows (227 KB in all):
- * the deepest component served at D = 2 / 21 / 43 / 64 is, at h = 512, K = 27 / 20 / 15 / 12 for Glow and 14 / 11 / 9 / 8
- * for RealNVP; at h = 64, K = 47 / 36 / 28 / 23 and 24 / 20 / 17 / 15.  Other configurations return GBNF_ERR_INVALID
- * before anything is written (`grads` and the handle stay as they were) and train through the caller's autograd.
+ * every coupling_network_depth gbnf_create accepts (0 to 4: W / b / grads carry depth + 2 layers per network), h <= 512,
+ * D <= 64.  The per-row kernel keeps every step's input and coupling-network outputs in shared memory, so
+ * K x (D + 64 x networks per step) must fit in it beside the h-wide activation rows (227 KB in all; the hidden layers of a
+ * deeper network reuse the same rows, so this bound does not depend on the depth): the deepest component served at
+ * D = 2 / 21 / 43 / 64 is, at h = 512, K = 27 / 20 / 15 / 12 for Glow and 14 / 11 / 9 / 8 for RealNVP; at h = 64,
+ * K = 47 / 36 / 28 / 23 and 24 / 20 / 17 / 15.  The device scratch the call keeps (B x K x (2 (depth + 1) x round_up(h, 64)
+ * + 64) floats per network) grows with the depth; an allocation failure returns GBNF_ERR_CUDA before `grads` is written.
+ * Other configurations return GBNF_ERR_INVALID before anything is written (`grads` and the handle stay as they were) and
+ * train through the caller's autograd.
  * d_dx_opt [B, D] (may be NULL) receives dL/dx. */
 typedef struct {
   float* an_bias;

@@ -2,10 +2,13 @@
 """One TRAINING step of the boosted objective (density_experiment.py:359-374: compute_kl_pq_loss -> backward -> clip -> optimizer
 step) on cfg3's architecture, component C-1 being trained: this library (fixed mixture + weights + resampling kernels, new
 component forward and backward through gbnf_component_backward) against the same host code with the new component on torch
-autograd, and against the UNMODIFIED reference moved to the same GPU.  Prints one JSON line."""
+autograd, and against the UNMODIFIED reference moved to the same GPU.  --depth sets coupling_network_depth (cfg3 itself has
+depth 1); the reference arm builds depth-1 networks only, so at any other depth its column is null and the JSON says why.
+Prints one JSON line with the card's name and power limit."""
 import argparse
 import json
 import os
+import subprocess
 import sys
 import time
 
@@ -29,9 +32,10 @@ def time_steps(step, n, warm=5):
     return e0.elapsed_time(e1) / n
 
 
-def ours(cfg, dev, batch, fused, mode, n):
+def ours(cfg, dev, batch, fused, mode, n, depth):
     torch.manual_seed(1)
     a = bench.make_args(cfg, dev)
+    a.coupling_network_depth = depth
     a.fused_backward = fused
     model = gbnf_b200.BoostedFlow(a, gemm_mode=mode).to(dev)
     x = torch.randn((batch, cfg["D"]), device=dev, generator=torch.Generator(device=dev).manual_seed(5))
@@ -45,6 +49,7 @@ def ours(cfg, dev, batch, fused, mode, n):
         for p in f.parameters():
             p.requires_grad_(i == C - 1)
     opt = torch.optim.Adam(list(model.flows[C - 1].parameters()), lr=1e-4)
+    assert model._fused_backward_ok(x) == fused, "the fused arm must train through gbnf_component_backward"
     largs = argparse.Namespace(flow="boosted")
     gen = torch.Generator(device=dev).manual_seed(3)
 
@@ -86,22 +91,33 @@ def reference(cfg, dev, batch, n):
     return time_steps(step, n)
 
 
+def card(index):
+    q = subprocess.run(["nvidia-smi", "-i", str(index), "--query-gpu=power.limit", "--format=csv,noheader"],
+                       capture_output=True, text=True)
+    return {"device": torch.cuda.get_device_name(index), "power_limit": q.stdout.strip()}
+
+
 def main():
     p = argparse.ArgumentParser()
     p.add_argument("--config", default="cfg3_miniboone")
     p.add_argument("--batches", default="512,4096")
     p.add_argument("--steps", type=int, default=30)
     p.add_argument("--mode", default="f16fast")
+    p.add_argument("--depth", type=int, default=1, help="coupling_network_depth of every coupling network (0 .. 4)")
     a = p.parse_args()
     cfg = bench.CONFIGS[a.config]
     dev = torch.device("cuda", 0)
     out = {"what": f"one training step of component {cfg['C'] - 1} of {a.config} (fixed mixture of {cfg['C'] - 1} components + weights + resampling + "
-                   "new-component forward/backward + clip + Adam)", "mode": a.mode, "rows": []}
+                   "new-component forward/backward + clip + Adam)", "mode": a.mode, "coupling_network_depth": a.depth,
+           **card(0), "rows": []}
+    if a.depth != 1:
+        out["reference_note"] = ("null: baseline/ref_harness builds the reference with coupling_network_depth 1 only, so the reference "
+                                 f"arm has no depth-{a.depth} model")
     for b in [int(v) for v in a.batches.split(",")]:
         row = {"batch": b,
-               "library_fused_backward_ms": ours(cfg, dev, b, True, a.mode, a.steps),
-               "library_torch_autograd_new_component_ms": ours(cfg, dev, b, False, a.mode, a.steps),
-               "reference_eager_same_gpu_ms": reference(cfg, dev, b, a.steps)}
+               "library_fused_backward_ms": ours(cfg, dev, b, True, a.mode, a.steps, a.depth),
+               "library_torch_autograd_new_component_ms": ours(cfg, dev, b, False, a.mode, a.steps, a.depth),
+               "reference_eager_same_gpu_ms": reference(cfg, dev, b, a.steps) if a.depth == 1 else None}
         row["samples_per_s_fused"] = b / (row["library_fused_backward_ms"] * 1e-3)
         out["rows"].append(row)
     print(json.dumps(out))
