@@ -63,6 +63,7 @@ SIGNATURES = {
     "gbnf_set_base": (C.c_int, [_vp, _vp, _vp, _vp]),
     "gbnf_component_logq": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp]),
     "gbnf_component_inverse": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp, _vp]),
+    "gbnf_mixture_inverse": (C.c_int, [_vp, _vp, _i64, _vp, _i32, _vp, _vp, _vp]),
     "gbnf_mixture_logdensity": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _i32, _i32, _vp, _vp]),
     "gbnf_fused_eval": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _i32, _i32, _vp, _vp, _vp]),
     "gbnf_boost_weights": (C.c_int, [_vp, _vp, _i64, _f32, _f32, _i32, _vp, _vp, _vp]),

@@ -262,12 +262,26 @@ class BoostedFlow(nn.Module):
             u = torch.rand(n, dtype=torch.float64, device=dev, generator=generator)
         if z is None:
             z = torch.randn((n, self.z_size), device=dev, generator=generator) * float(temperature)
-        comp = self.assign_components(u)
+        n_comp = self.num_components if self.all_trained else self.component + 1
+        comp = self.assign_components(u, n_comp)
+        return self.mixture_inverse(z.contiguous(), comp, n_comp)[0], comp
+
+    @torch.no_grad()
+    def mixture_inverse(self, z, comp, n=None):
+        """(x, log-det of the inverse map) with x[i] = flows[comp[i]]^{-1}(z[i]) through gbnf_mixture_inverse: one coupling launch
+        over every component's rows, no host synchronisation (after a first call at this batch size the call allocates nothing in
+        the library, so it can be captured in a CUDA graph).  comp: int64 ids in [0, n) (n defaults to every component); an id
+        outside it raises at the next check_status()."""
+        z = _f32c(z)
+        n = self.num_components if n is None else n
+        assert comp.dtype == torch.int64 and comp.is_cuda and comp.is_contiguous() and comp.shape == (z.shape[0],)
+        for c in range(n):
+            self.pack_component(c)
         x = torch.empty_like(z)
-        for c in torch.unique(comp).tolist():
-            rows = torch.nonzero(comp == c, as_tuple=False).squeeze(1)
-            x[rows] = self.component_inverse(z[rows].contiguous(), int(c))[0]
-        return x, comp
+        ldj = torch.empty(z.shape[0], device=z.device, dtype=torch.float32)
+        _lib.check(_lib.load().gbnf_mixture_inverse(self.handle(z.device), _ptr(z), z.shape[0], _ptr(comp), n, _ptr(x), _ptr(ldj),
+                                                    _stream(z.device)))
+        return x, ldj
 
     def forward(self, x=None, y_onehot=None, z=None, temperature=None, components=None, reverse=False):
         if reverse:

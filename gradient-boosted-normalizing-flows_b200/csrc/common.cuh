@@ -94,9 +94,20 @@ struct CouplingArgs {
                                    // the single-chain kernel on the last component, which reduces all n_mix terms)
   int* error_flag;                 // status words in MAPPED HOST memory (the host can read them after a trap, without a
                                    // synchronisation): [0] watchdog code of a timed-out wait, [1] fp16 weight overflow (pack),
-                                   // [2] a value entering an fp16 GEMM operand was not finite in fp16
+                                   // [2] a value entering an fp16 GEMM operand was not finite in fp16, [3] a component id
+                                   // given to gbnf_mixture_inverse was out of range
   long long* prof;                 // optional cycle counters (CTA 0), see gbnf_get_profile
 };
+
+// Work units of an inverse (sampling) launch, the kernels' third argument: unit u < min(num_units, *count) is
+// unit[u] = {component, first row, rows} over a.x, rows <= the kernel's tile height.  The count is written on the device
+// (gbnf_mixture_inverse sorts the rows by component first), so the grid is sized from the host bound num_units; every role of a
+// persistent kernel walks the same units.  Forward launches pass an empty table.
+struct UnitTable {
+  const int4* unit;
+  const int* count;
+};
+__device__ __forceinline__ int inverse_units(const CouplingArgs& a, const UnitTable& ut) { return min(a.num_units, __ldg(ut.count)); }
 
 // ---- peer-memory exchange between the ranks of one node (one process per GPU; gbnf_comm_init) ---------------------------------
 // Every rank owns one CommBlock in its own HBM, exported with cudaIpcGetMemHandle and mapped by all peers.  A rank PUBLISHES a

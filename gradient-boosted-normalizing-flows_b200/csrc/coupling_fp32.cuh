@@ -294,13 +294,14 @@ __global__ void __launch_bounds__(kF32Threads, 1) coupling_fp32_kernel(CouplingA
   }
 }
 
-// ---- inverse direction (sampling): x = f_c^{-1}(z) for ONE component -------------------------------------------------------
+// ---- inverse direction (sampling): x = f_c^{-1}(z) for the component of each work unit -----------------------------------------
 // Exact inverse of the forward kernel above, step by step in reverse order: coupling^-1 (the MLPs see z1, which the forward
 // step left untouched), then ActNorm^-1 / eval-BatchNorm^-1 on all columns.  Upstream: FlowStep.decode models/glow.py:344-366,
 // RealNVPFlow.decode models/realnvp.py:97-113 (whose flip pairing is not an inverse of encode, SURVEY 7 -- this one is).
-// a.x = z [B, D] (logical column order), a.z_out = x [B, D], a.ldj_out = log-det of the inverse map (= -forward log-det).
+// a.x = z [B, D] (logical column order), a.z_out = x [B, D], a.ldj_out = log-det of the inverse map (= -forward log-det); work
+// units from `ut` (one component and up to R rows each, common.cuh).
 template <int R>
-__global__ void __launch_bounds__(kF32Threads, 1) coupling_fp32_inverse_kernel(CouplingArgs a, int ld, int out_max) {
+__global__ void __launch_bounds__(kF32Threads, 1) coupling_fp32_inverse_kernel(CouplingArgs a, int ld, int out_max, UnitTable ut) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const ModelDims& md = a.md;
   const int D = md.D, Dv = md.Dv;
@@ -312,16 +313,18 @@ __global__ void __launch_bounds__(kF32Threads, 1) coupling_fp32_inverse_kernel(C
   float* coef = sh + R * out_max;
   float* ldj = coef + kMaxComponents;   // [R]
   const int tid = threadIdx.x;
-  const int c = a.c0;
-  const CompDesc& cd = a.comps[c];
-  const int* sig = a.iblob + cd.sigma_off;
-  for (int tile = blockIdx.x; tile < a.num_tiles; tile += gridDim.x) {
-    const long long row0 = (long long)tile * R;
+  const int num_units = min(a.num_units, __ldg(ut.count));
+  for (int u = blockIdx.x; u < num_units; u += gridDim.x) {
+    const int4 un = __ldg(ut.unit + u);
+    const int c = un.x;
+    const long long row0 = un.y, row_end = row0 + un.z;
+    const CompDesc& cd = a.comps[c];
+    const int* sig = a.iblob + cd.sigma_off;
     // z arrives in the flow's OUTPUT column order: logical column j lives at physical column sigma[j]
     for (int i = tid; i < R * D; i += kF32Threads) {
       int r = i / D, j = i % D;
       long long gr = row0 + r;
-      zs[r * Dv + sig[j]] = (gr < a.B) ? a.x[gr * D + j] : 0.f;
+      zs[r * Dv + sig[j]] = (gr < row_end) ? a.x[gr * D + j] : 0.f;
     }
     if (tid < R) ldj[tid] = 0.f;
     __syncthreads();
@@ -389,9 +392,9 @@ __global__ void __launch_bounds__(kF32Threads, 1) coupling_fp32_inverse_kernel(C
     for (int i = tid; i < R * D; i += kF32Threads) {
       int r = i / D, p = i % D;
       long long gr = row0 + r;
-      if (gr < a.B && a.z_out) a.z_out[gr * D + p] = zs[r * Dv + p];   // physical == logical at the flow's input
+      if (gr < row_end && a.z_out) a.z_out[gr * D + p] = zs[r * Dv + p];   // physical == logical at the flow's input
     }
-    if (tid < R && a.ldj_out && row0 + tid < a.B) a.ldj_out[row0 + tid] = ldj[tid] - a.fblob[cd.const_off];
+    if (tid < R && a.ldj_out && row0 + tid < row_end) a.ldj_out[row0 + tid] = ldj[tid] - a.fblob[cd.const_off];
     __syncthreads();
   }
 }

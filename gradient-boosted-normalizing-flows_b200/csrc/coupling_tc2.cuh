@@ -135,11 +135,13 @@ __device__ __forceinline__ void t2_act_pack(const uint32_t (&r)[N], const float*
 // ---- per-row epilogue code shared by the persistent tensor-core kernels (coupling_tc2/3/4/5.cuh): 512 epilogue threads,
 //      four per row (column group g), et = epilogue thread index ----
 
-// x tile of 128 rows -> xs (row-major, D floats a row, zero beyond row B), 8 independent loads in flight per thread
-__device__ __forceinline__ void t2_load_x_tile(float* xs, const CouplingArgs& a, int D, long long row0, int et) {
+// x tile of 128 rows -> xs (row-major, D floats a row, zero beyond row B; INV: from row row_end on), 8 independent loads in flight
+// per thread
+template <int INV = 0>
+__device__ __forceinline__ void t2_load_x_tile(float* xs, const CouplingArgs& a, int D, long long row0, int et, long long row_end = 0) {
   const int total = kTcRows * D;
   const long long gbase = row0 * D;
-  const long long glimit = a.B * (long long)D;
+  const long long glimit = (INV ? row_end : a.B) * (long long)D;
   for (int i0 = et; i0 < total; i0 += 8 * kT2EpiThreads) {
     float v[8];
 #pragma unroll
@@ -225,6 +227,17 @@ __device__ __forceinline__ void t2_component_logq(const CouplingArgs& a, const f
     }
     if (a.G_ll != nullptr && c < a.n_mix) __stcg(a.lse_terms + gr * a.n_mix + c, coef[c] + lq);
   }
+}
+
+// End of a component in the inverse direction: the log-det of the inverse map, the four groups' shares combined in
+// t2_component_logq's order, stored by the writer's group-0 thread for rows gr < row_end (the end of the work unit).
+__device__ __forceinline__ void t2_inverse_ldj(const CouplingArgs& a, float lsum, float* part, int row, int g, int quad,
+                                               float ldj_const, long long gr, long long row_end, bool writer) {
+  float* const part2 = part + 3 * kTcRows;
+  if (g > 0) part2[(g - 1) * kTcRows + row] = lsum;
+  t2_quad_bar(quad);
+  if (writer && g == 0 && gr < row_end && a.ldj_out)
+    a.ldj_out[gr] = (lsum + part2[row] + part2[kTcRows + row] + part2[2 * kTcRows + row]) + ldj_const;
 }
 
 // G_ll of the tile's rows: logsumexp over their mixture terms in component order (two passes: exact max, then the sum), by
@@ -367,13 +380,13 @@ __device__ __forceinline__ void t2_stage_bias_async(float* dst, const float* src
 // MV: model variant known at compile time - 1 = Glow / affine coupling / tanh nets (one net per step), 2 = RealNVP with tanh
 // s- and t-nets (two nets per step), 0 = read everything from the model: the other coupling variants, activations and net
 // counts drop out of the instantiation.
-// INV: 1 = inverse direction (sampling): a.x = z in the flow's output column order, ONE component (c0), steps walked from the
-// last to the first; every pass runs the same MLP(s) on z1 (which the forward step left untouched), un-does the coupling on
-// z2 and un-does the ActNorm / BatchNorm affine through the INVERSE gather-order tables (pack_meta_kernel); writes
-// a.z_out = x and a.ldj_out = log-det of the inverse map.  Upstream: FlowStep.decode models/glow.py:344-366,
-// RealNVPFlow.decode models/realnvp.py:97-113.
+// INV: 1 = inverse direction (sampling): a.x = z in the flow's output column order, work units from `ut` (one component and
+// up to 128 rows each, in any component order), steps walked from the last to the first; every pass runs the same MLP(s) on z1
+// (which the forward step left untouched), un-does the coupling on z2 and un-does the ActNorm / BatchNorm affine through the
+// INVERSE gather-order tables (pack_meta_kernel); writes a.z_out = x and a.ldj_out = log-det of the inverse map.  Upstream:
+// FlowStep.decode models/glow.py:344-366, RealNVPFlow.decode models/realnvp.py:97-113.
 template <int TANH_MODE, int PROF, int NQT, int MV = 0, int INV = 0>
-__global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArgs a, TcPlan plan) {
+__global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArgs a, TcPlan plan, UnitTable ut) {
   extern __shared__ __align__(1024) unsigned char smem[];
   // PTX predicate registers that carry the result of an early mbarrier.test_wait across the MMA block issued in between
   // (warps issue in order: converting the predicate to a value right away would stall the issuer for the ~100-cycle
@@ -433,8 +446,9 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
       ++sidx;
       if (++slot == nst) { slot = 0; par ^= 1u; }
     };
-    for (int u = blockIdx.x; u < a.num_units; u += gridDim.x) {
-      const int cb = a.c0 + (u % a.split) * a.comps_per_unit, ce = min(a.c1, cb + a.comps_per_unit);
+    for (int u = blockIdx.x; u < (INV ? inverse_units(a, ut) : a.num_units); u += gridDim.x) {
+      const int cb = INV ? __ldg(&ut.unit[u].x) : a.c0 + (u % a.split) * a.comps_per_unit;
+      const int ce = INV ? cb + 1 : min(a.c1, cb + a.comps_per_unit);
       for (int c = cb; c < ce; ++c)
         for (int kk = 0; kk < md.K; ++kk) {
           const int k = INV ? md.K - 1 - kk : kk;
@@ -514,8 +528,9 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
       m_wa += T2_CLOCK() - tw;
       ptx::tc_fence_after();
     };
-    for (int u = blockIdx.x; u < a.num_units; u += gridDim.x) {
-      const int cb = a.c0 + (u % a.split) * a.comps_per_unit, ce = min(a.c1, cb + a.comps_per_unit);
+    for (int u = blockIdx.x; u < (INV ? inverse_units(a, ut) : a.num_units); u += gridDim.x) {
+      const int cb = INV ? __ldg(&ut.unit[u].x) : a.c0 + (u % a.split) * a.comps_per_unit;
+      const int ce = INV ? cb + 1 : min(a.c1, cb + a.comps_per_unit);
       for (int c = cb; c < ce; ++c)
         for (int kk = 0; kk < md.K; ++kk) {
           const int k = INV ? md.K - 1 - kk : kk;
@@ -660,8 +675,8 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
     const uint32_t bstride = t2_bias_stride(md.h);
     // the first step's gather-order tables, scalars and biases; afterwards every pass stages what the next one needs
     // (cp.async issued while this pass waits for the tensor core, completed and published at the end of the pass)
-    if (blockIdx.x < a.num_units) {
-      const int cb0 = a.c0 + ((int)blockIdx.x % a.split) * a.comps_per_unit;
+    if (blockIdx.x < (INV ? inverse_units(a, ut) : a.num_units)) {
+      const int cb0 = INV ? __ldg(&ut.unit[blockIdx.x].x) : a.c0 + ((int)blockIdx.x % a.split) * a.comps_per_unit;
       const StepDesc* sd0 = a.steps + cb0 * md.K + (INV ? md.K - 1 : 0);
       if (et < 2 * kEpPad) ptx::cp_async16(tab_s + et, reinterpret_cast<const float4*>(a.fblob + __ldg(&sd0->ep_off)) + (INV ? 2 * kEpPad : 0) + et);
       if (et == 0) t2_stage_meta(sd0, nnets, misc->meta[0]);
@@ -670,10 +685,12 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
     const bool tr = (warp_e & 3) == 0;     // one tracing warp per group
     const long long e_t0 = T2_CLOCK();
     long long e_w1 = 0, e_w2 = 0, e_w3 = 0, e_l1 = 0, e_l2 = 0, e_l3 = 0, e_pro = 0, e_x = 0, e_tmp;
-    for (int u = blockIdx.x; u < a.num_units; u += gridDim.x) {
+    for (int u = blockIdx.x; u < (INV ? inverse_units(a, ut) : a.num_units); u += gridDim.x) {
       const int tile = u / a.split, cs = u - tile * a.split;
-      const int cb = a.c0 + cs * a.comps_per_unit, ce = min(a.c1, cb + a.comps_per_unit);
-      const long long row0 = (long long)tile * kTcRows;
+      const int4 un = INV ? __ldg(ut.unit + u) : make_int4(0, 0, 0, 0);   // INV: {component, first row, rows}
+      const int cb = INV ? un.x : a.c0 + cs * a.comps_per_unit, ce = INV ? cb + 1 : min(a.c1, cb + a.comps_per_unit);
+      const long long row0 = INV ? (long long)un.y : (long long)tile * kTcRows;
+      const long long row_end = row0 + un.z;         // INV: end of the unit's rows
       const long long gr = row0 + row;
       for (int c = cb; c < ce; ++c) {
         // ---- x tile: fetched from HBM once per tile (8 independent loads in flight per thread) and kept in shared
@@ -687,7 +704,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
         const float ldj_const = cconst.x, base_const = cconst.y;
         t2_epi_bar();                                // previous component's readers are done with zs / part
         if (c == cb) {
-          t2_load_x_tile(xs, a, D, row0, et);
+          t2_load_x_tile<INV>(xs, a, D, row0, et, row_end);
           t2_epi_bar();
         }
         if (INV) {   // z arrives in the flow's OUTPUT column order: logical column p lives at physical column sigma[p]
@@ -715,8 +732,9 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
           const int kfirst = INV ? md.K - 1 : 0;
           const StepDesc* sd_next = (kk + 1 < md.K) ? (INV ? sd - 1 : sd + 1)
                                     : (c + 1 < ce) ? a.steps + (c + 1) * md.K + kfirst
-                                    : (u + (int)gridDim.x < a.num_units)
-                                        ? a.steps + (a.c0 + ((u + (int)gridDim.x) % a.split) * a.comps_per_unit) * md.K + kfirst
+                                    : (u + (int)gridDim.x < (INV ? inverse_units(a, ut) : a.num_units))
+                                        ? a.steps + (INV ? __ldg(&ut.unit[u + gridDim.x].x)
+                                                         : a.c0 + ((u + (int)gridDim.x) % a.split) * a.comps_per_unit) * md.K + kfirst
                                         : nullptr;
           // ---- ActNorm / eval-BatchNorm affine fused into the gather of z1 -> A0 ----
           t2_gather_z1<INV>(zrow, tab1, in_dim, meta[2] >> 3, g, row, A0, a.error_flag);
@@ -912,10 +930,11 @@ __global__ void __launch_bounds__(kT2Threads, 1) coupling_tc2_kernel(CouplingArg
             e_l3 += T2_CLOCK() - e_tmp;
           }
         }
-        // ---- component log-density for this row ----
-        t2_component_logq(a, zrow, lsum, part, row, g, quad, h0col, h1col, Dv, base_off, INV ? -ldj_const : ldj_const, base_const,
-                          misc->coef, c, tile, true);
-        if (a.z_out != nullptr && gr < a.B) {
+        // ---- component log-density for this row (inverse: the log-det of the inverse map) ----
+        if (INV) t2_inverse_ldj(a, lsum, part, row, g, quad, -ldj_const, gr, row_end, true);
+        else     t2_component_logq(a, zrow, lsum, part, row, g, quad, h0col, h1col, Dv, base_off, ldj_const, base_const, misc->coef, c,
+                                   tile, true);
+        if (a.z_out != nullptr && gr < (INV ? row_end : a.B)) {
           if (INV) {   // physical == logical column order at the flow's input
             for (int j = h0col; j < h1col; ++j) a.z_out[gr * D + j] = zrow[j];
           } else {
@@ -965,14 +984,14 @@ inline cudaError_t tc2_configure() {
   return e;
 }
 
-inline int tc2_launch_inverse(const CouplingArgs& a, const TcPlan& p, int grid, cudaStream_t st) {
-  if (p.tanh_mode == 0) coupling_tc2_kernel<0, 0, 0, 0, 1><<<grid, kT2Threads, p.smem_bytes, st>>>(a, p);
-  else                  coupling_tc2_kernel<1, 0, 0, 0, 1><<<grid, kT2Threads, p.smem_bytes, st>>>(a, p);
+inline int tc2_launch_inverse(const CouplingArgs& a, const TcPlan& p, const UnitTable& ut, int grid, cudaStream_t st) {
+  if (p.tanh_mode == 0) coupling_tc2_kernel<0, 0, 0, 0, 1><<<grid, kT2Threads, p.smem_bytes, st>>>(a, p, ut);
+  else                  coupling_tc2_kernel<1, 0, 0, 0, 1><<<grid, kT2Threads, p.smem_bytes, st>>>(a, p, ut);
   return 0;
 }
 
 inline int tc2_launch(const CouplingArgs& a, const TcPlan& p, int grid, cudaStream_t st, int prof) {
-#define T2_GO(T, P, Q) coupling_tc2_kernel<T, P, Q><<<grid, kT2Threads, p.smem_bytes, st>>>(a, p)
+#define T2_GO(T, P, Q) coupling_tc2_kernel<T, P, Q><<<grid, kT2Threads, p.smem_bytes, st>>>(a, p, UnitTable{})
 #define T2_GO_Q(T, P) do { if (a.md.h == 512) T2_GO(T, P, 4); else T2_GO(T, P, 0); } while (0)
   if (prof == 1 || prof == 2) {
     if (p.tanh_mode == 0) { if (prof == 1) T2_GO_Q(0, 1); else T2_GO_Q(0, 2); }
@@ -986,8 +1005,8 @@ inline int tc2_launch(const CouplingArgs& a, const TcPlan& p, int grid, cudaStre
                : (a.md.kind == GBNF_KIND_REALNVP && a.md.act == GBNF_ACT_TANH && a.md.nnets == 2) ? 2 : 0;
 #define T2_GO_PROD(Q, MV) \
   if (q == Q && mv == MV) { \
-    if (p.tanh_mode == 0) coupling_tc2_kernel<0, 0, Q, MV><<<grid, kT2Threads, p.smem_bytes, st>>>(a, p); \
-    else                  coupling_tc2_kernel<1, 0, Q, MV><<<grid, kT2Threads, p.smem_bytes, st>>>(a, p); \
+    if (p.tanh_mode == 0) coupling_tc2_kernel<0, 0, Q, MV><<<grid, kT2Threads, p.smem_bytes, st>>>(a, p, UnitTable{}); \
+    else                  coupling_tc2_kernel<1, 0, Q, MV><<<grid, kT2Threads, p.smem_bytes, st>>>(a, p, UnitTable{}); \
     return 0; \
   }
   T2_FOR_PROD(T2_GO_PROD)

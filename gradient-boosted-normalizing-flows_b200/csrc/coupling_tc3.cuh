@@ -165,13 +165,14 @@ __device__ __forceinline__ void t3_act_pack32_add(const uint32_t (&r)[32], const
 // [11] wait xfull, [12] wait l2ship, [13] wait xfree, [14] wait l3f, [15] wait x3full, [19] gather, [20] layer-1 epilogues,
 // [21] own epilogues, [22] ship epilogues, [23] transform + end-of-pass barrier; [16] producer total, [17] wait empty.
 // INV: 1 = inverse direction (sampling), the contract of coupling_tc2_kernel's INV: a.x = z in the flow's output column order,
-// ONE component (c0), steps walked from the last to the first by all three roles (the ring and barrier phases stay in step);
+// work units from `ut` (one component and up to 128 rows each), steps walked from the last to the first by all three roles, which
+// walk the same units (the ring and barrier phases stay in step);
 // the gather and the coupling epilogue use the INVERSE gather-order tables; writes a.z_out = x and a.ldj_out = log-det of the
 // inverse map.  The exchange, the TMEM plan, the barriers and the weight image are those of the forward.
 // RNVP: 1 = RealNVP components (two passes per step, see the header), 0 = Glow.
 #define T3_CLK() (PROF ? clock64() : 0LL)
 template <int TANH_MODE, int PROF = 0, int INV = 0, int RNVP = 0>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupling_tc3_kernel(CouplingArgs a, TcPlan plan) {
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupling_tc3_kernel(CouplingArgs a, TcPlan plan, UnitTable ut) {
   constexpr int kPasses = RNVP ? 2 : 1;              // coupling passes per step
   extern __shared__ __align__(1024) unsigned char smem[];
   asm volatile(".reg .pred t3_p_full;" ::);
@@ -227,8 +228,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
       __syncwarp();
       if (++slot == nst) { slot = 0; par ^= 1u; }
     };
-    for (int u = pair; u < a.num_units; u += npairs) {
-      const int cb = a.c0 + (u % a.split) * a.comps_per_unit, ce = min(a.c1, cb + a.comps_per_unit);
+    for (int u = pair; u < (INV ? inverse_units(a, ut) : a.num_units); u += npairs) {
+      const int cb = INV ? __ldg(&ut.unit[u].x) : a.c0 + (u % a.split) * a.comps_per_unit;
+      const int ce = INV ? cb + 1 : min(a.c1, cb + a.comps_per_unit);
       for (int c = cb; c < ce; ++c)
         for (int pi = 0; pi < md.K * kPasses; ++pi) {
           const int kk = RNVP ? pi >> 1 : pi, net = t3_net<RNVP, INV>(pi & 1);
@@ -312,8 +314,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
       ptx::mbar_wait(bar, par, a.error_flag, code);
       ptx::tc_fence_after();
     };
-    for (int u = pair; u < a.num_units; u += npairs) {
-      const int cb = a.c0 + (u % a.split) * a.comps_per_unit, ce = min(a.c1, cb + a.comps_per_unit);
+    for (int u = pair; u < (INV ? inverse_units(a, ut) : a.num_units); u += npairs) {
+      const int cb = INV ? __ldg(&ut.unit[u].x) : a.c0 + (u % a.split) * a.comps_per_unit;
+      const int ce = INV ? cb + 1 : min(a.c1, cb + a.comps_per_unit);
       for (int c = cb; c < ce; ++c)
         for (int pi = 0; pi < md.K * kPasses; ++pi, ++units) {
           const int kk = RNVP ? pi >> 1 : pi, net = t3_net<RNVP, INV>(pi & 1);
@@ -463,14 +466,16 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
         m[0] = __ldg(&sd->in_dim); m[1] = __ldg(&sd->out_dim); m[2] = __ldg(&sd->layer[net][0].Kp); m[3] = __ldg(&sd->layer[net][2].Np);
       }
     };
-    if (pair < a.num_units) {
-      const int cb0 = a.c0 + (pair % a.split) * a.comps_per_unit;
+    if (pair < (INV ? inverse_units(a, ut) : a.num_units)) {
+      const int cb0 = INV ? __ldg(&ut.unit[pair].x) : a.c0 + (pair % a.split) * a.comps_per_unit;
       stage_pass(a.steps + cb0 * md.K + (INV ? md.K - 1 : 0), t3_net<RNVP, INV>(0), 0);
     }
-    for (int u = pair; u < a.num_units; u += npairs) {
+    for (int u = pair; u < (INV ? inverse_units(a, ut) : a.num_units); u += npairs) {
       const int tile = u / a.split, cs = u - tile * a.split;
-      const int cb = a.c0 + cs * a.comps_per_unit, ce = min(a.c1, cb + a.comps_per_unit);
-      const long long row0 = (long long)tile * kTcRows;
+      const int4 un = INV ? __ldg(ut.unit + u) : make_int4(0, 0, 0, 0);   // INV: {component, first row, rows}
+      const int cb = INV ? un.x : a.c0 + cs * a.comps_per_unit, ce = INV ? cb + 1 : min(a.c1, cb + a.comps_per_unit);
+      const long long row0 = INV ? (long long)un.y : (long long)tile * kTcRows;
+      const long long row_end = row0 + un.z;         // INV: end of the unit's rows
       const long long gr = row0 + row;
       for (int c = cb; c < ce; ++c) {
         const CompDesc* cdp = a.comps + c;
@@ -482,7 +487,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
           // INV: z arrives in the flow's OUTPUT column order, logical column j lives at physical column sigma[j]
           const int* sig = INV ? a.iblob + __ldg(&cdp->sigma_off) : nullptr;
           const long long gbase = row0 * D;
-          const long long glimit = a.B * (long long)D;
+          const long long glimit = (INV ? row_end : a.B) * (long long)D;
           const int total = kTcRows * D;
           for (int i0 = et; i0 < total; i0 += 8 * kT3EpiThreads) {
             float v[8];
@@ -517,8 +522,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
           const bool same = RNVP && (pi & 1) == 0;     // the step's second pass is next
           const StepDesc* sd_next = same ? sd : (kk + 1 < md.K) ? (INV ? sd - 1 : sd + 1)
                                     : (c + 1 < ce) ? a.steps + (c + 1) * md.K + kfirst
-                                    : (u + npairs < a.num_units) ? a.steps + (a.c0 + ((u + npairs) % a.split) * a.comps_per_unit) * md.K + kfirst
-                                                                 : nullptr;
+                                    : (u + npairs < (INV ? inverse_units(a, ut) : a.num_units))
+                                        ? a.steps + (INV ? __ldg(&ut.unit[u + npairs].x) : a.c0 + ((u + npairs) % a.split) * a.comps_per_unit) * md.K + kfirst
+                                        : nullptr;
           // mixed RealNVP networks: t = ReLU, s = tanh (as in coupling_tc2.cuh)
           const int act_kind = (md.act == GBNF_ACT_RELU || (RNVP && md.act == GBNF_ACT_MIXED && net == 0)) ? 2 : 1;
           // ---- ActNorm / eval-BatchNorm affine fused into the gather of z1 -> A0 (both CTAs build the same image); the RealNVP
@@ -752,10 +758,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kT3Threads, 1) coupl
           t2_epi_bar();                              // z2 updates, staged constants of the next pass
           e_c4 += T3_CLK() - tq;
         }
-        // ---- component log-density for this row (both CTAs hold the same z; rank 0 writes) ----
-        t2_component_logq(a, zrow, lsum, part, row, g, quad, h0col, h1col, Dv, base_off, INV ? -ldj_const : ldj_const, base_const,
-                          misc->coef, c, tile, p == 0);
-        if (p == 0 && a.z_out != nullptr && gr < a.B) {
+        // ---- component log-density for this row (inverse: the log-det of the inverse map; both CTAs hold the same z, rank 0
+        //      writes) ----
+        if (INV) t2_inverse_ldj(a, lsum, part, row, g, quad, -ldj_const, gr, row_end, p == 0);
+        else     t2_component_logq(a, zrow, lsum, part, row, g, quad, h0col, h1col, Dv, base_off, ldj_const, base_const, misc->coef, c,
+                                   tile, p == 0);
+        if (p == 0 && a.z_out != nullptr && gr < (INV ? row_end : a.B)) {
           if (INV) {   // physical == logical column order at the flow's input
             for (int j = h0col; j < h1col; ++j) a.z_out[gr * D + j] = zrow[j];
           } else {
@@ -816,24 +824,24 @@ inline int tc3_max_pairs(const TcPlan& p, int num_sms) {
 // Glow only: a profiling RealNVP handle runs the production kernel.
 inline int tc3_launch(const CouplingArgs& a, const TcPlan& p, int pairs, cudaStream_t st, int prof = 0) {
   if (a.md.nnets == 2) {
-    if (p.tanh_mode == 0) coupling_tc3_kernel<0, 0, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
-    else                  coupling_tc3_kernel<1, 0, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
+    if (p.tanh_mode == 0) coupling_tc3_kernel<0, 0, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p, UnitTable{});
+    else                  coupling_tc3_kernel<1, 0, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p, UnitTable{});
     return 0;
   }
-  if (prof) { coupling_tc3_kernel<0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p); return 0; }
-  if (p.tanh_mode == 0) coupling_tc3_kernel<0><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
-  else                  coupling_tc3_kernel<1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
+  if (prof) { coupling_tc3_kernel<0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p, UnitTable{}); return 0; }
+  if (p.tanh_mode == 0) coupling_tc3_kernel<0><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p, UnitTable{});
+  else                  coupling_tc3_kernel<1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p, UnitTable{});
   return 0;
 }
 
-inline int tc3_launch_inverse(const CouplingArgs& a, const TcPlan& p, int pairs, cudaStream_t st) {
+inline int tc3_launch_inverse(const CouplingArgs& a, const TcPlan& p, const UnitTable& ut, int pairs, cudaStream_t st) {
   if (a.md.nnets == 2) {
-    if (p.tanh_mode == 0) coupling_tc3_kernel<0, 0, 1, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
-    else                  coupling_tc3_kernel<1, 0, 1, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
+    if (p.tanh_mode == 0) coupling_tc3_kernel<0, 0, 1, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p, ut);
+    else                  coupling_tc3_kernel<1, 0, 1, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p, ut);
     return 0;
   }
-  if (p.tanh_mode == 0) coupling_tc3_kernel<0, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
-  else                  coupling_tc3_kernel<1, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p);
+  if (p.tanh_mode == 0) coupling_tc3_kernel<0, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p, ut);
+  else                  coupling_tc3_kernel<1, 0, 1><<<2 * pairs, kT3Threads, p.smem_bytes, st>>>(a, p, ut);
   return 0;
 }
 

@@ -91,7 +91,8 @@ struct gbnf_ctx {
   double* tile_offs = nullptr;   // [cap_tiles + 1]
   long long cum_cap = 0;
   int* flags_host = nullptr;     // status words in mapped pinned host memory: [0] watchdog code of a timed-out in-kernel wait,
-  int* flags = nullptr;          // [1] fp16 weight overflow (pack), [2] non-finite fp16 GEMM operand; `flags` = device alias
+  int* flags = nullptr;          // [1] fp16 weight overflow (pack), [2] non-finite fp16 GEMM operand, [3] component id out of range
+                                 // (gbnf_mixture_inverse); `flags` = device alias
   float* lse_part = nullptr;     // pipelined kernel: per-row mixture terms coef_c + log q_c (reduced by the last unit of a tile)
   unsigned int* tile_ctr = nullptr;
   long long lse_cap = 0, ctr_cap = 0;
@@ -129,6 +130,18 @@ struct gbnf_ctx {
   std::vector<TrainStep> tr_steps_h;
   std::vector<TrainPackJob> tr_pack_h;
   std::vector<WgradJob> tr_jobs_h;
+  // inverse launches (gbnf_component_inverse, gbnf_mixture_inverse): the work-unit table and, for a mixture, the rows sorted by
+  // component (counting sort of mixture.cuh) with z and the results in that order
+  int4* inv_units = nullptr;     // [inv_units_cap] {component, first row, rows}
+  int* inv_count = nullptr;      // [1] length of the table (written on the device)
+  long long inv_units_cap = 0;
+  int* mix_hist = nullptr;       // [(kMaxComponents + 1) x ceil(mix_cap / kSortRows)] per-block bin counts, then first positions
+  long long* mix_perm = nullptr; // [mix_cap] sorted position -> row
+  long long* mix_iperm = nullptr;// [mix_cap] row -> sorted position
+  float* mix_z = nullptr;        // [mix_cap][D] z in sorted order
+  float* mix_x = nullptr;        // [mix_cap][D] x in sorted order
+  float* mix_ldj = nullptr;      // [mix_cap]
+  long long mix_cap = 0;
 };
 constexpr size_t kCommBlockBytes = 4096;
 static_assert(sizeof(CommBlock) <= kCommBlockBytes, "CommBlock does not fit its slot");
@@ -169,6 +182,11 @@ int check_status(gbnf_ctx* h) {
     f[2] = 0;
     return fail(GBNF_ERR_NUMERIC, "an input or activation of an earlier launch was not finite in fp16 (|v| > 65504, inf or NaN): its "
                                   "results are invalid; standardise the data or use GBNF_GEMM_FP32");
+  }
+  if (f[3] != 0) {
+    f[3] = 0;
+    return fail(GBNF_ERR_INVALID, "a component id given to an earlier gbnf_mixture_inverse call was outside [0, n_comp): the rows "
+                                  "that carried one were not computed");
   }
   return GBNF_OK;
 }
@@ -451,6 +469,74 @@ int launch_coupling(gbnf_ctx* h, const float* x, long long B, int c0, int c1, fl
   return GBNF_OK;
 }
 
+// The checks an inverse launch over components [c0, c1) makes before anything is launched.
+int inverse_refusal(const gbnf_ctx* h, int c0, int c1) {
+  for (int c = c0; c < c1; ++c) {
+    if (!h->packed[c]) return fail(GBNF_ERR_STATE, "component " + std::to_string(c) + " has not been packed");
+    if (h->cfg.glow_invconv && !h->inv_ok[c])
+      return fail(GBNF_ERR_STATE, "inverse direction: component " + std::to_string(c) + " was packed without invconv_winv");
+  }
+  if (h->cfg.gemm_mode != GBNF_GEMM_FP32 && h->kernel == CouplingKernel::kSerial)
+    return fail(GBNF_ERR_INVALID, "inverse direction: the serial tensor-core kernel (hidden width 64, 192, 320 or 448, or depth > 1) "
+                                  "does not serve it; use GBNF_GEMM_FP32 for this configuration");
+  return GBNF_OK;
+}
+
+// Scratch of inverse launches of up to `rows` rows (`sorted`: with the counting sort of a mixture), grown and never shrunk: after
+// one call at a batch size, calls at that size allocate nothing (sampling can be captured in a CUDA graph).
+int ensure_inverse_workspace(gbnf_ctx* h, long long rows, bool sorted) {
+  const long long units = (rows + h->rows_per_cta - 1) / h->rows_per_cta + kMaxComponents;
+  if (!h->inv_count) CUDA_TRY(cudaMalloc(&h->inv_count, sizeof(int)));
+  if (units > h->inv_units_cap) {
+    cudaFree(h->inv_units);
+    h->inv_units = nullptr; h->inv_units_cap = 0;
+    CUDA_TRY(cudaMalloc(&h->inv_units, units * sizeof(int4)));
+    h->inv_units_cap = units;
+  }
+  if (sorted && rows > h->mix_cap) {
+    cudaFree(h->mix_hist); cudaFree(h->mix_perm); cudaFree(h->mix_iperm); cudaFree(h->mix_z); cudaFree(h->mix_x); cudaFree(h->mix_ldj);
+    h->mix_hist = nullptr; h->mix_perm = h->mix_iperm = nullptr; h->mix_z = h->mix_x = h->mix_ldj = nullptr; h->mix_cap = 0;
+    const long long nblk = (rows + kSortRows - 1) / kSortRows, D = h->md.D;
+    CUDA_TRY(cudaMalloc(&h->mix_hist, (kMaxComponents + 1) * nblk * sizeof(int)));
+    CUDA_TRY(cudaMalloc(&h->mix_perm, rows * sizeof(long long)));
+    CUDA_TRY(cudaMalloc(&h->mix_iperm, rows * sizeof(long long)));
+    CUDA_TRY(cudaMalloc(&h->mix_z, rows * D * sizeof(float)));
+    CUDA_TRY(cudaMalloc(&h->mix_x, rows * D * sizeof(float)));
+    CUDA_TRY(cudaMalloc(&h->mix_ldj, rows * sizeof(float)));
+    h->mix_cap = rows;
+  }
+  return GBNF_OK;
+}
+
+// One inverse launch over B rows of z whose work units (at most max_units) the handle's unit table holds.
+int launch_inverse(gbnf_ctx* h, const float* z, long long B, int max_units, float* x, float* ldj, cudaStream_t st) {
+  CouplingArgs a = coupling_args(h);
+  a.x = z; a.B = B; a.c0 = 0; a.c1 = h->cfg.C; a.z_out = x; a.ldj_out = ldj;
+  a.n_mix = 0; a.skip_c = -1;
+  const int R = h->rows_per_cta;
+  a.num_tiles = (int)((B + R - 1) / R);
+  a.split = 1; a.comps_per_unit = 1; a.num_units = max_units;
+  const UnitTable ut{h->inv_units, h->inv_count};
+  const bool pair = h->kernel == CouplingKernel::kPair;
+  const int grid = capped_grid(std::min(max_units, pair ? h->tc3_pairs : h->num_sms));     // CTAs, or CTA pairs
+  h->last_grid = pair ? 2 * grid : grid;
+  if (h->cfg.gemm_mode == GBNF_GEMM_FP32) {
+    if (R == 64) coupling_fp32_inverse_kernel<64><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max, ut);
+    else if (R == 32) coupling_fp32_inverse_kernel<32><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max, ut);
+    else coupling_fp32_inverse_kernel<16><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max, ut);
+  } else if (pair) {
+    tc3_launch_inverse(a, h->tc, ut, grid, st);
+  } else {
+    tc2_launch_inverse(a, h->tc, ut, grid, st);
+  }
+  h->launches++;
+  CUDA_TRY_H(h, cudaGetLastError());
+  return GBNF_OK;
+}
+
+// rows are independent: very large batches go through in slices, which bounds the scratch and keeps row and unit counts in an int
+constexpr long long kMaxInverseRows = 1LL << 22;
+
 }  // namespace
 
 extern "C" {
@@ -558,6 +644,8 @@ void gbnf_destroy(gbnf_handle h) {
   cudaFree(h->lse_part); cudaFree(h->tile_ctr);
   cudaFree(h->tr_w); cudaFree(h->tr_scratch); cudaFree(h->tr_steps_d); cudaFree(h->tr_pack_d); cudaFree(h->tr_jobs_d);
   cudaFree(h->cum); cudaFree(h->tile_sums); cudaFree(h->tile_offs); cudaFree(h->prof);
+  cudaFree(h->inv_units); cudaFree(h->inv_count);
+  cudaFree(h->mix_hist); cudaFree(h->mix_perm); cudaFree(h->mix_iperm); cudaFree(h->mix_z); cudaFree(h->mix_x); cudaFree(h->mix_ldj);
   delete h;
 }
 
@@ -662,37 +750,55 @@ int gbnf_component_inverse(gbnf_handle h, const float* d_z, int64_t B, int32_t c
   if (B < 0 || c < 0 || c >= h->cfg.C) return fail(GBNF_ERR_INVALID, "bad B or component index");
   if (B == 0) return GBNF_OK;
   if (!d_z || !d_x) return fail(GBNF_ERR_INVALID, "null pointer");
-  if (!h->packed[c]) return fail(GBNF_ERR_STATE, "component " + std::to_string(c) + " has not been packed");
-  if (h->cfg.glow_invconv && !h->inv_ok[c])
-    return fail(GBNF_ERR_STATE, "inverse direction: component " + std::to_string(c) + " was packed without invconv_winv");
-  const bool f16 = h->cfg.gemm_mode != GBNF_GEMM_FP32;
-  if (f16 && h->kernel == CouplingKernel::kSerial)
-    return fail(GBNF_ERR_INVALID, "inverse direction: the serial tensor-core kernel (hidden width 64, 192, 320 or 448, or depth > 1) "
-                                  "does not serve it; use GBNF_GEMM_FP32 for this configuration");
-  const bool pair = h->kernel == CouplingKernel::kPair;
+  int rc = inverse_refusal(h, c, c + 1);
+  if (rc != GBNF_OK) return rc;
   ENTER(h);
   cudaStream_t st = (cudaStream_t)stream;
-  constexpr long long kMaxRowsPerLaunch = 1LL << 22;
-  for (long long r0 = 0; r0 < B; r0 += kMaxRowsPerLaunch) {
-    const long long nb = std::min(kMaxRowsPerLaunch, (long long)B - r0);
-    CouplingArgs a = coupling_args(h);
-    a.x = d_z + r0 * h->md.D; a.B = nb; a.c0 = c; a.c1 = c + 1; a.z_out = d_x + r0 * h->md.D; a.ldj_out = d_ldj_opt ? d_ldj_opt + r0 : nullptr;
-    a.n_mix = 0; a.skip_c = -1;
-    const int R = h->rows_per_cta;
-    a.num_tiles = (int)((nb + R - 1) / R);
-    a.split = 1; a.comps_per_unit = 1; a.num_units = a.num_tiles;
-    const int grid = capped_grid(std::min(a.num_tiles, pair ? h->tc3_pairs : h->num_sms));     // CTAs, or CTA pairs
-    h->last_grid = pair ? 2 * grid : grid;
-    if (!f16) {
-      if (R == 64) coupling_fp32_inverse_kernel<64><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
-      else if (R == 32) coupling_fp32_inverse_kernel<32><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
-      else coupling_fp32_inverse_kernel<16><<<grid, kF32Threads, h->smem_bytes, st>>>(a, h->ld, h->out_max);
-    } else if (pair) {
-      tc3_launch_inverse(a, h->tc, grid, st);
-    } else {
-      tc2_launch_inverse(a, h->tc, grid, st);
-    }
+  rc = ensure_inverse_workspace(h, std::min<long long>(B, kMaxInverseRows), false);
+  if (rc != GBNF_OK) return rc;
+  const int R = h->rows_per_cta;
+  // the special case of gbnf_mixture_inverse: one component, rows in their own order, no gathers
+  for (long long r0 = 0; r0 < B; r0 += kMaxInverseRows) {
+    const long long nb = std::min(kMaxInverseRows, (long long)B - r0);
+    const int nu = (int)((nb + R - 1) / R);
+    component_units_kernel<<<grid_for(h, nu, 256), 256, 0, st>>>(c, nb, R, h->inv_units, h->inv_count);
     h->launches++;
+    rc = launch_inverse(h, d_z + r0 * h->md.D, nb, nu, d_x + r0 * h->md.D, d_ldj_opt ? d_ldj_opt + r0 : nullptr, st);
+    if (rc != GBNF_OK) return rc;
+  }
+  return GBNF_OK;
+}
+
+int gbnf_mixture_inverse(gbnf_handle h, const float* d_z, int64_t B, const int64_t* d_comp, int32_t n_comp, float* d_x,
+                         float* d_ldj_opt, void* stream) {
+  if (!h) return fail(GBNF_ERR_INVALID, "null handle");
+  if (B < 0 || n_comp < 1 || n_comp > h->cfg.C) return fail(GBNF_ERR_INVALID, "bad B or component count");
+  if (B == 0) return GBNF_OK;
+  if (!d_z || !d_comp || !d_x) return fail(GBNF_ERR_INVALID, "null pointer");
+  int rc = inverse_refusal(h, 0, n_comp);
+  if (rc != GBNF_OK) return rc;
+  ENTER(h);
+  cudaStream_t st = (cudaStream_t)stream;
+  rc = ensure_inverse_workspace(h, std::min<long long>(B, kMaxInverseRows), true);
+  if (rc != GBNF_OK) return rc;
+  const int R = h->rows_per_cta, D = h->md.D;
+  for (long long r0 = 0; r0 < B; r0 += kMaxInverseRows) {
+    const long long nb = std::min(kMaxInverseRows, (long long)B - r0);
+    const int nblk = (int)((nb + kSortRows - 1) / kSortRows);
+    const long long* comp = reinterpret_cast<const long long*>(d_comp) + r0;
+    const int gg = grid_for(h, nb * 32, kMixThreads);
+    // rows sorted by component (stable), the unit table of the sorted order, z gathered into it
+    mix_sort_count_kernel<<<nblk, kSortRows, 0, st>>>(comp, nb, n_comp, nblk, h->mix_hist, h->flags);
+    mix_sort_scan_kernel<<<1, kSortRows, 0, st>>>(h->mix_hist, nblk, n_comp, R, h->inv_units, h->inv_count);
+    mix_sort_scatter_kernel<<<nblk, kSortRows, 0, st>>>(comp, nb, n_comp, nblk, h->mix_hist, h->mix_perm, h->mix_iperm);
+    gather_rows_kernel<<<gg, kMixThreads, 0, st>>>(d_z + r0 * D, D, h->mix_perm, nb, h->mix_z);
+    h->launches += 4;
+    rc = launch_inverse(h, h->mix_z, nb, (int)((nb + R - 1) / R) + n_comp, h->mix_x, d_ldj_opt ? h->mix_ldj : nullptr, st);
+    if (rc != GBNF_OK) return rc;
+    // back to the caller's row order
+    gather_rows_kernel<<<gg, kMixThreads, 0, st>>>(h->mix_x, D, h->mix_iperm, nb, d_x + r0 * D);
+    if (d_ldj_opt) gather_rows_kernel<<<gg, kMixThreads, 0, st>>>(h->mix_ldj, 1, h->mix_iperm, nb, d_ldj_opt + r0);
+    h->launches += d_ldj_opt ? 2 : 1;
     CUDA_TRY_H(h, cudaGetLastError());
   }
   return GBNF_OK;

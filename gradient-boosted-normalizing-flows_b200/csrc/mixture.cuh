@@ -497,4 +497,105 @@ __global__ void __launch_bounds__(kMixThreads) gather_rows_kernel(const float* _
   }
 }
 
+// ---- planning of an inverse launch over many components (gbnf_mixture_inverse) ------------------------------------------------
+// A stable counting sort of the rows by component id: bins 0 .. n_comp - 1 are the components, bin n_comp takes the ids outside
+// [0, n_comp) (status word [3] is raised and their rows are left out of the work units).  hist is bin-major [n_comp + 1][nblk]
+// over blocks of kSortRows rows; the scan turns it into each (bin, block)'s first sorted position and writes the unit table.
+constexpr int kSortRows = 1024;   // rows per block of the count and scatter kernels, one per thread
+
+__device__ __forceinline__ int sort_bin(const long long* comp, long long i, long long B, int n_comp) {
+  if (i >= B) return -1;
+  const long long v = comp[i];
+  return (v < 0 || v >= n_comp) ? n_comp : (int)v;
+}
+
+__global__ void __launch_bounds__(kSortRows) mix_sort_count_kernel(const long long* __restrict__ comp, long long B, int n_comp,
+                                                                  int nblk, int* __restrict__ hist, int* status) {
+  __shared__ int cnt[kMaxComponents + 1];
+  for (int b = threadIdx.x; b <= n_comp; b += blockDim.x) cnt[b] = 0;
+  __syncthreads();
+  const int v = sort_bin(comp, (long long)blockIdx.x * kSortRows + threadIdx.x, B, n_comp);
+  if (v == n_comp) *reinterpret_cast<volatile int*>(status + 3) = 1;
+  if (v >= 0) atomicAdd(&cnt[v], 1);
+  __syncthreads();
+  for (int b = threadIdx.x; b <= n_comp; b += blockDim.x) hist[(long long)b * nblk + blockIdx.x] = cnt[b];
+}
+
+// One block: exclusive scan of hist in place, then the unit table -- component c's sorted segment cut into ceil(count_c / R)
+// units of R rows (the last one shorter), components in order, empty components without units.  *n_units = the table's length
+// (<= ceil(B / R) + n_comp).
+__global__ void __launch_bounds__(kSortRows) mix_sort_scan_kernel(int* __restrict__ hist, int nblk, int n_comp, int R,
+                                                                 int4* __restrict__ units, int* __restrict__ n_units) {
+  __shared__ int wsum[kSortRows / 32];
+  __shared__ int first[kMaxComponents + 1];    // first sorted row of each bin
+  __shared__ int ufirst[kMaxComponents + 1];   // first unit of each component, then the unit count
+  const int N = (n_comp + 1) * nblk;
+  const int per = (N + kSortRows - 1) / kSortRows;
+  const int lo = min(N, (int)threadIdx.x * per), hi = min(N, lo + per);
+  int s = 0;
+  for (int i = lo; i < hi; ++i) s += hist[i];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  int inc = s;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += t; }
+  if (lane == 31) wsum[wid] = inc;
+  __syncthreads();
+  if (wid == 0) {
+    const int w = wsum[lane];
+    int wi = w;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, wi, o); if (lane >= o) wi += t; }
+    wsum[lane] = wi - w;
+  }
+  __syncthreads();
+  int run = wsum[wid] + inc - s;
+  for (int i = lo; i < hi; ++i) { const int v = hist[i]; hist[i] = run; run += v; }
+  __syncthreads();
+  for (int b = threadIdx.x; b <= n_comp; b += blockDim.x) first[b] = hist[(long long)b * nblk];
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int t = 0;
+    for (int c = 0; c < n_comp; ++c) { ufirst[c] = t; t += (first[c + 1] - first[c] + R - 1) / R; }
+    ufirst[n_comp] = t;
+    *n_units = t;
+  }
+  __syncthreads();
+  for (int c = 0; c < n_comp; ++c) {
+    const int cnt = first[c + 1] - first[c], nu = ufirst[c + 1] - ufirst[c];
+    for (int t = threadIdx.x; t < nu; t += blockDim.x) units[ufirst[c] + t] = make_int4(c, first[c] + t * R, min(R, cnt - t * R), 0);
+  }
+}
+
+// perm[position] = row and iperm[row] = position: a row's position is its bin's first position in its block plus the rows of the
+// same bin before it in the block (earlier warps' counts, then its rank among its warp's matching lanes), so the order is stable.
+__global__ void __launch_bounds__(kSortRows) mix_sort_scatter_kernel(const long long* __restrict__ comp, long long B, int n_comp,
+                                                                    int nblk, const int* __restrict__ hist,
+                                                                    long long* __restrict__ perm, long long* __restrict__ iperm) {
+  __shared__ int wcnt[kSortRows / 32][kMaxComponents + 1];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const long long i = (long long)blockIdx.x * kSortRows + threadIdx.x;
+  const int v = sort_bin(comp, i, B, n_comp);
+  const unsigned peers = __match_any_sync(0xffffffffu, v);
+  const int rank = __popc(peers & ((1u << lane) - 1u));
+  for (int w = 0; w < kSortRows / 32; ++w)
+    for (int b = threadIdx.x; b <= n_comp; b += blockDim.x) wcnt[w][b] = 0;
+  __syncthreads();
+  if (v >= 0 && rank == 0) wcnt[wid][v] = __popc(peers);
+  __syncthreads();
+  if (v >= 0) {
+    long long pos = hist[(long long)v * nblk + blockIdx.x] + rank;
+    for (int w = 0; w < wid; ++w) pos += wcnt[w][v];
+    perm[pos] = i;
+    iperm[i] = pos;
+  }
+}
+
+// The unit table of ONE component over rows in their own order (gbnf_component_inverse): unit t = rows [t R, min((t + 1) R, B)).
+__global__ void component_units_kernel(int c, long long B, int R, int4* __restrict__ units, int* __restrict__ n_units) {
+  const int nu = (int)((B + R - 1) / R);
+  for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < nu; t += gridDim.x * blockDim.x)
+    units[t] = make_int4(c, t * R, (int)min((long long)R, B - (long long)t * R), 0);
+  if (blockIdx.x == 0 && threadIdx.x == 0) *n_units = nu;
+}
+
 }  // namespace gbnf

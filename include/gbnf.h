@@ -13,9 +13,10 @@
  *   - every launch goes on the caller's stream (`stream` is a cudaStream_t passed as void*); no entry point
  *     synchronises unless documented (gbnf_pack_component in the f16 modes, gbnf_check_status, the diagnostics);
  *   - every entry point runs on the handle's device and restores the caller's current device before returning;
- *   - the kernels report through three status words in mapped host memory, read (without a synchronisation) at the
+ *   - the kernels report through status words in mapped host memory, read (without a synchronisation) at the
  *     top of every entry point: an in-kernel watchdog timeout (GBNF_ERR_CUDA, with the code of the wait that
- *     timed out) or a value that fp16 cannot hold entering a tensor-core GEMM operand (GBNF_ERR_NUMERIC) is
+ *     timed out), a value that fp16 cannot hold entering a tensor-core GEMM operand (GBNF_ERR_NUMERIC) or a component id
+ *     outside [0, n_comp) given to gbnf_mixture_inverse (GBNF_ERR_INVALID) is
  *     reported by the first call made after the offending launch finished; gbnf_check_status() synchronises the
  *     stream and reports at once;
  *   - fp16 tensor-core modes: inputs, activations and weights must be finite in fp16 (|v| <= 65504); density data
@@ -159,6 +160,19 @@ int gbnf_component_logq(gbnf_handle h, const float* d_x, int64_t B, int32_t c0, 
  * 512 < h <= 1024, Glow and RealNVP); handles that run the serial tensor-core kernel (depth > 1, or h = 64 / 192 / 320 /
  * 448) return GBNF_ERR_INVALID. */
 int gbnf_component_inverse(gbnf_handle h, const float* d_z, int64_t B, int32_t c, float* d_x, float* d_ldj_opt, void* stream);
+
+/* x[i] = f_{comp[i]}^{-1}(z[i]) for every row i; comp[i] in [0, n_comp).  One coupling launch over all components.  No host
+   synchronisation.  The log-det of the inverse map goes to d_ldj_opt when it is not NULL.
+ * Sampling from the whole mixture (models/boosted_flow.py:209-218 with a component per sample): d_comp is int64 [B] (device), in
+ * any order.  The rows are sorted by component on the device (a stable counting sort), z is gathered into that order, one inverse
+ * launch covers every component's rows, and x / ldj are gathered back to the caller's order; each row gets the bits
+ * gbnf_component_inverse gives it.  Components 0 .. n_comp - 1 must be packed, and served as for gbnf_component_inverse (the same
+ * refusals, before anything is written).  An id outside [0, n_comp) is found on the device: its rows are left out and the next
+ * entry point, or gbnf_check_status, returns GBNF_ERR_INVALID.  The scratch (8 D + 20 bytes a row, up to 2^22 rows
+ * a launch; larger batches go through in slices) is kept on the handle and grows with B: after one call at a batch size, calls
+ * at that size allocate nothing, so they can be captured in a CUDA graph. */
+int gbnf_mixture_inverse(gbnf_handle h, const float* d_z, int64_t B, const int64_t* d_comp, int32_t n_comp,
+                         float* d_x, float* d_ldj_opt, void* stream);
 
 /* Mixture log-density from materialised per-component log q (d_logq is [B, ld], first n_comp columns used):
  * the 2-term logsumexp recursion of density_experiment.py:612-622 / :561-571 evaluated in its flat form
