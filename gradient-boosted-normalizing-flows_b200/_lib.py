@@ -71,6 +71,10 @@ SIGNATURES = {
     "gbnf_weight_apply": (C.c_int, [_vp, _vp, _i64, _vp, _f32, _f32, _i32, _vp, _vp, _vp]),
     "gbnf_weight_renorm": (C.c_int, [_vp, _vp, _i64, _vp, _i32, _vp]),
     "gbnf_component_backward": (C.c_int, [_vp, _i32, C.POINTER(ComponentParams), _vp, _i64, _vp, _vp, C.POINTER(StepGrads), _vp, _vp]),
+    "gbnf_component_inverse_backward": (C.c_int, [_vp, _i32, C.POINTER(ComponentParams), _vp, _i64, _vp, _vp, C.POINTER(StepGrads),
+                                                  _vp, _vp]),
+    "gbnf_mixture_inverse_backward": (C.c_int, [_vp, C.POINTER(ComponentParams), _vp, _i64, _vp, _i32, _vp, _vp,
+                                                C.POINTER(C.POINTER(StepGrads)), _vp, _vp]),
     "gbnf_comm_local_handle": (C.c_int, [_vp, _i64, _vp]),
     "gbnf_comm_init": (C.c_int, [_vp, _i32, _i32, _vp]),
     "gbnf_comm_destroy": (C.c_int, [_vp]),

@@ -71,6 +71,35 @@ class _FusedComponentFlow(torch.autograd.Function):
         return (None, None, dx) + tuple(grads[id(p)] if p.requires_grad else None for p in ctx.params)
 
 
+class _FusedMixtureInverse(torch.autograd.Function):
+    """(x, ldj_inv) with x[i] = flows[comp[i]]^{-1}(z[i]): the reparameterised sample of BoostedFlow.rsample, both directions
+    served by the library -- the forward is gbnf_mixture_inverse (nothing saved but z and the ids), the backward recomputes
+    in-kernel (gbnf_mixture_inverse_backward) and returns the gradients of every drawn component's parameters that require grad,
+    and dL/dz when z requires grad.  The inverse counterpart of _FusedComponentFlow."""
+
+    @staticmethod
+    def forward(ctx, model, n_comp, z, comp, *params):
+        with torch.no_grad():
+            x, ldj = model.mixture_inverse(z, comp, n_comp)
+        ctx.model, ctx.n_comp, ctx.params = model, n_comp, params
+        ctx.save_for_backward(z, comp)
+        return x, ldj
+
+    @staticmethod
+    def backward(ctx, dx, dldj):
+        z, comp = ctx.saved_tensors
+        model, n = ctx.model, ctx.n_comp
+        dx = torch.zeros_like(z) if dx is None else dx.contiguous().float()
+        dldj = torch.zeros(z.shape[0], device=z.device) if dldj is None else dldj.contiguous().float()
+        trained = {c for c in range(n) if any(p.requires_grad for p in model.flows[c].parameters())}
+        grads, dz = model._mixture_inverse_backward(z, comp, n, dx, dldj, trained, with_dz=ctx.needs_input_grad[2])
+        return (None, None, dz, None) + tuple(grads.get(id(p)) if p.requires_grad else None for p in ctx.params)
+
+
+# the inverse backward's largest batch (gbnf_mixture_inverse_backward); rsample differentiates larger ones through autograd
+FUSED_INVERSE_MAX_ROWS = 1 << 22
+
+
 class BoostedFlow(nn.Module):
     def __init__(self, args, gemm_mode=None):
         super().__init__()
@@ -184,13 +213,22 @@ class BoostedFlow(nn.Module):
         """Gradients of component c's parameters for upstream (dz, dldj) through gbnf_component_backward:
         ({id(param): grad}, dL/dx if with_dx else None).  Every Linear layer of every coupling network is passed, depth + 2 per
         network at any coupling_network_depth."""
-        lib = _lib.load()
         device = x.device
         h = self.handle(device)
+        keep, out = [], {}
+        cp, garr = self._backward_arrays(c, device, keep, out)
+        dx = torch.empty_like(x, dtype=torch.float32) if with_dx else None
+        _lib.check(_lib.load().gbnf_component_backward(h, c, C.byref(cp), _ptr(x), x.shape[0], _ptr(dz), _ptr(dldj),
+                                                       C.cast(garr, C.POINTER(_lib.StepGrads)), _ptr(dx), _stream(device)))
+        self._keepalive[("bwd", c)] = keep
+        return out, dx
+
+    def _backward_arrays(self, c, device, keep, out, with_grads=True):
+        """(gbnf_component_params, gbnf_step_grads array or None) of component c for the fused backward calls: the raw parameters
+        (device copies appended to `keep`) and, with_grads, fresh gradient buffers registered in out[id(param)]."""
         steps = self._component_tensors(c)
         parr = (_lib.StepParams * len(steps))()
-        garr = (_lib.StepGrads * len(steps))()
-        keep, out = [], {}
+        garr = (_lib.StepGrads * len(steps))() if with_grads else None
 
         def dev(t, dtype=torch.float32):
             t = t.detach().to(device=device, dtype=dtype).contiguous()
@@ -203,23 +241,43 @@ class BoostedFlow(nn.Module):
             return g.data_ptr()
 
         for k, (d, step) in enumerate(zip(steps, self.flows[c].steps())):
-            sp, sg = parr[k], garr[k]
+            sp = parr[k]
             if "an_bias" in d:
                 sp.an_bias, sp.an_logs = dev(d["an_bias"].reshape(-1)), dev(d["an_logs"].reshape(-1))
                 sp.perm = dev(d["perm"], torch.int64)
-                sg.an_bias, sg.an_logs = grad_of(step.actnorm.bias), grad_of(step.actnorm.logs)
+                if with_grads:
+                    garr[k].an_bias, garr[k].an_logs = grad_of(step.actnorm.bias), grad_of(step.actnorm.logs)
+            if "bn" in d:                                  # passed so that the library refuses these steps
+                sp.bn_log_gamma, sp.bn_beta, sp.bn_mean, sp.bn_var = [dev(t) for t in d["bn"]]
             for n, lins in enumerate(d["nets"]):          # Glow: the block; RealNVP: t_net, s_net
                 for l, lin in enumerate(lins):
                     sp.W[n][l], sp.b[n][l] = dev(lin.weight), dev(lin.bias)
-                    sg.W[n][l], sg.b[n][l] = grad_of(lin.weight), grad_of(lin.bias)
+                    if with_grads:
+                        garr[k].W[n][l], garr[k].b[n][l] = grad_of(lin.weight), grad_of(lin.bias)
         cp = _lib.ComponentParams()
         cp.flip_init, cp.n_steps = getattr(self.flows[c], "flip_init", 0), len(steps)
         cp.steps = C.cast(parr, C.POINTER(_lib.StepParams))
-        dx = torch.empty_like(x, dtype=torch.float32) if with_dx else None
-        _lib.check(lib.gbnf_component_backward(h, c, C.byref(cp), _ptr(x), x.shape[0], _ptr(dz), _ptr(dldj),
-                                               C.cast(garr, C.POINTER(_lib.StepGrads)), _ptr(dx), _stream(device)))
-        self._keepalive[("bwd", c)] = keep
-        return out, dx
+        keep.append(parr)
+        return cp, garr
+
+    def _mixture_inverse_backward(self, z, comp, n_comp, dx, dldj, trained, with_dz=False):
+        """Gradients through x[i] = flows[comp[i]]^{-1}(z[i]) for upstream (dx, dldj) through gbnf_mixture_inverse_backward:
+        ({id(param): grad} for the components in `trained`, dL/dz if with_dz else None)."""
+        device = z.device
+        h = self.handle(device)
+        keep, out = [], {}
+        parr = (_lib.ComponentParams * n_comp)()
+        gptrs = (C.POINTER(_lib.StepGrads) * n_comp)()
+        for c in range(n_comp):
+            parr[c], garr = self._backward_arrays(c, device, keep, out, with_grads=c in trained)
+            if garr is not None:
+                keep.append(garr)
+                gptrs[c] = C.cast(garr, C.POINTER(_lib.StepGrads))
+        dz = torch.empty_like(z) if with_dz else None
+        _lib.check(_lib.load().gbnf_mixture_inverse_backward(h, parr, _ptr(z), z.shape[0], _ptr(comp), n_comp, _ptr(dx), _ptr(dldj),
+                                                             gptrs, _ptr(dz), _stream(device)))
+        self._keepalive["inv_bwd"] = keep
+        return out, dz
 
     def decode(self, z, y_onehot, temperature, components):
         """x = flows[c]^{-1}(z) for ONE component c (models/boosted_flow.py:209-218; upstream's `y_onhot` keyword typo is not
@@ -265,6 +323,39 @@ class BoostedFlow(nn.Module):
         n_comp = self.num_components if self.all_trained else self.component + 1
         comp = self.assign_components(u, n_comp)
         return self.mixture_inverse(z.contiguous(), comp, n_comp)[0], comp
+
+    def rsample(self, n, u=None, z=None, temperature=1.0, generator=None, comp=None):
+        """Reparameterised draws from the boosted mixture: (x, ldj_inv, comp) with x[i] = flows[comp[i]]^{-1}(z[i]) and the log-det
+        of the inverse map, so that log q_c(x) = log N(z) - ldj_inv (reverse-KL / density-matching losses).  Draws u, z and the
+        component ids as sample() does (comp, when given, is used instead of u).  Differentiable: gradients reach the parameters of
+        every drawn component that requires grad, and z (or the temperature) when it requires grad.  Inside the fused backward's
+        envelope (_fused_backward_ok) x and ldj are bitwise those of mixture_inverse and the backward runs in the library
+        (gbnf_mixture_inverse_backward); elsewhere, or with args.fused_backward = False, each component's rows go through its
+        inverse_autograd (the parameters' dtype, one host synchronisation for the row counts)."""
+        dev = self.rho.device
+        n_comp = self.num_components if self.all_trained else self.component + 1
+        if comp is None:
+            if u is None:
+                u = torch.rand(n, dtype=torch.float64, device=dev, generator=generator)
+            comp = self.assign_components(u, n_comp)
+        if z is None:
+            z = torch.randn((n, self.z_size), device=dev, generator=generator) * temperature
+        if self._fused_backward_ok(z) and z.shape[0] <= FUSED_INVERSE_MAX_ROWS:
+            params = [p for c in range(n_comp) for p in self.flows[c].parameters()]
+            x, ldj = _FusedMixtureInverse.apply(self, n_comp, z.contiguous(), comp, *params)
+            return x, ldj, comp
+        if bool(((comp < 0) | (comp >= n_comp)).any()):
+            raise ValueError(f"rsample: component ids must lie in [0, {n_comp})")
+        order = torch.argsort(comp, stable=True)
+        counts = torch.bincount(comp, minlength=n_comp).tolist()
+        xs, ls = [], []
+        for c, rows in zip(range(n_comp), torch.split(order, counts)):
+            if len(rows):
+                xc, lc = self.flows[c].inverse_autograd(z[rows])
+                xs.append(xc)
+                ls.append(lc)
+        back = torch.argsort(order)
+        return torch.cat(xs)[back], torch.cat(ls)[back], comp
 
     @torch.no_grad()
     def mixture_inverse(self, z, comp, n=None):

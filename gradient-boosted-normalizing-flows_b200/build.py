@@ -8,7 +8,7 @@ CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libgbnf_b200.so")
 SOURCES = ["gbnf_api.cu"]
 HEADERS = ["common.cuh", "pack.cuh", "mixture.cuh", "actnorm_init.cuh", "coupling_fp32.cuh", "coupling_tc.cuh", "coupling_tc2.cuh", "coupling_tc3.cuh", "coupling_tc4.cuh", "coupling_tc5.cuh", "train_bwd.cuh",
-           "tc_ptx.cuh"]
+           "inverse_bwd.cuh", "tc_ptx.cuh"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
 

@@ -19,6 +19,7 @@
 #include "coupling_tc4.cuh"
 #include "coupling_tc5.cuh"
 #include "train_bwd.cuh"
+#include "inverse_bwd.cuh"
 
 using namespace gbnf;
 
@@ -130,6 +131,18 @@ struct gbnf_ctx {
   std::vector<TrainStep> tr_steps_h;
   std::vector<TrainPackJob> tr_pack_h;
   std::vector<WgradJob> tr_jobs_h;
+  // backward of the inverse map (gbnf_component_inverse_backward, gbnf_mixture_inverse_backward): the (component, step)
+  // descriptors, pack and weight-gradient jobs (ib_cap entries each), and the table of 16-row work units
+  TrainStep* ib_steps_d = nullptr;
+  TrainPackJob* ib_pack_d = nullptr;
+  RangedWgradJob* ib_jobs_d = nullptr;
+  long long ib_cap = 0;
+  int4* ib_units = nullptr;      // [ib_units_cap] {component slot, first sorted position, rows}
+  int* ib_count = nullptr;       // [1] length of the table (written on the device)
+  long long ib_units_cap = 0;
+  std::vector<TrainStep> ib_steps_h;
+  std::vector<TrainPackJob> ib_pack_h;
+  std::vector<RangedWgradJob> ib_jobs_h;
   // inverse launches (gbnf_component_inverse, gbnf_mixture_inverse): the work-unit table and, for a mixture, the rows sorted by
   // component (counting sort of mixture.cuh) with z and the results in that order
   int4* inv_units = nullptr;     // [inv_units_cap] {component, first row, rows}
@@ -534,8 +547,50 @@ int launch_inverse(gbnf_ctx* h, const float* z, long long B, int max_units, floa
   return GBNF_OK;
 }
 
+// Geometry of coupling step k of component c for the fused backward kernels (train_bwd.cuh, inverse_bwd.cuh): RealNVP steps
+// alternate |z1| / |z2| when D is odd (flipped iff (k + c) is odd, models/realnvp.py:37-43); layer l maps Kd[l] -> Nn[l]: in_dim
+// -> h, then depth times h -> h, then h -> the coupling's output width.  wfloats counts the step's fp32 weight copies (both layouts
+// and the padded biases of every network).
+struct BwdGeo { int in_dim, out_dim, Kd[GBNF_MAX_LAYERS], Nn[GBNF_MAX_LAYERS], Kp[GBNF_MAX_LAYERS], Np[GBNF_MAX_LAYERS],
+                NKp[GBNF_MAX_LAYERS], KNp[GBNF_MAX_LAYERS]; long long wfloats; };
+BwdGeo bwd_geo(const gbnf_config& cf, int c, int k) {
+  const bool glow = cf.kind == GBNF_KIND_GLOW;
+  const int hD0 = cf.D / 2, hD1 = cf.D - hD0, L = cf.depth + 2;
+  BwdGeo g{};
+  const bool flipped = !glow && (((k + c) % 2) > 0);
+  g.in_dim = flipped ? hD1 : hD0; g.out_dim = flipped ? hD0 : hD1;
+  const int n3 = glow ? ((cf.coupling == GBNF_COUPLING_AFFINE) ? 2 * g.out_dim : g.out_dim) : g.out_dim;
+  for (int l = 0; l < L; ++l) {
+    g.Kd[l] = (l == 0) ? g.in_dim : cf.h; g.Nn[l] = (l == L - 1) ? n3 : cf.h;
+    g.Kp[l] = round_up(g.Kd[l], kF32KT); g.Np[l] = round_up(g.Nn[l], kF32NT);
+    g.NKp[l] = round_up(g.Nn[l], kF32KT); g.KNp[l] = round_up(g.Kd[l], kF32NT);
+    g.wfloats += (long long)g.Kp[l] * g.Np[l] + (long long)g.NKp[l] * g.KNp[l] + g.Np[l];
+  }
+  g.wfloats *= glow ? 1 : 2;
+  return g;
+}
+
 // rows are independent: very large batches go through in slices, which bounds the scratch and keeps row and unit counts in an int
 constexpr long long kMaxInverseRows = 1LL << 22;
+
+// The fused backward kernels' fp32 weight copies (need_w floats) and L2 scratch (rows x per_row x K floats), grown and never
+// shrunk; shared by gbnf_component_backward and the inverse backward (calls on one handle are stream-ordered).
+int ensure_backward_buffers(gbnf_ctx* h, long long need_w, long long B, long long per_row) {
+  if (need_w > h->tr_w_floats) {
+    if (h->tr_w) cudaFree(h->tr_w);
+    h->tr_w = nullptr; h->tr_w_floats = 0;
+    CUDA_TRY_H(h, cudaMalloc(&h->tr_w, need_w * sizeof(float)));
+    h->tr_w_floats = need_w;
+  }
+  if (B > h->tr_rows || per_row > h->tr_per_row) {
+    if (h->tr_scratch) cudaFree(h->tr_scratch);
+    h->tr_scratch = nullptr; h->tr_rows = 0;
+    const long long rows = std::max<long long>(std::max<long long>(B, h->tr_rows), 1024);
+    CUDA_TRY_H(h, cudaMalloc(&h->tr_scratch, (size_t)rows * per_row * h->cfg.K * sizeof(float)));
+    h->tr_rows = rows; h->tr_per_row = per_row;
+  }
+  return GBNF_OK;
+}
 
 }  // namespace
 
@@ -645,6 +700,7 @@ void gbnf_destroy(gbnf_handle h) {
   cudaFree(h->tr_w); cudaFree(h->tr_scratch); cudaFree(h->tr_steps_d); cudaFree(h->tr_pack_d); cudaFree(h->tr_jobs_d);
   cudaFree(h->cum); cudaFree(h->tile_sums); cudaFree(h->tile_offs); cudaFree(h->prof);
   cudaFree(h->inv_units); cudaFree(h->inv_count);
+  cudaFree(h->ib_steps_d); cudaFree(h->ib_pack_d); cudaFree(h->ib_jobs_d); cudaFree(h->ib_units); cudaFree(h->ib_count);
   cudaFree(h->mix_hist); cudaFree(h->mix_perm); cudaFree(h->mix_iperm); cudaFree(h->mix_z); cudaFree(h->mix_x); cudaFree(h->mix_ldj);
   delete h;
 }
@@ -911,32 +967,17 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
   if (B <= 0) return fail(GBNF_ERR_INVALID, "empty batch");
   ENTER(h);
   cudaStream_t st = (cudaStream_t)stream;
-  const int K = cf.K, D = cf.D, hD0 = D / 2, hD1 = D - hD0;
+  const int K = cf.K, D = cf.D;
   const int nnets = glow ? 1 : 2;
   const int L = cf.depth + 2;                  // Linear layers per coupling network (gbnf_create bounds L <= GBNF_MAX_LAYERS)
   const int hp = round_up(cf.h, 64);
-  // per-step geometry: RealNVP steps alternate |z1| / |z2| when D is odd (flipped iff (k + c) is odd, models/realnvp.py:37-43);
-  // layer l maps Kd[l] -> Nn[l]: in_dim -> h, then depth times h -> h, then h -> the coupling's output width
-  struct Geo { int in_dim, out_dim, Kd[GBNF_MAX_LAYERS], Nn[GBNF_MAX_LAYERS], Kp[GBNF_MAX_LAYERS], Np[GBNF_MAX_LAYERS],
-               NKp[GBNF_MAX_LAYERS], KNp[GBNF_MAX_LAYERS]; long long wfloats; };
-  std::vector<Geo> geo(K);
+  std::vector<BwdGeo> geo(K);
   long long need_w = 1024;
   int ldz1 = 0;
   for (int k = 0; k < K; ++k) {
-    Geo& g = geo[k];
-    const bool flipped = !glow && (((k + c) % 2) > 0);
-    g.in_dim = flipped ? hD1 : hD0; g.out_dim = flipped ? hD0 : hD1;
-    const int n3 = glow ? ((cf.coupling == GBNF_COUPLING_AFFINE) ? 2 * g.out_dim : g.out_dim) : g.out_dim;
-    g.wfloats = 0;
-    for (int l = 0; l < L; ++l) {
-      g.Kd[l] = (l == 0) ? g.in_dim : cf.h; g.Nn[l] = (l == L - 1) ? n3 : cf.h;
-      g.Kp[l] = round_up(g.Kd[l], kF32KT); g.Np[l] = round_up(g.Nn[l], kF32NT);
-      g.NKp[l] = round_up(g.Nn[l], kF32KT); g.KNp[l] = round_up(g.Kd[l], kF32NT);
-      g.wfloats += (long long)g.Kp[l] * g.Np[l] + (long long)g.NKp[l] * g.KNp[l] + g.Np[l];
-    }
-    g.wfloats *= nnets;
-    need_w += g.wfloats;
-    ldz1 = std::max(ldz1, g.Kp[0]);
+    geo[k] = bwd_geo(cf, c, k);
+    need_w += geo[k].wfloats;
+    ldz1 = std::max(ldz1, geo[k].Kp[0]);
   }
   // every refusal comes before the first allocation, memset or copy: a refused call leaves the handle and `grads` untouched
   for (int k = 0; k < K; ++k) {
@@ -958,21 +999,10 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
     return fail(GBNF_ERR_INVALID, "fused backward: the shared-memory history of K = " + std::to_string(K) + " steps at D = " + std::to_string(D) +
                                   ", h = " + std::to_string(cf.h) + " needs " + std::to_string(smem) + " bytes > " + std::to_string(kTrMaxSmem) +
                                   " (train through the caller's autograd)");
-  if (need_w > h->tr_w_floats) {
-    if (h->tr_w) cudaFree(h->tr_w);
-    h->tr_w = nullptr; h->tr_w_floats = 0;
-    CUDA_TRY_H(h, cudaMalloc(&h->tr_w, need_w * sizeof(float)));
-    h->tr_w_floats = need_w;
-  }
   // per row and step: z1, then per network depth + 1 hidden activations, as many hidden d pre-activations and the last layer's
   const long long per_row = (long long)ldz1 + nnets * (2LL * (L - 1) * hp + 64);
-  if (B > h->tr_rows || per_row > h->tr_per_row) {
-    if (h->tr_scratch) cudaFree(h->tr_scratch);
-    h->tr_scratch = nullptr; h->tr_rows = 0;
-    const long long rows = std::max<long long>(std::max<long long>(B, h->tr_rows), 1024);
-    CUDA_TRY_H(h, cudaMalloc(&h->tr_scratch, (size_t)rows * per_row * K * sizeof(float)));
-    h->tr_rows = rows; h->tr_per_row = per_row;
-  }
+  int rc = ensure_backward_buffers(h, need_w, B, per_row);
+  if (rc != GBNF_OK) return rc;
   const int njobs = K * nnets * L;
   if (!h->tr_steps_d || njobs > h->tr_njobs) {
     if (h->tr_steps_d) { cudaFree(h->tr_steps_d); cudaFree(h->tr_pack_d); cudaFree(h->tr_jobs_d); }
@@ -988,7 +1018,7 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
   for (int k = 0; k < K; ++k) {
     const gbnf_step_params& sp = p->steps[k];
     const gbnf_step_grads& sg = grads[k];
-    const Geo& g = geo[k];
+    const BwdGeo& g = geo[k];
     TrainStep& ts = h->tr_steps_h[k];
     if (glow) {
       ts.an_bias = sp.an_bias; ts.an_logs = sp.an_logs; ts.perm = (const long long*)sp.perm;
@@ -1038,6 +1068,188 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
   h->launches += 3;
   CUDA_TRY_H(h, cudaGetLastError());
   return GBNF_OK;
+}
+
+}  // extern "C"
+
+// ---- sampling with gradients: backward of the inverse map (inverse_bwd.cuh) --------------------------------------------------------
+namespace {
+
+// Shared by gbnf_component_inverse_backward (one component c0, rows in their own order: d_comp == NULL) and
+// gbnf_mixture_inverse_backward (components 0 .. n - 1, rows sorted by d_comp on the device).  p[i] / grads[i] belong to component
+// c0 + i; grads[i] == NULL: no parameter gradient for it (its rows still get dL/dz).
+int inverse_backward(gbnf_ctx* h, int c0, int n, const gbnf_component_params* p, const gbnf_step_grads* const* grads,
+                     const float* d_z, long long B, const long long* d_comp, const float* d_dx, const float* d_dldj, float* d_dz,
+                     cudaStream_t st) {
+  const gbnf_config& cf = h->cfg;
+  const bool glow = cf.kind == GBNF_KIND_GLOW;
+  if (cf.glow_invconv || cf.act == GBNF_ACT_RESIDUAL || cf.h > 512 || cf.D > 64)
+    return fail(GBNF_ERR_INVALID, "inverse backward: Glow (with a permutation) or RealNVP (without BatchNorm) components with "
+                                  "coupling_network_depth 0 to 4, tanh / relu (RealNVP: or mixed) networks, h <= 512, D <= 64 (others "
+                                  "differentiate the sample through the caller's autograd)");
+  if (B < 1 || B > kMaxInverseRows) return fail(GBNF_ERR_INVALID, "inverse backward: B must be in [1, 2^22] (split larger batches)");
+  const int K = cf.K, D = cf.D, nnets = glow ? 1 : 2, L = cf.depth + 2, hp = round_up(cf.h, 64);
+  // every refusal comes before the first allocation, memset or copy: a refused call leaves the handle, `grads` and dz untouched
+  std::vector<BwdGeo> geo((size_t)n * K);
+  long long need_w = 1024;
+  int ldz1 = 0;
+  for (int i = 0; i < n; ++i) {
+    const int c = c0 + i;
+    if (!p[i].steps || p[i].n_steps != K) return fail(GBNF_ERR_INVALID, "component " + std::to_string(c) + ": null steps or n_steps != K");
+    if (!glow && p[i].flip_init != c) return fail(GBNF_ERR_INVALID, "RealNVP component c must have flip_init == c (models/boosted_flow.py:46)");
+    if (!h->packed[c]) return fail(GBNF_ERR_STATE, "component " + std::to_string(c) + " has not been packed");
+    for (int k = 0; k < K; ++k) {
+      const gbnf_step_params& sp = p[i].steps[k];
+      const gbnf_step_grads* sg = grads[i] ? grads[i] + k : nullptr;
+      if (glow) {
+        if (!sp.an_bias || !sp.an_logs || !sp.perm || (sg && (!sg->an_bias || !sg->an_logs)))
+          return fail(GBNF_ERR_INVALID, "glow step needs ActNorm / perm / gradient pointers");
+      } else if (sp.bn_log_gamma || sp.bn_beta || sp.bn_mean || sp.bn_var) {
+        return fail(GBNF_ERR_INVALID, "inverse backward: RealNVP steps with BatchNorm differentiate the sample through the caller's autograd");
+      }
+      for (int net = 0; net < nnets; ++net)
+        for (int l = 0; l < L; ++l)
+          if (!sp.W[net][l] || !sp.b[net][l] || (sg && (!sg->W[net][l] || !sg->b[net][l])))
+            return fail(GBNF_ERR_INVALID, "missing Linear weight / bias / gradient pointer");
+      BwdGeo& g = geo[(size_t)i * K + k];
+      g = bwd_geo(cf, c, k);
+      need_w += g.wfloats;
+      ldz1 = std::max(ldz1, g.Kp[0]);
+    }
+  }
+  const int ld = std::max(hp, ldz1) + 4;
+  const size_t smem = train_bwd_smem_bytes(K, D, nnets, ld);
+  if (smem > kTrMaxSmem)
+    return fail(GBNF_ERR_INVALID, "inverse backward: the shared-memory history of K = " + std::to_string(K) + " steps at D = " + std::to_string(D) +
+                                  ", h = " + std::to_string(cf.h) + " needs " + std::to_string(smem) + " bytes > " + std::to_string(kTrMaxSmem) +
+                                  " (differentiate the sample through the caller's autograd)");
+  ENTER(h);
+  // per row and step, as for the training backward; the scratch of step k is shared by every component (indexed by sorted
+  // position, and z1's stride Kp[0] is 32 for every step at D <= 64)
+  const long long per_row = (long long)ldz1 + nnets * (2LL * (L - 1) * hp + 64);
+  int rc = ensure_backward_buffers(h, need_w, B, per_row);
+  if (rc != GBNF_OK) return rc;
+  const long long njobs = (long long)n * K * nnets * L;
+  if (njobs > h->ib_cap) {
+    cudaFree(h->ib_steps_d); cudaFree(h->ib_pack_d); cudaFree(h->ib_jobs_d);
+    h->ib_steps_d = nullptr; h->ib_pack_d = nullptr; h->ib_jobs_d = nullptr; h->ib_cap = 0;
+    CUDA_TRY_H(h, cudaMalloc(&h->ib_steps_d, (size_t)njobs * sizeof(TrainStep)));
+    CUDA_TRY_H(h, cudaMalloc(&h->ib_pack_d, (size_t)njobs * sizeof(TrainPackJob)));
+    CUDA_TRY_H(h, cudaMalloc(&h->ib_jobs_d, (size_t)njobs * sizeof(RangedWgradJob)));
+    h->ib_cap = njobs;
+  }
+  const long long units = (B + kTrR - 1) / kTrR + n;
+  if (!h->ib_count) CUDA_TRY_H(h, cudaMalloc(&h->ib_count, sizeof(int)));
+  if (units > h->ib_units_cap) {
+    cudaFree(h->ib_units);
+    h->ib_units = nullptr; h->ib_units_cap = 0;
+    CUDA_TRY_H(h, cudaMalloc(&h->ib_units, units * sizeof(int4)));
+    h->ib_units_cap = units;
+  }
+  if (d_comp) {
+    rc = ensure_inverse_workspace(h, B, true);      // the counting sort's histogram and permutations
+    if (rc != GBNF_OK) return rc;
+  }
+  const int nblk = (int)((B + kSortRows - 1) / kSortRows);
+  h->ib_steps_h.assign((size_t)n * K, TrainStep{}); h->ib_pack_h.assign((size_t)njobs, TrainPackJob{}); h->ib_jobs_h.clear();
+  float* w = h->tr_w;
+  float* zeros = h->tr_w + (need_w - 1024);
+  int tile0 = 0, job = 0;
+  for (int i = 0; i < n; ++i)
+    for (int k = 0; k < K; ++k) {
+      const gbnf_step_params& sp = p[i].steps[k];
+      const gbnf_step_grads* sg = grads[i] ? grads[i] + k : nullptr;
+      const BwdGeo& g = geo[(size_t)i * K + k];
+      TrainStep& ts = h->ib_steps_h[(size_t)i * K + k];
+      if (glow) {
+        ts.an_bias = sp.an_bias; ts.an_logs = sp.an_logs; ts.perm = (const long long*)sp.perm;
+        if (sg) { ts.g_bias = sg->an_bias; ts.g_logs = sg->an_logs; }
+      }
+      ts.flipped = (!glow && (((k + c0 + i) % 2) > 0)) ? 1 : 0; ts.in_dim = g.in_dim; ts.out_dim = g.out_dim;
+      float* sc = h->tr_scratch + (size_t)k * h->tr_rows * per_row;
+      ts.z1 = sc; sc += h->tr_rows * ldz1;
+      for (int l = 0; l < L; ++l) { ts.Kp[l] = g.Kp[l]; ts.Np[l] = g.Np[l]; ts.NKp[l] = g.NKp[l]; ts.KNp[l] = g.KNp[l]; }
+      for (int net = 0; net < nnets; ++net) {
+        for (int l = 0; l < L - 1; ++l) { ts.hid[net][l] = sc; sc += h->tr_rows * hp; }
+        for (int l = 0; l < L - 1; ++l) { ts.dpre[net][l] = sc; sc += h->tr_rows * hp; }
+        ts.dpre[net][L - 1] = sc; sc += h->tr_rows * 64;
+        for (int l = 0; l < L; ++l, ++job) {
+          TrainPackJob& pj = h->ib_pack_h[(size_t)job];
+          pj.W = sp.W[net][l]; pj.b = sp.b[net][l]; pj.N = g.Nn[l]; pj.Kd = g.Kd[l]; pj.Kp = g.Kp[l]; pj.Np = g.Np[l]; pj.NKp = g.NKp[l]; pj.KNp = g.KNp[l];
+          pj.Wt = w; w += (long long)g.Kp[l] * g.Np[l];
+          pj.Wn = w; w += (long long)g.NKp[l] * g.KNp[l];
+          pj.bp = w; w += g.Np[l];
+          ts.Wt[net][l] = pj.Wt; ts.Wn[net][l] = pj.Wn; ts.b[net][l] = pj.bp;
+          if (!sg) continue;
+          RangedWgradJob rj{};
+          WgradJob& wj = rj.w;
+          wj.dact = ts.dpre[net][l];                        wj.ld_d = (l == L - 1) ? g.Np[L - 1] : hp;
+          wj.in = (l == 0) ? ts.z1 : ts.hid[net][l - 1];    wj.ld_i = (l == 0) ? g.Kp[0] : hp;
+          wj.dW = sg->W[net][l]; wj.db = sg->b[net][l]; wj.N = g.Nn[l]; wj.Kd = g.Kd[l];
+          wj.tiles_n = (g.Nn[l] + 63) / 64; wj.tiles_k = (g.Kd[l] + 63) / 64; wj.tile0 = tile0;
+          tile0 += wj.tiles_n * wj.tiles_k;
+          if (d_comp) { rj.lo = h->mix_hist + (long long)i * nblk; rj.hi = h->mix_hist + (long long)(i + 1) * nblk; }   // bin starts
+          h->ib_jobs_h.push_back(rj);
+        }
+      }
+      if (glow && sg) {
+        CUDA_TRY_H(h, cudaMemsetAsync(sg->an_bias, 0, (size_t)D * sizeof(float), st));
+        CUDA_TRY_H(h, cudaMemsetAsync(sg->an_logs, 0, (size_t)D * sizeof(float), st));
+      }
+    }
+  const int nw = (int)h->ib_jobs_h.size();
+  CUDA_TRY_H(h, cudaMemcpyAsync(h->ib_steps_d, h->ib_steps_h.data(), h->ib_steps_h.size() * sizeof(TrainStep), cudaMemcpyHostToDevice, st));
+  CUDA_TRY_H(h, cudaMemcpyAsync(h->ib_pack_d, h->ib_pack_h.data(), (size_t)njobs * sizeof(TrainPackJob), cudaMemcpyHostToDevice, st));
+  if (nw) CUDA_TRY_H(h, cudaMemcpyAsync(h->ib_jobs_d, h->ib_jobs_h.data(), (size_t)nw * sizeof(RangedWgradJob), cudaMemcpyHostToDevice, st));
+  CUDA_TRY_H(h, cudaMemsetAsync(zeros, 0, 1024 * sizeof(float), st));
+  train_pack_kernel<<<dim3(32, (unsigned)njobs), 256, 0, st>>>(h->ib_pack_d);
+  h->launches++;
+  int grid;
+  if (d_comp) {
+    // the stable counting sort of gbnf_mixture_inverse, cut into units of the backward's 16 rows
+    mix_sort_count_kernel<<<nblk, kSortRows, 0, st>>>(d_comp, B, n, nblk, h->mix_hist, h->flags);
+    mix_sort_scan_kernel<<<1, kSortRows, 0, st>>>(h->mix_hist, nblk, n, kTrR, h->ib_units, h->ib_count);
+    mix_sort_scatter_kernel<<<nblk, kSortRows, 0, st>>>(d_comp, B, n, nblk, h->mix_hist, h->mix_perm, h->mix_iperm);
+    h->launches += 3;
+    grid = (int)units;
+  } else {
+    grid = (int)((B + kTrR - 1) / kTrR);
+    component_units_kernel<<<grid_for(h, grid, 256), 256, 0, st>>>(0, B, kTrR, h->ib_units, h->ib_count);
+    h->launches++;
+  }
+  InvBwdArgs ia{};
+  ia.z = d_z; ia.B = B; ia.dx = d_dx; ia.dldj = d_dldj; ia.perm = d_comp ? h->mix_perm : nullptr; ia.units = h->ib_units;
+  ia.n_units = h->ib_count; ia.steps = h->ib_steps_d; ia.K = K; ia.D = D; ia.hp = hp; ia.act = cf.act; ia.coupling = cf.coupling;
+  ia.kind = cf.kind; ia.nnets = nnets; ia.nlayers = L; ia.ld = ld; ia.zeros = zeros; ia.dz = d_dz;
+  CUDA_TRY_H(h, cudaFuncSetAttribute(inv_bwd_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTrMaxSmem));
+  inv_bwd_rows_kernel<<<grid, kF32Threads, smem, st>>>(ia);
+  h->launches++;
+  if (nw) {
+    inv_wgrad_kernel<<<tile0, 256, 0, st>>>(h->ib_jobs_d, nw, B);
+    h->launches++;
+  }
+  CUDA_TRY_H(h, cudaGetLastError());
+  return GBNF_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int gbnf_component_inverse_backward(gbnf_handle h, int32_t c, const gbnf_component_params* p, const float* d_z, int64_t B,
+                                    const float* d_dx, const float* d_dldj, const gbnf_step_grads* grads, float* d_dz_opt, void* stream) {
+  if (!h || !p || !grads || !d_z || !d_dx || !d_dldj) return fail(GBNF_ERR_INVALID, "null argument");
+  if (c < 0 || c >= h->cfg.C) return fail(GBNF_ERR_INVALID, "bad component index");
+  return inverse_backward(h, c, 1, p, &grads, d_z, B, nullptr, d_dx, d_dldj, d_dz_opt, (cudaStream_t)stream);
+}
+
+int gbnf_mixture_inverse_backward(gbnf_handle h, const gbnf_component_params* p, const float* d_z, int64_t B, const int64_t* d_comp,
+                                  int32_t n_comp, const float* d_dx, const float* d_dldj, const gbnf_step_grads* const* grads,
+                                  float* d_dz_opt, void* stream) {
+  if (!h || !p || !grads || !d_z || !d_comp || !d_dx || !d_dldj) return fail(GBNF_ERR_INVALID, "null argument");
+  if (n_comp < 1 || n_comp > h->cfg.C) return fail(GBNF_ERR_INVALID, "bad component count");
+  return inverse_backward(h, 0, n_comp, p, grads, d_z, B, reinterpret_cast<const long long*>(d_comp), d_dx, d_dldj, d_dz_opt,
+                          (cudaStream_t)stream);
 }
 
 // ---- multi-GPU: peer-memory exchange over NVLink (one process per GPU; handles exchanged by the caller's plumbing) ---------------

@@ -16,7 +16,9 @@ torch.manual_seed has bit-identical initial parameters and permutations (tests/g
 
 Evaluation of FIXED components never runs through these modules' torch code: BoostedFlow routes it to the CUDA
 library.  `forward_autograd` below exists only for the component that is currently being trained, whose loss needs
-autograd (SURVEY 8 a12 / 8(f).1: its fused backward is the next row of the scope table).
+autograd (SURVEY 8 a12 / 8(f).1: its fused backward is the next row of the scope table).  `inverse_autograd` is its sampling
+counterpart: x = f^{-1}(z) and the log-det of the inverse map, differentiable in the parameters and in z.  It is the fp64
+reference of the library's fused inverse backward and the path BoostedFlow.rsample takes where that backward does not serve.
 """
 import math
 
@@ -126,6 +128,12 @@ class ActNorm1d(nn.Module):
         if not self.inited:
             self.initialize_parameters(x)
         return (x + self.bias) * torch.exp(self.logs), logdet + self.logs.sum()
+
+    def inverse(self, y, logdet):
+        """Reverse: scale then centre (models/layers.py:505-518)."""
+        if not self.inited:
+            raise ValueError("In Eval mode, but ActNorm not initiated")
+        return y * torch.exp(-self.logs) - self.bias, logdet - self.logs.sum()
 
 
 class Permute1d(nn.Module):
@@ -237,6 +245,26 @@ class GlowStep(nn.Module):
             logdet = logdet + torch.log(gate).sum(dim=1)
         return torch.cat((y1, y2), dim=1), logdet
 
+    def inverse_autograd(self, y, logdet):
+        """Coupling^-1, then permutation^-1 / 1x1 convolution^-1, then ActNorm^-1 (models/glow.py:344-366)."""
+        d_in = y.shape[1] // 2
+        y1, y2 = y[:, :d_in], y[:, d_in:]
+        out = self.block(y1)
+        if self.flow_coupling == "additive":
+            y2 = y2 - out
+        else:
+            gate = torch.sigmoid(out[:, 1::2] + 2.0)
+            y2 = y2 / gate - out[:, 0::2]
+            logdet = logdet - torch.log(gate).sum(dim=1)
+        z = torch.cat((y1, y2), dim=1)
+        if hasattr(self, "invconv"):
+            w, dlogdet = self.invconv.get_weight()
+            z = z @ torch.linalg.inv(w).t()
+            logdet = logdet - dlogdet
+        else:
+            z = z[:, self.permutation.indices_inverse.to(z.device)]
+        return self.actnorm.inverse(z, logdet)
+
 
 class GlowNet(nn.Module):
     def __init__(self, dim, hidden_dim, K, **kw):
@@ -279,6 +307,14 @@ class Glow(nn.Module):
             z, logdet = s.forward_autograd(z, logdet)
         return z, logdet
 
+    def inverse_autograd(self, z):
+        """(x, log-det of the inverse map) = f^{-1}(z), differentiable: the steps from the last to the first."""
+        logdet = torch.zeros(z.size(0), device=z.device, dtype=z.dtype)
+        x = z
+        for s in reversed(self.flow.layers):
+            x, logdet = s.inverse_autograd(x, logdet)
+        return x, logdet
+
 
 class BatchNorm(nn.Module):
     """RealNVP batch norm with log-det (models/layers.py:320-372).  Kernels implement the eval-mode branch."""
@@ -305,6 +341,13 @@ class BatchNorm(nn.Module):
         y = self.log_gamma.exp() * ((x - mean) / torch.sqrt(var + self.eps)) + self.beta
         ladj = self.log_gamma - 0.5 * torch.log(var + self.eps)
         return y, ladj.expand_as(x).sum(dim=1)
+
+    def inverse_eval(self, y):
+        """Inverse of the eval-mode branch (running statistics, as every inverse kernel uses): (x, its log-det)."""
+        sd = torch.sqrt(self.running_var + self.eps)
+        x = (y - self.beta) * torch.exp(-self.log_gamma) * sd + self.running_mean
+        ladj = -(self.log_gamma - 0.5 * torch.log(self.running_var + self.eps))
+        return x, ladj.expand_as(x).sum(dim=1)
 
 
 class RealNVPFlow(nn.Module):
@@ -359,6 +402,26 @@ class RealNVPFlow(nn.Module):
             z = torch.cat([z_a, z_b], dim=1)
             logdet = logdet + log_s.sum(dim=1)
         return z, logdet
+
+    def inverse_autograd(self, z):
+        """(x, log-det of the inverse map) = f^{-1}(z), differentiable: per step from the last, coupling^-1 (the forward's
+        output is [z1, z2'] for both flips) then eval-mode BatchNorm^-1."""
+        logdet = torch.zeros(z.size(0), device=z.device, dtype=z.dtype)
+        x = z
+        h0 = self.z_size // 2
+        for k in range(self.num_flows - 1, -1, -1):
+            t_net, s_net, bn = self.flow_param[k]
+            flipped = ((k + self.flip_init) % 2) > 0
+            n1 = self.z_size - h0 if flipped else h0
+            z1, z2 = x[:, :n1], x[:, n1:]
+            log_s = s_net(z1)
+            z2 = (z2 - t_net(z1)) * torch.exp(-log_s)
+            x = torch.cat([z2, z1], dim=1) if flipped else torch.cat([z1, z2], dim=1)
+            logdet = logdet - log_s.sum(dim=1)
+            if bn is not None:
+                x, l_bn = bn.inverse_eval(x)
+                logdet = logdet + l_bn
+        return x, logdet
 
 
 def rho_initial(num_components, rho_init, device):

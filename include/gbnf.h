@@ -237,6 +237,32 @@ int gbnf_component_backward(gbnf_handle h, int32_t c, const gbnf_component_param
                             const float* d_dz, const float* d_dldj, const gbnf_step_grads* grads, float* d_dx_opt,
                             void* stream);
 
+/* ---- sampling with gradients: backward of the inverse map (reparameterised samples, BoostedFlow.rsample) -------------------
+ * Gradients of any loss L(x, ldj_inv) of the inverse map x = f_c^{-1}(z) (gbnf_component_inverse / gbnf_mixture_inverse) with
+ * respect to the parameters of the components, given the upstream gradients dL/dx [B, D] and dL/dldj_inv [B] (for reverse KL,
+ * log q_c(x) = log N(z) - ldj_inv).  Recompute-in-kernel from z: the forward call saves nothing and its scratch is not read (other
+ * inverse calls may run in between); fp32 CUDA-core arithmetic whatever the GEMM mode.  The same envelope, shared-memory bound and
+ * scratch as gbnf_component_backward: Glow components with a permutation (tanh / relu, affine or additive) and RealNVP components
+ * WITHOUT BatchNorm (tanh / relu / mixed), coupling_network_depth 0 to 4, h <= 512, D <= 64, K within the bound listed there;
+ * 1 <= B <= 2^22.  The components must be packed (as for the forward call).  `p` holds their CURRENT raw parameters, `grads` the
+ * gradient buffers, which are OVERWRITTEN (a component that drew no rows gets zeros).  Every refusal (GBNF_ERR_INVALID for a
+ * configuration outside the envelope, GBNF_ERR_STATE for an unpacked component) comes before anything is written: `grads`,
+ * d_dz_opt and the handle stay as they were.  Weight and bias gradients are deterministic (no atomics); the ActNorm gradients
+ * are accumulated with atomics.  No host synchronisation.  d_dz_opt [B, D] (may be NULL) receives dL/dz.
+ *   gbnf_component_inverse_backward: component c, d_z in row order.
+ *   gbnf_mixture_inverse_backward:   x[i] = f_{comp[i]}^{-1}(z[i]) as for gbnf_mixture_inverse: p[n_comp] (host array), grads[n_comp]
+ *                                    (host array; grads[c] == NULL: component c needs no parameter gradient).  The rows are
+ *                                    sorted by component on the device again; the weight gradients of component c sum its rows in
+ *                                    their order, so they equal, bit for bit, a gbnf_component_inverse_backward call on those rows
+ *                                    alone.  An id outside [0, n_comp) is reported as for gbnf_mixture_inverse (its row's dz is
+ *                                    not written). */
+int gbnf_component_inverse_backward(gbnf_handle h, int32_t c, const gbnf_component_params* p, const float* d_z, int64_t B,
+                                    const float* d_dx, const float* d_dldj, const gbnf_step_grads* grads, float* d_dz_opt,
+                                    void* stream);
+int gbnf_mixture_inverse_backward(gbnf_handle h, const gbnf_component_params* p, const float* d_z, int64_t B,
+                                  const int64_t* d_comp, int32_t n_comp, const float* d_dx, const float* d_dldj,
+                                  const gbnf_step_grads* const* grads, float* d_dz_opt, void* stream);
+
 /* ---- multi-GPU on one node: one process per GPU, values exchanged through PEER MEMORY over NVLink ------------
  * The reference has no distributed code (SURVEY 2); this is the library-owned collective SURVEY 8(b) lists as
  * gbnf_comm_init.  No NCCL call sits on the data path: a rank publishes a value by storing it into every rank's
